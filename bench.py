@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- NanoWrap CG shrinkwrap hot path on B200 (contract: see DESIGN.md "Measurement").
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c2|c1]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c2|c1] [--dump-outputs DIR]
 
 A *step* is one CG iteration of ``ShrinkwrapMeshConjGrad.search`` over the rank's whole point shard
 (nearest-face rebuild included, as the reference rebuilds it every iteration; host remesh excluded,
@@ -27,6 +27,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 WORKLOADS = {
     # name: (points per GPU, geodesic frequency n -> 10 n^2 + 2 vertices, curvature_weight, block length)
@@ -122,9 +123,9 @@ class ClockSampler:
 def run_blocks(mesh, pts, s_inv, lam, n_iters, block, handle_profile=True):
     """n_iters CG iterations in blocks: new solver object + topology upload per block (what
     MembraneMesh.opt_conjugate_gradient does, _membrane_mesh.pyx:1510-1517).  Returns
-    (device ms inside nw_search summed over blocks, wall seconds of constructor+search, launches)."""
+    (device ms inside nw_search summed over blocks, wall seconds of constructor+search, last solver object, blocks run)."""
     from ch_shrinkwrap_b200.mesh_conj_grad import ShrinkwrapMeshConjGrad
-    dev_ms, wall, done = 0.0, 0.0, 0
+    dev_ms, wall, done, blocks = 0.0, 0.0, 0, 0
     sm = ctypes.c_double(0.0)
     cg = None
     while done < n_iters:
@@ -136,8 +137,9 @@ def run_blocks(mesh, pts, s_inv, lam, n_iters, block, handle_profile=True):
         wall += time.perf_counter() - t0
         cg._h.call('nw_get_profile', None, None, ctypes.byref(sm))
         dev_ms += sm.value
-        done += n_it
-    return dev_ms, wall, cg
+        done += cg.loopcount          # the stop rule may end a block early: count the iterations that ran
+        blocks += 1
+    return dev_ms, wall, cg, blocks
 
 
 def cpu_reference_run(workload, steps, warmup, seed):
@@ -205,7 +207,14 @@ def main():
     ap.add_argument('--cpu-steps', type=int, default=5, help='timed iterations of the cpu_baseline sample (our arm)')
     ap.add_argument('--ref-steps', type=int, default=0, help='reference arm: timed full-size iterations (default min(steps, 2))')
     ap.add_argument('--ref-warmup', type=int, default=-1, help='reference arm: untimed full-size iterations (default 0)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed search() call returned (vertices, float32 (M, 3)) '
+                         'and its test statistic / residual norm histories (tests, ress, float64) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -310,11 +319,10 @@ def main():
     mesh._nw_session.points_key = None
     barrier()
     t0 = time.perf_counter()
-    _, e2e_wall, cg = run_blocks(mesh, pts, s_inv, lam, K, block)
+    _, e2e_wall, cg, n_blocks = run_blocks(mesh, pts, s_inv, lam, K, block)
     e2e_s = allmax(time.perf_counter() - t0)
     h = cg._h
     topo_bytes = M * 12 * 2 + F * 12 + M * 80 + M
-    n_blocks = -(-K // block)
     e2e = {'value': P * world * K / e2e_s, 'unit': unit,
            'h2d_bytes_per_step': int((P * 24 + n_blocks * (topo_bytes + M * 12)) / K),
            'd2h_bytes_per_step': int(n_blocks * M * 12 / K),
@@ -334,10 +342,17 @@ def main():
     barrier()
     h.call('nw_sync')
     clocks.start()
-    dev_ms, _, cg = run_blocks(mesh, pts, s_inv, lam, K, block)
-    h.call('nw_sync')
-    barrier()
-    clk = clocks.stop()
+    try:
+        dev_ms, _, cg, _ = run_blocks(mesh, pts, s_inv, lam, K, block)
+        h.call('nw_sync')
+        barrier()
+    finally:
+        clk = clocks.stop()           # never leave the nvidia-smi sampler running
+    if args.dump_outputs and rank == 0:
+        # every rank ends with the same vertices; the histories are those of the last block's solver object
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in (('vertices', cg.fs), ('tests', np.array(cg.tests, np.float64)), ('ress', np.array(cg.ress, np.float64))):
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     launches = int(h.lib.nw_launch_count(h.h) - launches0)
     dev_ms = allmax(dev_ms)
     stage_ms = (ctypes.c_double * 16)()

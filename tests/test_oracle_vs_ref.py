@@ -1,4 +1,4 @@
-"""Live check of the oracle restatement against the reference itself (only where /root/reference exists)."""
+"""Live check of the oracle restatement against the reference itself (only where oracle/refharness.py can import it)."""
 import copy
 
 import numpy as np
