@@ -3,7 +3,6 @@
 // are read back once at the end (the reference's loop is mesh_conj_grad.py:218-290).
 #include <nvtx3/nvToolsExt.h>
 #include <cmath>
-#include <cstdio>
 #include <cstring>
 #include "common.cuh"
 
@@ -50,7 +49,7 @@ extern "C" void nw_destroy(nw_ctx *h) {
     nw_free(&h->w0); nw_free(&h->w1); nw_free(&h->w2);
     nw_free(&h->rx); nw_free(&h->ry); nw_free(&h->rz);
     nw_free(&h->posq); nw_free(&h->nrmq); nw_free(&h->faces); nw_free(&h->nbrT); nw_free(&h->valence); nw_free(&h->valid); nw_free(&h->stage_nbr); nw_free(&h->stage_hev); nw_free(&h->tb_small); nw_free(&h->tb_i0); nw_free(&h->tb_i1); nw_free(&h->tb_u0); nw_free(&h->tb_u1); nw_free(&h->tb_u2); nw_free(&h->fcells); nw_free(&h->cent64); nw_free(&h->parent_g); nw_free(&h->kids);
-    nw_free(&h->sfaces); nw_free(&h->cent); nw_free(&h->boxes); nw_free(&h->par); nw_free(&h->cbegin); nw_free(&h->leaf_of_slot); nw_free(&h->node_f);
+    nw_free(&h->sfaces); nw_free(&h->cent); nw_free(&h->boxes); nw_free(&h->leaf_of_slot); nw_free(&h->node_f);
     nw_free(&h->acc); nw_free(&h->Sq); nw_free(&h->fdef);
     nw_free(&h->partials); nw_free(&h->st); nw_free(&h->hist);
     nw_free((char **)&h->cub_tmp); nw_free(&h->scratchM); nw_free(&h->scratchP);
@@ -154,11 +153,6 @@ extern "C" int nw_get_traversal_stats(nw_ctx *h, uint64_t out[4]) {
     if (!h || !out) return NW_ERR_ARG;
     SolverState r;
     NW_CUDA(cudaMemcpy(&r, h->st, sizeof(SolverState), cudaMemcpyDeviceToHost));
-#ifdef NW_LEVEL_STATS
-    for (int l = 0; l < 12; ++l) fprintf(stderr, "level %2d tests %12llu pass %12llu\n", l, r.lvl_tests[l], r.lvl_pass[l]);
-    for (int b = 0; b <= 10; ++b) fprintf(stderr, "points with < %5u tests: %10llu  (%12llu tests)\n", 16u << b, r.lvl_pass[16 + b], r.lvl_tests[16 + b]);
-    fprintf(stderr, "lane slots paid (32 x slowest lane per warp): %llu\n", r.lvl_tests[31]);
-#endif
     for (int k = 0; k < 4; ++k) out[k] = r.trav[k];
     return NW_OK;
 }
@@ -224,12 +218,10 @@ extern "C" int nw_search(nw_ctx *h, float lam, int num_iters, int last_step, con
         // fits the iteration is launch-bound (C1: 0.25 ms of launches around microseconds of work).  Not under profiling
         // (per-stage events).  With a communicator the two ncclAllReduce calls of the iteration are captured with it
         // (NCCL supports stream capture; the eager first iteration has already run both collectives once, so nothing is
-        // allocated or connected inside the capture); NW_NO_COMM_GRAPH=1 keeps multi-rank runs eager.  The instantiated
-        // graph is kept for as long as the points and the topology stay (h->epoch): a fit calls nw_search once per block,
-        // and repeated calls on one block (continue / finishing iterations) replay the same executable.
-        static const bool no_graph = getenv("NW_NO_GRAPH") != nullptr;
-        static const bool no_comm_graph = getenv("NW_NO_COMM_GRAPH") != nullptr;
-        if (!no_graph && !h->profile && (h->nranks == 1 || !no_comm_graph) && num_iters - it >= 2) {
+        // allocated or connected inside the capture).  The instantiated graph is kept for as long as the points and the
+        // topology stay (h->epoch): a fit calls nw_search once per block, and repeated calls on one block (continue /
+        // finishing iterations) replay the same executable.
+        if (!h->profile && num_iters - it >= 2) {
             if (h->iter_graph && (h->iter_graph_epoch != h->epoch || h->iter_graph_last_step != last_step)) {
                 cudaGraphExecDestroy(h->iter_graph);
                 h->iter_graph = nullptr;

@@ -9,9 +9,7 @@
 
 #define NW_MAX_LEVELS 12
 #define NW_MAX_ITERS 4096
-#ifndef NW_S2_PTS
 #define NW_S2_PTS 4      // k_sweep2: points per thread (their dependent load chains slot -> face -> S overlap); sizes its partials
-#endif
 #define NW_N_STAGES 11   // refit, shift, sweep1, allreduce_acc, mesh_prior, sweep2, allreduce_scalars, solve_update, seed_leaders,
                          // topology_build (device side of nw_set_topology*: feet, unpack, Hilbert sort, tables, frames), adjoint
 
@@ -19,9 +17,10 @@
 // axis-aligned box is mostly empty space.  Axes n (patch normal), t1 = tangent_of(n), t2 = n x t1; one interval per axis.
 // It only ever prunes: the answer never depends on how tight it is.  (A spherical shell fitted to each node, which
 // removes the sagitta of large curved patches, was implemented and measured at C3: -4 % node tests, +15 % per test.)
-// -DNW_BOUNDS_CHECK (tools/build_variant.sh bounds "-DNW_BOUNDS_CHECK"): device-side assertions on every index the search
-// and the adjoint scatter form -- node ids, slots, vertex ids, shared-memory rows.  compute-sanitizer is closed on the GPU
-// pool this was developed on; the -m gpu suite run against that build is the memory-safety evidence (profiles/).
+// -DNW_BOUNDS_CHECK (NW_EXTRA_FLAGS=-DNW_BOUNDS_CHECK python -m ch_shrinkwrap_b200.build -f): device-side assertions on every
+// index the search and the adjoint scatter form -- node ids, slots, vertex ids, shared-memory rows.  compute-sanitizer is
+// closed on the GPU pool this was developed on; the -m gpu suite run against that build is the memory-safety evidence
+// (profiles/).
 #ifdef NW_BOUNDS_CHECK
 #include <cassert>
 #define NW_ASSERT(c) assert(c)
@@ -55,8 +54,7 @@ __host__ __device__ __forceinline__ float3 nw_tangent_of(const float nx, const f
 struct TreeLevels {
     int n_levels;                 // level 0 = root, n_levels-1 = leaf level
     int count[NW_MAX_LEVELS];     // nodes per level
-    int off[NW_MAX_LEVELS];       // node offset of the level in boxes[] / par[]
-    int cb_off[NW_MAX_LEVELS];    // offset of the level in cbegin[] (count+1 entries: first child; leaf level: first slot)
+    int off[NW_MAX_LEVELS];       // global id of the first node of the level: levels are stored back to back, root = 0
 };
 
 // Scalars produced and consumed on the device inside one search() call.
@@ -79,9 +77,6 @@ struct SolverState {
     float coord_l1;               // bound on |x|+|y|+|z| over vertices and points (rounding slack of the box tests)
     float lam;
     float cell_escape;            // grid units: how far any centroid has left the 1024^3 cell it was keyed into at upload (k_refit_centroids)
-#ifdef NW_LEVEL_STATS
-    unsigned long long lvl_tests[32], lvl_pass[32];   // diagnosis builds only: node tests / passes per tree level
-#endif
     unsigned long long trav[4];   // traversal statistics: node tests, leaf visits, exact fp64 evaluations, max node tests of one point
 };
 
@@ -126,8 +121,9 @@ struct nw_ctx {
     // ---- search hierarchy over the face centroids (tree.cu) ----
     int4 *sfaces = nullptr;                      // per sorted slot: corner ids + face id
     float4 *cent = nullptr;                      // per sorted slot: centroid xyz + face id bits
-    Box *boxes = nullptr;
-    int *par = nullptr, *cbegin = nullptr, *leaf_of_slot = nullptr;   // octree tables (see tree.cu)
+    Box *boxes = nullptr;                        // per global node id (levels back to back, root = 0; see tree.cu)
+    int *parent_g = nullptr; int2 *kids = nullptr;   // per global node id: parent | (the parent is a last child) << 31; first child / slot, count
+    int *leaf_of_slot = nullptr;                 // per sorted slot: its leaf, numbered within the leaf level
     float *node_f = nullptr;                     // 5 floats per node: normal sums, then sphere-fit moments (upload time)
     TreeLevels tl;
     bool seeds_cold = true;                      // no nearest-face seeds yet for this topology
@@ -136,7 +132,6 @@ struct nw_ctx {
     unsigned *fkeys = nullptr;                   // sorted Hilbert keys of the face centroids at upload time
     int *fkey_tab = nullptr;                     // lower_bound(fkeys, b << 15) for b = 0 .. 2^15: first step of the foot-point lookup
     float key_lo[3] = {0, 0, 0}, key_inv = 0.f;  // quantisation used for those keys
-    int *parent_g = nullptr; int2 *kids = nullptr;  // the same tree addressed by global node ids (what the search walks)
     unsigned *fcells = nullptr;                  // per sorted slot: grid cell of the centroid at upload time, x | y << 10 | z << 20
     bool points_mode = false;                    // the "faces" are raw target points (nw_set_point_targets): centroid = the point itself
     double *cent64 = nullptr;                    // points mode with float64 targets: exact coordinates per sorted slot (3 doubles)

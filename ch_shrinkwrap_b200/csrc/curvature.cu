@@ -116,13 +116,9 @@ __global__ void k_valid_flags(const VertRec *__restrict__ V, int M, int *__restr
 
 struct CurvOut { float *k0, *k1, *e0, *e1, *H, *K, *dH, *dK, *E, *pE, *dEnb, *dEdN; int *n_deleted; };
 
-#ifndef NW_CURV_MINB
-#define NW_CURV_MINB 4      // 128 registers, 16 warps per SM: measured at C3 0.285 ms (3 blocks, 152 registers) -> 0.242 ms; 5 blocks (96 registers, spills) 0.248 ms
-#endif
-#ifndef NW_CURV_BLOCK
 #define NW_CURV_BLOCK 128
-#endif
-__global__ void __launch_bounds__(NW_CURV_BLOCK, NW_CURV_MINB) k_curvature(const VertRec *__restrict__ V, const FaceRec *__restrict__ F,
+// 4 blocks per SM = 128 registers, 16 warps per SM: measured at C3 0.285 ms (3 blocks, 152 registers) -> 0.242 ms; 5 blocks (96 registers, spills) 0.248 ms
+__global__ void __launch_bounds__(NW_CURV_BLOCK, 4) k_curvature(const VertRec *__restrict__ V, const FaceRec *__restrict__ F,
                                                    const HeRec *__restrict__ HE, int M, float dN, float kc, float kg, float c0,
                                                    const double *__restrict__ jitter_u, const int *__restrict__ jitter_off,
                                                    unsigned long long seed, CurvOut o) {

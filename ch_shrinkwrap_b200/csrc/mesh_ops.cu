@@ -72,11 +72,8 @@ __global__ void k_shift_final(float plo_x, float plo_y, float plo_z, float phi_x
 
 #define NW_MSUM 14  // hw00 hw01 hw11 hw02 hw12 hw22 gw0 gw1 gw2 | s0.s1 s0.s0 s1.s1 | sum prefs32^2 | sum prefs64^2
 
-#ifndef NW_MP_MINB
-#define NW_MP_MINB 3
-#endif
 template <bool WRITE_DIRS>
-__global__ void __launch_bounds__(256, NW_MP_MINB) k_mesh_prior(int M, unsigned long long *__restrict__ acc, SolverState *__restrict__ st,
+__global__ void __launch_bounds__(256, 3) k_mesh_prior(int M, unsigned long long *__restrict__ acc, SolverState *__restrict__ st,
                                                     const float4 *__restrict__ posq, const float4 *__restrict__ nrmq,
                                                     const int *__restrict__ nbrT, const int *__restrict__ valence,
                                                     float4 *__restrict__ Sq,

@@ -12,7 +12,6 @@
 // float atomics are not); the Gram sums use a fixed thread->point assignment and a fixed two-stage tree.
 #include <cub/cub.cuh>
 #include <cfloat>
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 #include "common.cuh"
@@ -90,31 +89,6 @@ struct Nearest {
     }
 };
 
-// packed float32 pairs (sm_100a: FFMA2 / FMUL2 / FADD2 take an aligned 64-bit register pair and, for one source, a scalar
-// broadcast): two IEEE operations per instruction.  Only used with -DNW_PACKED_NODE_TEST (tools/build_variant.sh): measured at
-// C3, the packed stage-1 node test is 6 instructions shorter (23 instead of 29) and the warm sweep 3 % SLOWER (1.85 vs 1.79
-// ms) -- on B200 a packed instruction evidently occupies the FMA pipe for both halves, and the kernel's dependent chain per
-// step gets longer.  The box layout (both axes interleaved) is what that experiment needed; the scalar test does not care.
-#ifdef NW_PACKED_NODE_TEST
-__device__ __forceinline__ unsigned long long f2_pack(float2 v) { unsigned long long r; asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(v.x), "f"(v.y)); return r; }
-__device__ __forceinline__ float2 f2_unpack(unsigned long long v) { float2 r; asm("mov.b64 {%0,%1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(v)); return r; }
-__device__ __forceinline__ float2 f2_fma(float2 a, float s, float2 c) {          // a * s + c, one rounding per component
-    unsigned long long r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(f2_pack(a)), "l"(f2_pack(make_float2(s, s))), "l"(f2_pack(c)));
-    return f2_unpack(r);
-}
-__device__ __forceinline__ float2 f2_mul(float2 a, float s) {
-    unsigned long long r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(f2_pack(a)), "l"(f2_pack(make_float2(s, s))));
-    return f2_unpack(r);
-}
-__device__ __forceinline__ float2 f2_sub(float2 a, float2 b) {
-    unsigned long long r;
-    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(f2_pack(a)), "l"(f2_pack(b)));
-    return f2_unpack(r);
-}
-#endif
-
 // Conservative lower bound of the squared distance from the query to anything inside a node: the sum over the three
 // box axes of (interval gap)^2.  Projections are float32, so every interval is widened by an absolute slack (>= 4x the worst-case rounding error of
 // both the query's and the members' evaluation, DESIGN.md "exactness") and the squares by a relative 1e-5 (axes are
@@ -122,12 +96,11 @@ __device__ __forceinline__ float2 f2_sub(float2 a, float2 b) {
 // so skipping can never change the answer.
 // (The walk itself uses the two-stage form of this test, Traversal::test_node.  Each 128-bit load of a node quarter also
 // costs two moves of the warp-uniform node address into the vector registers it is about to overwrite; an opaque per-thread
-// copy of the address does not change that allocation at 32 registers, and 256-bit loads do not pay either -- see test_node.)
+// copy of the address does not change that allocation at 32 registers, and 256-bit loads do not pay either: DESIGN.md.)
 template <typename Q>
-__device__ __forceinline__ float node_lb(const Q &q, const Box *__restrict__ bp, float eps, int *link = nullptr) {
+__device__ __forceinline__ float node_lb(const Q &q, const Box *__restrict__ bp) {
     const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), c = __ldg(&bp->c), d = __ldg(&bp->d);
     const float x = q.fx(), y = q.fy(), z = q.fz();
-    if (link) *link = __float_as_int(d.z);           // first child | last-child flag (k_global_tables)
     const float pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
     const float p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
     const float p2 = fmaf(c.x, x, fmaf(c.y, y, c.z * z));      // t2 = n x t1
@@ -142,7 +115,7 @@ __device__ __forceinline__ float node_lb(const Q &q, const Box *__restrict__ bp,
 // greedy-descent score: the bound, with the squared distance to the box centre as a tie-breaker (several overlapping
 // boxes can contain the query and all have bound 0)
 template <typename Q>
-__device__ __forceinline__ float node_score(const Q &q, const Box *__restrict__ bp, float eps) {
+__device__ __forceinline__ float node_score(const Q &q, const Box *__restrict__ bp) {
     const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), c = __ldg(&bp->c), d = __ldg(&bp->d);
     const float x = q.fx(), y = q.fy(), z = q.fz();
     const float pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
@@ -201,10 +174,6 @@ struct Traversal {
     TreeView tv;
     float eps;
     unsigned n_tests = 0, n_leaves = 0, n_exact = 0;
-#ifdef NW_LEVEL_STATS
-    SolverState *dbg = nullptr;
-    const TreeLevels *dbg_tl = nullptr;
-#endif
     unsigned budget = 0xffffffffu;   // seeds only: stop refining after this many node tests (the result is then approximate)
     // COUNT = false (the production sweep): no statistics, no budget -- three registers and three instructions per step
     __device__ __forceinline__ bool tick() { if constexpr (COUNT) return ++n_tests > budget; else return false; }
@@ -265,15 +234,6 @@ struct Traversal {
             } else if (q.lb_box(c, c) <= best.ub) { if constexpr (COUNT) ++n_exact; best.offer(q.d2(c), s, __float_as_int(c.w)); }
         }
     }
-#ifdef NW_LEVEL_STATS
-    __device__ __forceinline__ void count_test(int node, bool pass) {
-        if (!dbg || !active) return;
-        int level = 0;
-        while (level + 1 < dbg_tl->n_levels && node >= dbg_tl->off[level + 1]) ++level;
-        atomicAdd(&dbg->lvl_tests[level], 1ull);
-        if (pass) atomicAdd(&dbg->lvl_pass[level], 1ull);
-    }
-#endif
     // Depth-first search of the subtree rooted at node I.  First child and next sibling come from two small integer
     // tables, so no per-thread stack is needed.  Children are visited in index (= Hilbert) order: with a seed the bound
     // is already (nearly) exact, so nearest-first ordering would buy nothing.
@@ -283,36 +243,13 @@ struct Traversal {
     // bound is formed from the same partial sum: the same nodes are opened as with a one-stage test.
     __device__ __forceinline__ bool test_node(const Box *__restrict__ bp, int &link) {
         NW_ASSERT(bp >= tv.boxes && bp < tv.boxes + tv.n_nodes);
-#ifdef NW_LDG256
-        // quarters a and b with ONE 256-bit load (LDG.E.ENL2.256 on sm_100a; the v4.b64 spelling -- ptxas 12.9 segfaults on
-        // ld.global.nc.v8.f32 in this file).  Measured at C3: one instruction and two address moves less per test, and the
-        // warm sweep does not move (1.80 vs 1.80 ms); loading c and d the same way costs registers the kernel does not
-        // have (spills, 3.4 ms)
-        float4 a, b;
-        {
-            unsigned long long v0, v1, v2, v3;
-            asm volatile("ld.global.nc.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(v0), "=l"(v1), "=l"(v2), "=l"(v3) : "l"(bp));
-            a.x = __uint_as_float((unsigned)v0); a.y = __uint_as_float((unsigned)(v0 >> 32));
-            a.z = __uint_as_float((unsigned)v1); a.w = __uint_as_float((unsigned)(v1 >> 32));
-            b.x = __uint_as_float((unsigned)v2); b.y = __uint_as_float((unsigned)(v2 >> 32));
-            b.z = __uint_as_float((unsigned)v3); b.w = __uint_as_float((unsigned)(v3 >> 32));
-        }
-        const float4 d = __ldg(&bp->d);
-#else
         const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), d = __ldg(&bp->d);
-#endif
         const float x = q.fx(), y = q.fy(), z = q.fz();
         link = __float_as_int(d.z);
         // (pn, p1) = (n, t1) . q ; same operations and association as node_lb
-#ifdef NW_PACKED_NODE_TEST
-        const float2 p = f2_fma(make_float2(a.x, a.y), x, f2_fma(make_float2(a.z, a.w), y, f2_mul(make_float2(b.x, b.y), z)));
-        const float2 glo = f2_sub(make_float2(b.z, b.w), p), ghi = f2_sub(p, make_float2(d.x, d.y));
-        const float g0 = fmaxf(fmaxf(glo.x, ghi.x), 0.f), g1 = fmaxf(fmaxf(glo.y, ghi.y), 0.f);
-#else
         const float pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
         const float p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
         const float g0 = fmaxf(fmaxf(b.z - pn, pn - d.x), 0.f), g1 = fmaxf(fmaxf(b.w - p1, p1 - d.y), 0.f);
-#endif
         const float s01 = __fmaf_rd(g1, g1, __fmul_rd(g0, g0));            // <= g0^2 + g1^2
         if (!any(s01 <= best.ub)) return false;                     // (best.ub already holds the frames' 1e-5, Nearest::offer)
         const float4 c = __ldg(&bp->c);
@@ -325,14 +262,7 @@ struct Traversal {
         while (true) {
             int link;                                      // first child | (node is a last child) << 31, stored in the node itself
             if (tick()) return;
-#ifdef NW_ONE_STAGE_TEST
-            const bool pass = any(node_lb(q, &tv.boxes[node], eps, &link) <= best.ub);
-#else
             const bool pass = test_node(&tv.boxes[node], link);
-#endif
-#ifdef NW_LEVEL_STATS
-            count_test(node, pass);
-#endif
             if (pass) {
                 if (node >= tv.leaf0) leaf(node);
                 else {
@@ -368,7 +298,7 @@ struct Traversal {
         const QueryF32 pk_c = packet_centre();
         const int j = (int)(threadIdx.x & 31);
         bool hit = false;
-        if (j < n && c0 + j != skip) hit = !(__fsqrt_rd(node_lb(pk_c, &tv.boxes[c0 + j], eps)) > reach);
+        if (j < n && c0 + j != skip) hit = !(__fsqrt_rd(node_lb(pk_c, &tv.boxes[c0 + j])) > reach);
         if constexpr (COUNT) ++n_tests;
         return __ballot_sync(0xffffffffu, hit);
     }
@@ -400,7 +330,7 @@ struct Traversal {
             const int2 k = __ldg(&tv.kids[node]);
             float bl = FLT_MAX * 2.0f;
             for (int ch = k.x; ch < k.x + k.y; ++ch) {
-                float l = node_score(q, &tv.boxes[ch], eps);
+                float l = node_score(q, &tv.boxes[ch]);
                 if constexpr (PACKET) l = __shfl_sync(0xffffffffu, l, lead);
                 if constexpr (COUNT) ++n_tests;
                 if (l < bl) { bl = l; node = ch; }
@@ -585,29 +515,19 @@ struct Sweep1Args {
     const float4 *posq;
     const int4 *sfaces;
     TreeView tv;
-    TreeLevels tl;
     int F;
     unsigned long long *acc;
     SolverState *st;
 };
 
-#ifndef NW_FN_INLINE
-#define NW_FN_INLINE __noinline__
-#endif
-#ifndef NW_S1_MINB
-#define NW_S1_MINB 16     // blocks of 128 per SM for the search kernels: 32 registers, 64 warps per SM (see k_sweep1)
-#endif
 template <bool F64, bool STATS, bool T64>
-__device__ NW_FN_INLINE Nearest find_nearest(const Sweep1Args &a, int64_t i, bool active, float x, float y, float z,
+__device__ __noinline__ Nearest find_nearest(const Sweep1Args &a, int64_t i, bool active, float x, float y, float z,
                                              double xd, double yd, double zd, Nearest best, int block_seed = -1) {
     const float eps = (fabsf(x) + fabsf(y) + fabsf(z) + a.st->coord_l1) * 9.5367431640625e-7f;   // 2^-20 * L1 magnitude
     typename std::conditional<F64, QueryF64, QueryF32>::type q;
     if constexpr (F64) q.set(xd, yd, zd);
     else { q.x = x; q.y = y; q.z = z; }
     Traversal<decltype(q), true, STATS, T64> tr(q, best, a.tv, eps, a.st->cell_escape, active);
-#ifdef NW_LEVEL_STATS
-    tr.dbg = a.st; tr.dbg_tl = &a.tl;
-#endif
     int seed = active ? a.slot[i] : -1;
     const unsigned alive = __ballot_sync(0xffffffffu, active);
     if (alive) {                                             // warp-uniform
@@ -637,18 +557,7 @@ __device__ NW_FN_INLINE Nearest find_nearest(const Sweep1Args &a, int64_t i, boo
     if ((threadIdx.x & 31) == 0) {
         atomicAdd(&a.st->trav[0], (unsigned long long)t); atomicAdd(&a.st->trav[1], (unsigned long long)l);
         atomicAdd(&a.st->trav[2], (unsigned long long)e); atomicMax(&a.st->trav[3], (unsigned long long)m);
-#ifdef NW_LEVEL_STATS
-        atomicAdd(&a.st->lvl_tests[31], 32ull * m);          // lane slots a warp pays for: 32 x its slowest lane
-#endif
     }
-#ifdef NW_LEVEL_STATS
-    if (active) {                                            // histogram of node tests per point, log2 buckets from 16
-        int b = 0;
-        while (b < 10 && (16u << b) <= tr.n_tests) ++b;
-        atomicAdd(&a.st->lvl_pass[16 + b], 1ull);
-        atomicAdd(&a.st->lvl_tests[16 + b], (unsigned long long)tr.n_tests);
-    }
-#endif
     }
     return tr.best;
 }
@@ -740,10 +649,11 @@ __global__ void __launch_bounds__(128) k_seed_from_feet(const __grid_constant__ 
 }
 
 // MODE 0: nearest face + weights only (what calc_w triggers);  MODE 1: + residual + adjoint scatter
-// 32 registers, 64 warps per SM (NW_S1_MINB = 16).  Measured at C3 (warm sweep, ms): 56 regs 3.23, 48 regs 3.08, 40 regs 3.00 before the
-// global-id tables; after them 48 regs 2.47, 40 regs 2.51, 32 regs 2.33 -- the packet walk is a dependent chain, occupancy hides it
+// 16 blocks of 128 per SM: 32 registers, 64 warps per SM (12 blocks with float64 points).  Measured at C3 (warm sweep, ms): 56 regs
+// 3.23, 48 regs 3.08, 40 regs 3.00 before the global-id tables; after them 48 regs 2.47, 40 regs 2.51, 32 regs 2.33 -- the packet
+// walk is a dependent chain, occupancy hides it
 template <bool F64, int MODE, bool STATS, bool T64 = false>
-__global__ void __launch_bounds__(128, F64 ? (NW_S1_MINB > 12 ? 12 : NW_S1_MINB) : NW_S1_MINB) k_sweep1(const __grid_constant__ Sweep1Args a) {
+__global__ void __launch_bounds__(128, F64 ? 12 : 16) k_sweep1(const __grid_constant__ Sweep1Args a) {
     if (MODE == 1 && a.st->stop) return;
 
     // schedule entry: block of points | quarter << 28.  quarter 0: all 32 lanes of every warp are points; 1..4: only lanes
@@ -849,14 +759,9 @@ __global__ void __launch_bounds__(256) k_apply_A(int64_t P, const int *__restric
 // out_v += sum w_pj r_p  (Ahfunc, conj_grad_utils.c:123-167) into the fixed-point accumulators; INFL: channel 3 += sum w_pj
 // (AH applied to ones) in the same pass -- the form the CG iteration runs right after k_sweep1.  st != NULL: the shifts are
 // the device-side ones of this iteration (k_shift_final) and a raised stop flag makes the kernel a no-op.
-#ifndef NW_ADJ_TILES
 #define NW_ADJ_TILES 2      // points per thread: the loads of all of them are in flight before the first one is processed
-#endif
-#ifndef NW_ADJ_MINB
-#define NW_ADJ_MINB 4
-#endif
 template <bool INFL>
-__global__ void __launch_bounds__(256, NW_ADJ_MINB) k_adjoint(int64_t P, const int *__restrict__ slot, const int4 *__restrict__ sfaces,
+__global__ void __launch_bounds__(256, 4) k_adjoint(int64_t P, const int *__restrict__ slot, const int4 *__restrict__ sfaces,
                                                  const float *__restrict__ w0, const float *__restrict__ w1, const float *__restrict__ w2,
                                                  const float *__restrict__ rx, const float *__restrict__ ry, const float *__restrict__ rz,
                                                  unsigned long long *__restrict__ acc, const SolverState *__restrict__ st, int shift, int shift_i,
@@ -906,11 +811,7 @@ __global__ void __launch_bounds__(256) k_apply_infl(int64_t P, const int *__rest
 // ---- Gram pass -------------------------------------------------------------------------------------
 #define NW_NSUM 11   // hc00 hc01 hc11 hc02 hc12 hc22 gc0 gc1 gc2 c0 res2
 
-#ifndef NW_S2_MINB
-#define NW_S2_MINB 1
-#endif
-
-__global__ void __launch_bounds__(256, NW_S2_MINB) k_sweep2(int64_t P, const int *__restrict__ slot, const int4 *__restrict__ sfaces,
+__global__ void __launch_bounds__(256, 1) k_sweep2(int64_t P, const int *__restrict__ slot, const int4 *__restrict__ sfaces,
                                                 const float *__restrict__ w0, const float *__restrict__ w1, const float *__restrict__ w2,
                                                 const float *__restrict__ rx, const float *__restrict__ ry, const float *__restrict__ rz,
                                                 const float4 *__restrict__ Sq,
@@ -1072,14 +973,12 @@ static Sweep1Args make_args(nw_ctx *h) {
     a.sinv_scalar = h->sinv_scalar; a.wmean = h->wmean;
     a.slot = h->slot;
     a.w0 = h->w0; a.w1 = h->w1; a.w2 = h->w2; a.rx = h->rx; a.ry = h->ry; a.rz = h->rz;
-    a.posq = h->posq; a.sfaces = h->sfaces; a.tl = h->tl; a.F = h->F;
+    a.posq = h->posq; a.sfaces = h->sfaces; a.F = h->F;
     a.tv.cent = h->cent; a.tv.cent64 = h->points_mode ? h->cent64 : nullptr; a.tv.boxes = h->boxes; a.tv.parent = h->parent_g; a.tv.kids = h->kids; a.tv.leaf_of_slot = h->leaf_of_slot;
     a.tv.leaf_level = h->tl.n_levels - 1; a.tv.leaf0 = h->tl.n_levels > 0 ? h->tl.off[h->tl.n_levels - 1] : 0;
     a.tv.n_nodes = h->tl.n_levels > 0 ? h->tl.off[h->tl.n_levels - 1] + h->tl.count[h->tl.n_levels - 1] : 0; a.tv.n_slots = h->F;
     a.tv.fcells = h->fcells; a.tv.grid_lo = make_float3(h->key_lo[0], h->key_lo[1], h->key_lo[2]); a.tv.grid_inv = h->key_inv;
     a.tv.grid_cellw = h->key_inv > 0.f ? 1.f / h->key_inv : 0.f;
-    static const bool no_clear = getenv("NW_NO_CELL_CLEARANCE") != nullptr;      // A/B switch for measurements
-    if (no_clear) a.tv.grid_inv = 0.f;
     a.acc = h->acc; a.st = h->st;
     a.order = nullptr;
     return a;
@@ -1114,8 +1013,8 @@ int nw_launch_seed_leaders(nw_ctx *h) {
     // point seeded by them -- the sweep gains 0.8 ms from exact seeds, but packets of points that lie 32 apart cost 6 ms)
     // one bounded root search per block of k_sweep1 (128 points, Hilbert neighbours): measured at C3, seeds + first sweep in
     // ms -- every 32nd point, budget 512: 3.4 + 5.6; 256: 2.5 + 5.7; 128: 1.8 + 6.3; 64: 0.9 + 42 (seeds too poor)
-    static const unsigned budget = getenv("NW_SEED_BUDGET") ? (unsigned)atoi(getenv("NW_SEED_BUDGET")) : 256u;
-    static const int stride = getenv("NW_SEED_STRIDE") ? std::max(32, atoi(getenv("NW_SEED_STRIDE")) / 32 * 32) : 128;
+    const unsigned budget = 256;
+    const int stride = 128;
     const int GL = nw_grid(((h->P + stride - 1) / stride) * 32, B);
     if (h->px64) k_seed_leaders<true><<<GL, B, 0, h->stream>>>(a, stride, budget);
     else k_seed_leaders<false><<<GL, B, 0, h->stream>>>(a, stride, budget);
@@ -1179,13 +1078,11 @@ static int build_block_order(nw_ctx *h, int G) {
     h->launches += 2;
     h->order_stale = false;
     h->cold_grid = 0;
-    static const bool no_split = getenv("NW_NO_COLD_SPLIT") != nullptr;           // A/B switch for measurements
-    if (h->leaders_fresh && !no_split && G >= 64 && G < (1 << 26)) {
+    if (h->leaders_fresh && G >= 64 && G < (1 << 26)) {
         // how many: measured at C3 (78 k blocks), first sweep in ms for the costliest 1/4 .. 1/1024 of the blocks split --
         // 11.6, 8.8, 7.1, 6.5, 6.0, 5.8, 5.7, 5.6, 5.5 (9.5 unsplit): the pathological packets are a handful, and every
         // other block that is split pays for 24 idle lanes per warp
-        static const int far_div = getenv("NW_COLD_FAR_DIV") ? std::max(1, atoi(getenv("NW_COLD_FAR_DIV"))) : 512;
-        const int n_far = std::min(G, std::max(32, G / far_div));
+        const int n_far = std::min(G, std::max(32, G / 512));
         NW_CHECK(nw_alloc(h, &h->blk_order_cold, (size_t)G + 3 * (size_t)n_far));
         k_cold_order<<<nw_grid(G, 256), 256, 0, h->stream>>>(h->blk_order, G, n_far, h->blk_order_cold);
         NW_LAUNCH_CHECK();
@@ -1199,19 +1096,14 @@ int nw_launch_sweep1(nw_ctx *h, bool scatter) {
     const int B = 128;
     const int G = nw_grid(h->P, B);
     NW_CHECK(nw_launch_seed_leaders(h));
-    static const bool no_order = getenv("NW_NO_BLOCK_ORDER") != nullptr;          // A/B switch for measurements
-    if (h->order_stale && !no_order) NW_CHECK(build_block_order(h, G));
+    if (h->order_stale) NW_CHECK(build_block_order(h, G));
     Sweep1Args a = make_args(h);
-    a.order = no_order ? nullptr : h->blk_order;
+    a.order = h->blk_order;
     int G1 = G;
-    if (h->leaders_fresh && h->cold_grid > 0 && !no_order) { a.order = h->blk_order_cold; G1 = h->cold_grid; }
+    if (h->leaders_fresh && h->cold_grid > 0) { a.order = h->blk_order_cold; G1 = h->cold_grid; }
     h->leaders_fresh = false;                       // only the very first sweep after the root searches is scheduled this way
     // traversal statistics (nw_get_traversal_stats) are collected only when asked for: nw_set_profile(h, 3)
-#ifdef NW_LEVEL_STATS
-    const bool stats = true;
-#else
     const bool stats = (h->profile & 2) != 0;
-#endif
     if (a.tv.cent64) {
         // points mode with float64 targets (nw_set_point_targets): only the nearest-target query exists, no statistics
         NW_ARG(!scatter, "sweep1: float64 point targets support nearest-point queries only");

@@ -7,9 +7,7 @@
 // re-measures each node's oriented box.
 #include <cub/cub.cuh>
 #include <cfloat>
-#include <cstdlib>
 #include "common.cuh"
-#include <chrono>
 #include <thread>
 #include <vector>
 
@@ -152,9 +150,15 @@ __device__ __forceinline__ void project3(const float3 n, const float4 c, float &
 // bits of their (sorted) Hilbert key, i.e. one cube of the 2^k grid -- always a compact piece of surface.  (Cutting the
 // sorted order into fixed-size chunks instead mixes pieces that are consecutive on the curve but far apart in space:
 // measured boxes of 1/120 of the surface spanned half the object.)  Because the keys are sorted every node is a
-// contiguous range of slots, its children are a contiguous range of nodes one level down, and traversal needs two small
-// integer tables per level: `par` (parent index, top bit = "last child of its parent") and `cbegin` (first child; at the
-// leaf level: first slot).
+// contiguous range of slots and its children are a contiguous range of nodes one level down.  Nodes have ONE numbering,
+// the global id: the levels are stored back to back (root = 0, TreeLevels::off), and within a level nodes are in key
+// order.  Three tables per node, all in global ids, are what the search and the refit walk:
+//   kids[g]     = {first child, number of children}; for a leaf {first slot, number of centroids}
+//   parent_g[g] = parent | (the PARENT is the last child of ITS parent) << 31, so that popping a level is one load
+//                 (the root's entry: 0 | 1 << 31)
+//   Box::d.z    = kids[g].x | (this node is a last child) << 31, as int bits: what a search step needs next, whether the
+//                 node is pruned (next sibling or pop) or opened (first child), arrives with the box it has just loaded
+// leaf_of_slot numbers the leaves within the leaf level (the leaf of slot s is leaf0 + leaf_of_slot[s]).
 // ======================================================================================================================
 
 // histogram of the level at which consecutive keys first differ (-> number of nodes of every level)
@@ -178,31 +182,32 @@ __global__ void k_level_flags(const unsigned *__restrict__ keys, int F, int shif
     flag[i] = (i == 0) ? 1 : (shift >= 32 ? 0 : ((keys[i] >> shift) != (keys[i - 1] >> shift)));
 }
 
-// id = inclusive scan of the flags (1-based node id per slot).  Writes, for the nodes of this level: first slot, parent,
-// and for the parent level the first-child table.
-__global__ void k_level_tables(const int *__restrict__ flag, const int *__restrict__ id, const int *__restrict__ id_parent,
-                               int F, int *__restrict__ start, int *__restrict__ par, int *__restrict__ cbegin_parent) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= F || !flag[i]) return;
-    const int j = id[i] - 1;
-    start[j] = i;
-    if (id_parent) {
-        const int pj = id_parent[i] - 1;
-        par[j] = pj;
-        if (i == 0 || id_parent[i - 1] != id_parent[i]) cbegin_parent[pj] = j;     // first child of pj
-    } else par[j] = 0;
+// slot i is the last slot of its level-`lvl` node
+__device__ __forceinline__ bool ends_node(const unsigned *__restrict__ keys, int F, int lvl, int i) {
+    return i == F - 1 || ((keys[i] ^ keys[i + 1]) >> (30 - 3 * lvl)) != 0;
 }
-// top bit of par = this node is the last child of its parent
-__global__ void k_mark_last_child(int *__restrict__ par, int n) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
-    const int p = par[j] & 0x7fffffff;
-    const bool last = (j == n - 1) || ((par[j + 1] & 0x7fffffff) != p);
-    par[j] = p | (last ? 0x80000000 : 0);
-}
-__global__ void k_copy_minus1(const int *__restrict__ id, int F, int *__restrict__ out) {
+
+// The tables of the level-`lvl` nodes, written once the level below them is numbered.  id_up / start_up: number within
+// level `lvl` (inclusive scan of its flags, 1-based) of every slot / first slot of every node; id / start: the same for
+// level `lvl` + 1, whose `start` is recorded here for the next call.  id == nullptr: level `lvl` is the leaf level, its
+// children are the slots, and leaf_of_slot is written.  lvl < 0: only the root's start.
+__global__ void k_level_tables(const unsigned *__restrict__ keys, int F, int lvl, int off_up, const int *__restrict__ id_up,
+                               const int *__restrict__ start_up, int off, const int *__restrict__ id, int *__restrict__ start,
+                               int *__restrict__ parent_g, int2 *__restrict__ kids, Box *__restrict__ boxes,
+                               int *__restrict__ leaf_of_slot) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < F) out[i] = id[i] - 1;
+    if (i >= F) return;
+    if (!id) leaf_of_slot[i] = id_up[i] - 1;
+    else if (i == 0 || id[i - 1] != id[i]) start[id[i] - 1] = i;
+    if (lvl < 0 || !ends_node(keys, F, lvl, i)) return;
+    // slot i ends node p: its children are the nodes (slots) from the one of its first slot to the one of slot i
+    const int p = off_up + id_up[i] - 1, s0 = start_up[id_up[i] - 1];
+    const int c0 = id ? off + id[s0] - 1 : s0, c1 = id ? off + id[i] - 1 : i;
+    const unsigned last = (lvl == 0 || ends_node(keys, F, lvl - 1, i)) ? 0x80000000u : 0u;    // p ends where its parent does
+    kids[p] = make_int2(c0, c1 - c0 + 1);
+    boxes[p].d.z = __int_as_float((int)((unsigned)c0 | last));
+    if (id) for (int c = c0; c <= c1; ++c) parent_g[c] = (int)((unsigned)p | last);
+    if (lvl == 0) parent_g[0] = (int)0x80000000u;
 }
 
 // centroids at the current f, in sorted order
@@ -233,7 +238,7 @@ __global__ void k_refit_centroids(const int4 *__restrict__ sfaces, const float4 
 // children.  (The first version summed every face into all of its ancestors with MATCH + 96 shuffles per level: 183 us per
 // build at C3 against ~40 now.)
 __global__ void __launch_bounds__(256) k_leaf_normals(const int4 *__restrict__ sfaces, const float4 *__restrict__ pos, int F,
-                                                      const int *__restrict__ leaf_of_slot, float *__restrict__ nsum_leaf) {
+                                                      const int *__restrict__ leaf_of_slot, int leaf0, float *__restrict__ nsum) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= F) return;
     const int4 sf = sfaces[i];
@@ -241,19 +246,19 @@ __global__ void __launch_bounds__(256) k_leaf_normals(const int4 *__restrict__ s
     const float ux = b.x - a.x, uy = b.y - a.y, uz = b.z - a.z, vx = d.x - a.x, vy = d.y - a.y, vz = d.z - a.z;
     float3 fn = make_float3(uy * vz - uz * vy, uz * vx - ux * vz, ux * vy - uy * vx);
     if (!(fabsf(fn.x) <= FLT_MAX && fabsf(fn.y) <= FLT_MAX && fabsf(fn.z) <= FLT_MAX)) return;
-    float *dst = nsum_leaf + 3 * (size_t)leaf_of_slot[i];
+    float *dst = nsum + 3 * (size_t)(leaf0 + leaf_of_slot[i]);
     atomicAdd(dst, fn.x); atomicAdd(dst + 1, fn.y); atomicAdd(dst + 2, fn.z);
 }
-__global__ void __launch_bounds__(256) k_up_normals(float *__restrict__ nsum, const int *__restrict__ cbegin, int count, int off,
-                                                    int off_child) {
+__global__ void __launch_bounds__(256) k_up_normals(float *__restrict__ nsum, const int2 *__restrict__ kids, int first, int count) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= count) return;
+    const int2 k = kids[first + j];
     float sx = 0.f, sy = 0.f, sz = 0.f;
-    for (int c = cbegin[j]; c < cbegin[j + 1]; ++c) {
-        const float *s = nsum + 3 * (size_t)(off_child + c);
+    for (int c = k.x; c < k.x + k.y; ++c) {
+        const float *s = nsum + 3 * (size_t)c;
         sx += s[0]; sy += s[1]; sz += s[2];
     }
-    float *d = nsum + 3 * (size_t)(off + j);
+    float *d = nsum + 3 * (size_t)(first + j);
     d[0] = sx; d[1] = sy; d[2] = sz;
 }
 
@@ -285,7 +290,7 @@ __global__ void k_node_frames(Box *__restrict__ boxes, const float *__restrict__
     b->b = make_float4(n.z, t1.z, NW_EMPTY_LO, NW_EMPTY_LO);
     // t2 = n x t1, exactly as project3 forms it
     b->c = make_float4(n.y * t1.z - n.z * t1.y, n.z * t1.x - n.x * t1.z, n.x * t1.y - n.y * t1.x, NW_EMPTY_HI);
-    b->d = make_float4(NW_EMPTY_HI, NW_EMPTY_HI, 0.f, NW_EMPTY_LO);      // d.z: the search's link, written by k_global_tables
+    b->d.x = NW_EMPTY_HI; b->d.y = NW_EMPTY_HI; b->d.w = NW_EMPTY_LO;      // d.z: the search's link, written by k_level_tables
 }
 
 // every iteration: intervals back to "empty" (frames are kept for the whole block)
@@ -299,14 +304,14 @@ __global__ void k_reset_extents(Box *__restrict__ boxes, int first, int count) {
 // every iteration: each centroid projects onto the frame of every ancestor; lanes of a warp that
 // share the node are reduced with REDUX first, then one ordered-int atomic min/max per quantity
 __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent, int F, const int *__restrict__ leaf_of_slot,
-                                                 const int *__restrict__ par, Box *__restrict__ boxes, TreeLevels tl) {
+                                                 int leaf0, int leaf_level, const int *__restrict__ parent_g, Box *__restrict__ boxes) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = i < F;
     const float4 c = live ? cent[i] : make_float4(0.f, 0.f, 0.f, 0.f);
     const bool finite = live && (c.x == c.x) && (c.y == c.y) && (c.z == c.z);
-    int node = live ? leaf_of_slot[i] : 0;
+    int node = live ? leaf0 + leaf_of_slot[i] : 0;
     const unsigned lane = threadIdx.x & 31;
-    for (int l = tl.n_levels - 1; l >= 1; --l) {
+    for (int l = leaf_level; l >= 1; --l) {
         // lanes that share the node: the slots are sorted by key, so equal nodes are runs of consecutive lanes -- run
         // heads from one shuffle and a ballot (match_any costs several times more)
         const int prev = __shfl_up_sync(0xffffffffu, node, 1);
@@ -315,7 +320,7 @@ __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent
         const int first = 31 - __clz(heads & upto);
         const unsigned above = heads & ~upto;
         const unsigned grp = (above ? ((1u << (__ffs(above) - 1)) - 1u) : 0xffffffffu) & ~((1u << first) - 1u);
-        Box *b = &boxes[tl.off[l] + node];
+        Box *b = &boxes[node];
         float p[3] = {0.f, 0.f, 0.f};
         if (live) {
             const float4 ba = b->a;
@@ -340,7 +345,7 @@ __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent
             if (u2ord(mn[2]) < __float_as_int(cd.w)) atomicMin((int *)&b->d.w, u2ord(mn[2]));
             if (u2ord(mx[2]) > __float_as_int(ch2)) atomicMax((int *)&b->c.w, u2ord(mx[2]));
         }
-        if (live) node = par[tl.off[l] + node] & 0x7fffffff;
+        if (live) node = parent_g[node] & 0x7fffffff;
     }
 }
 // ordered-int -> float for the extents written by k_extents.  The intervals are widened by the rounding slack of the
@@ -389,38 +394,6 @@ extern "C" int nw_set_topology_records(nw_ctx *h, const void *vertex_records, co
     return set_topology_impl(h, (const float *)vertex_records, nullptr, faces, nullptr, he_vertex, n_halfedges, nullptr, M, F, he_stride_bytes);
 }
 
-// The per-level tables (local indices, what the build and refit kernels use) rewritten with global node ids for the
-// search:  kids = {first child (global) or first slot, count};  parent_g = global parent | (the PARENT is the last child
-// of ITS parent) << 31, so that popping a level is one load;  and inside the node itself (Box::d.z) first child / first slot | (this node is a last child) << 31 -- what a search step needs next, whether the
-// node is pruned (next sibling or pop) or opened (first child), arrives with the box it has just loaded.
-__global__ void k_global_tables(const int *__restrict__ par, const int *__restrict__ cbegin_level, int count, int off, int off_parent,
-                                int off_child, bool is_leaf_level, int *__restrict__ parent_g, int2 *__restrict__ kids,
-                                Box *__restrict__ boxes) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= count) return;
-    const int pv = par[off + i];
-    const int p = (pv & 0x7fffffff) + off_parent;
-    const unsigned parent_last = off ? ((unsigned)par[p] & 0x80000000u) : 0x80000000u;
-    parent_g[off + i] = (int)((unsigned)p | parent_last);
-    const int c0 = cbegin_level[i], c1 = cbegin_level[i + 1];
-    const int first = is_leaf_level ? c0 : off_child + c0;
-    kids[off + i] = make_int2(first, c1 - c0);
-    boxes[off + i].d.z = __int_as_float((int)((unsigned)first | ((unsigned)pv & 0x80000000u)));
-}
-
-// NW_TRACE_BUILD=1: wall-clock checkpoints (with a stream sync each) through nw_tree_build, on stderr
-struct BuildTrace {
-    bool on; cudaStream_t s; std::chrono::steady_clock::time_point t;
-    BuildTrace(cudaStream_t s_) : on(getenv("NW_TRACE_BUILD") != nullptr), s(s_) { if (on) { cudaStreamSynchronize(s); t = std::chrono::steady_clock::now(); } }
-    void mark(const char *what) {
-        if (!on) return;
-        cudaStreamSynchronize(s);
-        auto n = std::chrono::steady_clock::now();
-        fprintf(stderr, "[nw build] %-22s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(n - t).count());
-        t = n;
-    }
-};
-
 // profiling: device time of the compute segments of an upload (the host->device copies between them are not counted)
 static int seg_begin(nw_ctx *h) {
     if (!(h->profile & 1)) return NW_OK;
@@ -454,7 +427,6 @@ static int set_topology_impl(nw_ctx *h, const float *pos, const float *nrm, cons
         const long long shape[7] = {M, F, n_he, records, valid != nullptr, he_vertex != nullptr, he_stride};
         NW_CHECK(nw_check_replicated(h, shape, 7, "nw_set_topology: mesh shape"));
     }
-    BuildTrace trace_up(s);
     NW_CHECK(seg_begin(h));
     NW_CHECK(nw_save_feet(h));       // seeds for the next block, taken from the mesh that is about to be replaced
     NW_CHECK(seg_end(h));
@@ -520,7 +492,6 @@ static int set_topology_impl(nw_ctx *h, const float *pos, const float *nrm, cons
     }
     }
     NW_CUDA(cudaStreamSynchronize(s));
-    trace_up.mark("feet + uploads + unpack");
     NW_CHECK(seg_begin(h));
     NW_CUDA(cudaMemsetAsync(h->acc, 0, sizeof(unsigned long long) * 4 * M, s));
     NW_CUDA(cudaMemsetAsync(h->Sq, 0, sizeof(float4) * 3 * M, s));
@@ -549,7 +520,8 @@ static int extents_pass(nw_ctx *h) {
     const int first = tl.off[1], count = tl.off[tl.n_levels - 1] + tl.count[tl.n_levels - 1] - first;
     k_reset_extents<<<nw_grid(count, B), B, 0, s>>>(h->boxes, first, count);
     NW_LAUNCH_CHECK();
-    k_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->cent, h->F, h->leaf_of_slot, h->par, h->boxes, tl);
+    k_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->cent, h->F, h->leaf_of_slot, tl.off[tl.n_levels - 1], tl.n_levels - 1, h->parent_g,
+                                             h->boxes);
     NW_LAUNCH_CHECK();
     k_box_decode<<<nw_grid(count, B), B, 0, s>>>(h->boxes, first, count, h->st);
     NW_LAUNCH_CHECK();
@@ -572,7 +544,6 @@ int nw_tree_refit(nw_ctx *h) {
 int nw_tree_build(nw_ctx *h) {
     cudaStream_t s = h->stream;
     const int B = 256, F = h->F;
-    BuildTrace trace(s);
     // build temporaries are members: reused from block to block (cudaFree synchronises and is slow)
     int *&d_bbox = h->tb_small, *&idx = h->tb_i0, *&order = h->tb_i1;
     unsigned *&keys = h->tb_u0, *&keys2 = h->tb_u1;
@@ -583,7 +554,6 @@ int nw_tree_build(nw_ctx *h) {
     int bb[6];
     NW_CUDA(cudaMemcpyAsync(bb, d_bbox, sizeof(bb), cudaMemcpyDeviceToHost, s));
     NW_CUDA(cudaStreamSynchronize(s));
-    trace.mark("face bbox");
     float lo[3], hi[3];
     for (int a = 0; a < 3; ++a) { lo[a] = ordered_to_float(bb[a]); hi[a] = ordered_to_float(bb[3 + a]); }
     float ext = fmaxf(fmaxf(hi[0] - lo[0], hi[1] - lo[1]), hi[2] - lo[2]);
@@ -604,7 +574,6 @@ int nw_tree_build(nw_ctx *h) {
     h->key_lo[0] = lo[0]; h->key_lo[1] = lo[1]; h->key_lo[2] = lo[2]; h->key_inv = inv;
     k_sorted_faces<<<nw_grid(F, B), B, 0, s>>>(h->faces, order, F, h->sfaces, cells, h->fcells);
     h->launches += 7;
-    trace.mark("keys + sort");
 
     // ---- level sizes: nodes of level k = distinct 3k-bit key prefixes; leaf level = deepest with >= 4 centroids per node
     int *hist = d_bbox;                                   // 16 ints
@@ -613,20 +582,18 @@ int nw_tree_build(nw_ctx *h) {
     int hh[16];
     NW_CUDA(cudaMemcpyAsync(hh, hist, sizeof(hh), cudaMemcpyDeviceToHost, s));
     NW_CUDA(cudaStreamSynchronize(s));
-    trace.mark("level histogram");
     int cnt[11];
     cnt[0] = 1;
     for (int k = 1; k <= 10; ++k) cnt[k] = cnt[k - 1] + hh[k];
     int kL = 1;
-    double occ = 3.0;                                     // mean centroids per leaf cell, at least (measured at C3 with the packet search, blocks 0/1/2 of a fit: 1 -> 17.4/2.45/2.27 ms, 1.5 -> 13.6/2.27/2.19, 3 -> 12.1/2.27/2.09, 6 -> 12.3/2.58/2.45, 12 -> 13.4/2.59/2.43)
-    if (const char *e = getenv("NW_LEAF_OCC")) occ = atof(e);
+    const double occ = 3.0;                               // mean centroids per leaf cell, at least (measured at C3 with the packet search, blocks 0/1/2 of a fit: 1 -> 17.4/2.45/2.27 ms, 1.5 -> 13.6/2.27/2.19, 3 -> 12.1/2.27/2.09, 6 -> 12.3/2.58/2.45, 12 -> 13.4/2.59/2.43)
     for (int k = 1; k <= 10; ++k) if ((double)F / cnt[k] >= occ) kL = k;
     TreeLevels &tl = h->tl;
     tl.n_levels = kL + 1;
-    int off = 0, cb = 0;
+    int off = 0;
     for (int k = 0; k <= kL; ++k) {
-        tl.count[k] = cnt[k]; tl.off[k] = off; tl.cb_off[k] = cb;
-        off += cnt[k]; cb += cnt[k] + 1;
+        tl.count[k] = cnt[k]; tl.off[k] = off;
+        off += cnt[k];
     }
     const int total = off;
     // the node count follows the shape of the mesh: the leaf level can change from one block to the next, which changes
@@ -634,52 +601,38 @@ int nw_tree_build(nw_ctx *h) {
     // and, for a surface, a third of that above them (0.9 F in all; 1.33 F if the levels only double), so 1.5 F nodes is
     // a size that depends on the topology alone.
     const size_t room = std::max((size_t)total + total / 4, (size_t)F + F / 2) + 64;
-    NW_CHECK(nw_alloc(h, &h->boxes, room)); NW_CHECK(nw_alloc(h, &h->par, room));
-    NW_CHECK(nw_alloc(h, &h->cbegin, room + NW_MAX_LEVELS + 1)); NW_CHECK(nw_alloc(h, &h->leaf_of_slot, (size_t)F));
+    NW_CHECK(nw_alloc(h, &h->boxes, room)); NW_CHECK(nw_alloc(h, &h->parent_g, room)); NW_CHECK(nw_alloc(h, &h->kids, room));
+    NW_CHECK(nw_alloc(h, &h->leaf_of_slot, (size_t)F));
     NW_CHECK(nw_alloc(h, &h->node_f, (size_t)NW_NMOM * room));
-    trace.mark("allocations");
-    // ---- per-level tables
-    int *flag = idx, *id_cur = order, *id_prev = (int *)keys, *start = (int *)keys2;     // reuse the sort buffers (F ints each)
+    // ---- tables: level k is numbered (flags, scan), then the level above it is linked to it; the leaf level last
+    // reuse the sort buffers (F ints each; cells is no longer needed once k_sorted_faces has run)
+    int *flag = idx, *id_cur = order, *id_prev = (int *)keys, *start_cur = (int *)keys2, *start_prev = (int *)cells;
     for (int k = 0; k <= kL; ++k) {
         k_level_flags<<<nw_grid(F, B), B, 0, s>>>(h->fkeys, F, 30 - 3 * k, flag);
         NW_LAUNCH_CHECK();
         NW_CHECK(scan_inclusive(h, flag, id_cur, F));
-        k_level_tables<<<nw_grid(F, B), B, 0, s>>>(flag, id_cur, k ? id_prev : nullptr, F, start, h->par + tl.off[k],
-                                                   k ? h->cbegin + tl.cb_off[k - 1] : nullptr);
-        NW_LAUNCH_CHECK();
-        if (k) NW_CUDA(cudaMemcpyAsync(h->cbegin + tl.cb_off[k - 1] + tl.count[k - 1], &tl.count[k], sizeof(int), cudaMemcpyHostToDevice, s));
-        if (k == kL) {
-            NW_CUDA(cudaMemcpyAsync(h->cbegin + tl.cb_off[k], start, sizeof(int) * tl.count[k], cudaMemcpyDeviceToDevice, s));
-            NW_CUDA(cudaMemcpyAsync(h->cbegin + tl.cb_off[k] + tl.count[k], &h->F, sizeof(int), cudaMemcpyHostToDevice, s));
-            k_copy_minus1<<<nw_grid(F, B), B, 0, s>>>(id_cur, F, h->leaf_of_slot);
-            NW_LAUNCH_CHECK();
-        }
-        k_mark_last_child<<<nw_grid(tl.count[k], B), B, 0, s>>>(h->par + tl.off[k], tl.count[k]);
+        k_level_tables<<<nw_grid(F, B), B, 0, s>>>(h->fkeys, F, k - 1, k ? tl.off[k - 1] : 0, id_prev, start_prev, tl.off[k], id_cur,
+                                                   start_cur, h->parent_g, h->kids, h->boxes, h->leaf_of_slot);
         NW_LAUNCH_CHECK();
         std::swap(id_cur, id_prev);
+        std::swap(start_cur, start_prev);
     }
-    trace.mark("level tables");
+    k_level_tables<<<nw_grid(F, B), B, 0, s>>>(h->fkeys, F, kL, tl.off[kL], id_prev, start_prev, 0, nullptr, nullptr, h->parent_g,
+                                               h->kids, h->boxes, h->leaf_of_slot);
+    NW_LAUNCH_CHECK();
     // ---- frames (fixed for the block), then the first extents
     launch_refit_centroids(h);
     NW_LAUNCH_CHECK();
     NW_CUDA(cudaMemsetAsync(h->node_f, 0, sizeof(float) * NW_NMOM * total, s));
-    k_leaf_normals<<<nw_grid(F, B), B, 0, s>>>(h->sfaces, h->posq, F, h->leaf_of_slot, h->node_f + (size_t)NW_NMOM * tl.off[kL]);
+    k_leaf_normals<<<nw_grid(F, B), B, 0, s>>>(h->sfaces, h->posq, F, h->leaf_of_slot, tl.off[kL], h->node_f);
     NW_LAUNCH_CHECK();
     for (int k = kL - 1; k >= 0; --k) {
-        k_up_normals<<<nw_grid(tl.count[k], B), B, 0, s>>>(h->node_f, h->cbegin + tl.cb_off[k], tl.count[k], tl.off[k], tl.off[k + 1]);
+        k_up_normals<<<nw_grid(tl.count[k], B), B, 0, s>>>(h->node_f, h->kids, tl.off[k], tl.count[k]);
         NW_LAUNCH_CHECK();
     }
     k_node_frames<<<nw_grid(total, B), B, 0, s>>>(h->boxes, h->node_f, 0, total);
     NW_LAUNCH_CHECK();
-    NW_CHECK(nw_alloc(h, &h->parent_g, room)); NW_CHECK(nw_alloc(h, &h->kids, room));
-    for (int k = 0; k <= kL; ++k) {
-        k_global_tables<<<nw_grid(tl.count[k], B), B, 0, s>>>(h->par, h->cbegin + tl.cb_off[k], tl.count[k], tl.off[k], k ? tl.off[k - 1] : 0,
-                                                              k < kL ? tl.off[k + 1] : 0, k == kL, h->parent_g, h->kids, h->boxes);
-        NW_LAUNCH_CHECK();
-    }
-    trace.mark("normals + frames");
     NW_CHECK(extents_pass(h));
-    trace.mark("extents");
     return NW_OK;
 }
 

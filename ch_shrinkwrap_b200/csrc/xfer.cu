@@ -6,12 +6,9 @@
 // pinned 4 MB buffers of its own and issues the DMA on its own stream, so the host memcpy of one piece overlaps the DMA of
 // the previous one and the lanes add up to PCIe rate.  On return the source has been read completely (the caller may
 // free it) and the handle's stream waits for every lane.
-#include <chrono>
-#include <cstdio>
 #include <thread>
 #include <vector>
 #include <cstring>
-#include <cstdlib>
 #include <algorithm>
 #include "common.cuh"
 
@@ -31,9 +28,7 @@ struct nw_uploader {
 
 static int uploader_init(nw_ctx *h) {
     if (h->uploader) return NW_OK;
-    int n = 0;
-    if (const char *e = getenv("NW_UPLOAD_THREADS")) n = atoi(e);
-    if (n <= 0) n = (int)std::min(8u, std::max(1u, std::thread::hardware_concurrency() / 2));
+    const int n = (int)std::min(8u, std::max(1u, std::thread::hardware_concurrency() / 2));
     nw_uploader *u = new nw_uploader;
     u->lanes.resize(n);
     h->uploader = u;                      // owned by the handle from here on (nw_uploader_destroy releases partial state)
@@ -150,8 +145,6 @@ int nw_h2d_strided32(nw_ctx *h, void *dst, const void *src, size_t bytes, size_t
         NW_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->stream));
         return NW_OK;
     }
-    static const bool trace = getenv("NW_TRACE_BUILD") != nullptr;
-    auto T0 = std::chrono::steady_clock::now();
     NW_CHECK(uploader_init(h));
     nw_uploader *u = h->uploader;
     NW_CUDA(cudaEventRecord(u->ev_start, h->stream));
@@ -167,13 +160,7 @@ int nw_h2d_strided32(nw_ctx *h, void *dst, const void *src, size_t bytes, size_t
         if (t == n_lanes - 1) lane_copy(h->device, u, &u->lanes[t], (char *)dst, (const char *)src, a, b - a, stride);   // caller's thread takes the last range
         else th.emplace_back(lane_copy, h->device, u, &u->lanes[t], (char *)dst, (const char *)src, a, b - a, stride);
     }
-    auto T1 = std::chrono::steady_clock::now();
     for (auto &t : th) t.join();
-    if (trace) {
-        auto T2 = std::chrono::steady_clock::now();
-        fprintf(stderr, "[nw h2d] %8.1f MB  own lane %7.3f ms  join %7.3f ms\n", bytes / 1048576.0,
-                std::chrono::duration<double, std::milli>(T1 - T0).count(), std::chrono::duration<double, std::milli>(T2 - T1).count());
-    }
     for (int t = 0; t < n_lanes; ++t) {
         UploadLane &l = u->lanes[t];
         if (l.err != cudaSuccess) { h->err = std::string("nw_h2d: ") + cudaGetErrorString(l.err); return NW_ERR_CUDA; }
