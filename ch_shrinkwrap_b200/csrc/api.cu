@@ -50,6 +50,8 @@ extern "C" void nw_destroy(nw_ctx *h) {
     nw_free(&h->rx); nw_free(&h->ry); nw_free(&h->rz);
     nw_free(&h->posq); nw_free(&h->nrmq); nw_free(&h->faces); nw_free(&h->nbrT); nw_free(&h->valence); nw_free(&h->valid); nw_free(&h->stage_nbr); nw_free(&h->stage_hev); nw_free(&h->tb_small); nw_free(&h->tb_i0); nw_free(&h->tb_i1); nw_free(&h->tb_u0); nw_free(&h->tb_u1); nw_free(&h->tb_u2); nw_free(&h->fcells); nw_free(&h->cent64); nw_free(&h->parent_g); nw_free(&h->kids);
     nw_free(&h->sfaces); nw_free(&h->cent); nw_free(&h->boxes); nw_free(&h->leaf_of_slot); nw_free(&h->node_f);
+    nw_free(&h->tboxes); nw_free(&h->surf_q); nw_free(&h->surf_bits); nw_free(&h->surf_dist); nw_free(&h->surf_closest);
+    nw_free(&h->surf_part); nw_free(&h->surf_face);
     nw_free(&h->acc); nw_free(&h->Sq); nw_free(&h->fdef);
     nw_free(&h->partials); nw_free(&h->st); nw_free(&h->hist);
     nw_free((char **)&h->cub_tmp); nw_free(&h->scratchM); nw_free(&h->scratchP);

@@ -135,6 +135,12 @@ struct nw_ctx {
     unsigned *fcells = nullptr;                  // per sorted slot: grid cell of the centroid at upload time, x | y << 10 | z << 20
     bool points_mode = false;                    // the "faces" are raw target points (nw_set_point_targets): centroid = the point itself
     double *cent64 = nullptr;                    // points mode with float64 targets: exact coordinates per sorted slot (3 doubles)
+    // ---- nw_surface_distance (surface.cu): only that call reads or writes these ----
+    Box *tboxes = nullptr;                       // per global node id: the frames and links of `boxes`, intervals over face CORNERS
+    char *surf_q = nullptr;                      // copy of explicit queries
+    unsigned *surf_bits = nullptr;               // per-axis max |coordinate| of vertices and queries (rounding slack of the call)
+    double *surf_dist = nullptr, *surf_closest = nullptr, *surf_part = nullptr;
+    int *surf_face = nullptr;
     // ---- solver vectors ----
     unsigned long long *acc = nullptr;           // (M,4) int64 fixed point: AH res xyz, AH 1
     float4 *Sq = nullptr;                        // search directions, interleaved: S_k of vertex v at Sq[3v + k] (48 B per vertex)

@@ -1,0 +1,466 @@
+// surface.cu -- exact distance from query points to the handle's triangle mesh (nw_surface_distance).
+//
+// The fit's nearest-face search measures distances to face CENTROIDS (mesh_conj_grad.py:451-454); this file measures the
+// Euclidean distance to the closed triangles.  It walks the same octree of Hilbert cells (tree.cu: kids, parent_g,
+// leaf_of_slot, the frames of the node boxes), but against a second array of boxes, h->tboxes, whose intervals cover the
+// three CORNERS of every face below the node instead of its centroid.  Those intervals are re-measured at the start of
+// every call from the current positions, so they are never stale; h->boxes, cent, the seeds and the iteration graph are
+// only read.
+//
+// Exactness: every candidate face's distance is evaluated in fp64 (corners widened exactly from float32, queries in
+// float32 widened exactly or in float64) by one fixed sequence of operations, Ericson's closest-point region test
+// (Real-Time Collision Detection, 5.1.5).  This file is compiled with -fmad=false so that the compiler performs exactly the
+// written operations: tests/surface_oracle.py (closest_point_triangle) restates them in numpy and gets the same bits.
+// Ties of the fp64 squared distance go to the lowest face index.  The box test only prunes: its float32 lower bound is
+// made conservative by the rounding slack of the call (below), so it can never discard the true minimum.
+#include <cfloat>
+#include <cmath>
+#include "common.cuh"
+
+namespace {
+
+__device__ __forceinline__ int f2ord(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
+__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
+__device__ __forceinline__ unsigned f2u(float f) { return (unsigned)f2ord(f) ^ 0x80000000u; }      // order-preserving float -> unsigned
+__device__ __forceinline__ int u2ord(unsigned u) { return (int)(u ^ 0x80000000u); }
+#define NW_EMPTY_LO __int_as_float(f2ord(FLT_MAX))      // ordered-int encodings of an empty interval
+#define NW_EMPTY_HI __int_as_float(f2ord(-FLT_MAX))
+
+// projection onto a node frame as the box stores it (t2 = c.xyz): the operations of the search's node test (sweep.cu)
+__device__ __forceinline__ void project_frame(const float4 a, const float4 b, const float4 c, float x, float y, float z, float &pn,
+                                              float &p1, float &p2) {
+    pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
+    p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
+    p2 = fmaf(c.x, x, fmaf(c.y, y, c.z * z));
+}
+
+// ---- rounding slack of the call -----------------------------------------------------------------------------------
+// per-axis max |coordinate| over the finite values, as the bits of non-negative floats (which order like unsigned ints)
+__device__ __forceinline__ float abs_up(float v) { return fabsf(v); }
+__device__ __forceinline__ float abs_up(double v) { return __double2float_ru(fabs(v)); }
+template <typename T>
+__global__ void __launch_bounds__(256) k_absmax3(const T *__restrict__ x, const T *__restrict__ y, const T *__restrict__ z, int64_t n,
+                                                 int64_t stride, unsigned *__restrict__ out3) {
+    float m[3] = {0.f, 0.f, 0.f};
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float v[3] = {abs_up(x[i * stride]), abs_up(y[i * stride]), abs_up(z[i * stride])};
+        for (int k = 0; k < 3; ++k) if (v[k] <= FLT_MAX) m[k] = fmaxf(m[k], v[k]);
+    }
+    for (int k = 0; k < 3; ++k) {
+        const unsigned r = __reduce_max_sync(0xffffffffu, __float_as_uint(m[k]));
+        if ((threadIdx.x & 31) == 0 && r) atomicMax(out3 + k, r);
+    }
+}
+// The slack of the box test: 2^-19 x the L1 bound of everything that is projected (the vertices, bits 0..2, and the queries,
+// bits 3..5) -- the rule of tree.cu's k_box_decode, whose coord_l1 covers the fit's vertices and points only.  Queries given
+// explicitly can lie much farther out than either.
+__device__ __forceinline__ float call_slack(const unsigned *__restrict__ bits6) {
+    float l1 = 0.f;
+    for (int k = 0; k < 3; ++k) l1 += fmaxf(__uint_as_float(bits6[k]), __uint_as_float(bits6[3 + k]));
+    return l1 * 1.9073486328125e-6f;
+}
+
+// ---- triangle-bounded boxes ------------------------------------------------------------------------------------------
+// frames and search links of h->boxes, intervals empty
+__global__ void k_tbox_init(const Box *__restrict__ boxes, int n, Box *__restrict__ tb) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const Box s = boxes[j];
+    Box t;
+    t.a = s.a;
+    t.b = make_float4(s.b.x, s.b.y, NW_EMPTY_LO, NW_EMPTY_LO);
+    t.c = make_float4(s.c.x, s.c.y, s.c.z, NW_EMPTY_HI);
+    t.d = make_float4(NW_EMPTY_HI, NW_EMPTY_HI, s.d.z, NW_EMPTY_LO);
+    tb[j] = t;
+}
+
+// k_extents (tree.cu) with the three corners of each face in place of its centroid: every face projects its corners onto the
+// frame of every ancestor; lanes of a warp that share the node are reduced first, then one ordered-int atomic per quantity.
+// A face with a non-finite corner contributes nothing (the query kernel skips it too).
+__global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sfaces, const float4 *__restrict__ pos, int F,
+                                                     const int *__restrict__ leaf_of_slot, int leaf0, int leaf_level,
+                                                     const int *__restrict__ parent_g, Box *__restrict__ boxes) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = i < F;
+    float4 v[3] = {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)};
+    bool finite = live;
+    if (live) {
+        const int4 sf = sfaces[i];
+        v[0] = pos[sf.x]; v[1] = pos[sf.y]; v[2] = pos[sf.z];
+        for (int k = 0; k < 3; ++k) finite = finite && fabsf(v[k].x) <= FLT_MAX && fabsf(v[k].y) <= FLT_MAX && fabsf(v[k].z) <= FLT_MAX;
+    }
+    int node = live ? leaf0 + leaf_of_slot[i] : 0;
+    const unsigned lane = threadIdx.x & 31;
+    for (int l = leaf_level; l >= 1; --l) {
+        const int prev = __shfl_up_sync(0xffffffffu, node, 1);
+        const unsigned heads = __ballot_sync(0xffffffffu, lane == 0 || prev != node || !live);
+        const unsigned upto = 0xffffffffu >> (31 - lane);
+        const int first = 31 - __clz(heads & upto);
+        const unsigned above = heads & ~upto;
+        const unsigned grp = (above ? ((1u << (__ffs(above) - 1)) - 1u) : 0xffffffffu) & ~((1u << first) - 1u);
+        Box *b = &boxes[node];
+        float lo[3] = {0.f, 0.f, 0.f}, hi[3] = {0.f, 0.f, 0.f};
+        if (live) {
+            const float4 ba = b->a, bb = b->b, bc = b->c;
+            project_frame(ba, bb, bc, v[0].x, v[0].y, v[0].z, lo[0], lo[1], lo[2]);
+            hi[0] = lo[0]; hi[1] = lo[1]; hi[2] = lo[2];
+            for (int c = 1; c < 3; ++c) {
+                float p[3];
+                project_frame(ba, bb, bc, v[c].x, v[c].y, v[c].z, p[0], p[1], p[2]);
+                for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], p[k]); hi[k] = fmaxf(hi[k], p[k]); }
+            }
+        }
+        unsigned mn[3], mx[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            mn[k] = __reduce_min_sync(grp, finite ? f2u(lo[k]) : 0xffffffffu);
+            mx[k] = __reduce_max_sync(grp, finite ? f2u(hi[k]) : 0u);
+        }
+        if (live && lane == (unsigned)first && mn[0] <= mx[0]) {
+            const float4 cb = __ldcg(&b->b), cd = __ldcg(&b->d);
+            const float ch2 = __ldcg(&b->c.w);
+            if (u2ord(mn[0]) < __float_as_int(cb.z)) atomicMin((int *)&b->b.z, u2ord(mn[0]));
+            if (u2ord(mx[0]) > __float_as_int(cd.x)) atomicMax((int *)&b->d.x, u2ord(mx[0]));
+            if (u2ord(mn[1]) < __float_as_int(cb.w)) atomicMin((int *)&b->b.w, u2ord(mn[1]));
+            if (u2ord(mx[1]) > __float_as_int(cd.y)) atomicMax((int *)&b->d.y, u2ord(mx[1]));
+            if (u2ord(mn[2]) < __float_as_int(cd.w)) atomicMin((int *)&b->d.w, u2ord(mn[2]));
+            if (u2ord(mx[2]) > __float_as_int(ch2)) atomicMax((int *)&b->c.w, u2ord(mx[2]));
+        }
+        if (live) node = parent_g[node] & 0x7fffffff;
+    }
+}
+
+// ordered-int -> float, widened by the slack of the call (k_box_decode's rule)
+__global__ void k_tbox_decode(Box *__restrict__ tb, int first, int count, const unsigned *__restrict__ bits6) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    const float w = call_slack(bits6);
+    Box *b = &tb[first + i];
+    b->b.z = ord2f(__float_as_int(b->b.z)) - w; b->d.x = ord2f(__float_as_int(b->d.x)) + w;
+    b->b.w = ord2f(__float_as_int(b->b.w)) - w; b->d.y = ord2f(__float_as_int(b->d.y)) + w;
+    b->d.w = ord2f(__float_as_int(b->d.w)) - w; b->c.w = ord2f(__float_as_int(b->c.w)) + w;
+}
+
+// ---- exact point-to-triangle distance (fp64, fixed operation order; restated in tests/surface_oracle.py) -------------------
+struct D3 { double x, y, z; };
+__device__ __forceinline__ D3 d3(const float4 v) { return D3{(double)v.x, (double)v.y, (double)v.z}; }
+__device__ __forceinline__ D3 sub(const D3 a, const D3 b) { return D3{a.x - b.x, a.y - b.y, a.z - b.z}; }
+__device__ __forceinline__ double dot(const D3 a, const D3 b) { return (a.x * b.x + a.y * b.y) + a.z * b.z; }
+__device__ __forceinline__ D3 axpy(const D3 a, const double t, const D3 e) { return D3{a.x + t * e.x, a.y + t * e.y, a.z + t * e.z}; }
+__device__ __forceinline__ double dist2(const D3 p, const D3 c) { const D3 d = sub(p, c); return dot(d, d); }
+
+__device__ __forceinline__ D3 closest_on_segment(const D3 p, const D3 p0, const D3 p1) {
+    const D3 e = sub(p1, p0);
+    const double ee = dot(e, e);
+    double t = ee > 0.0 ? dot(sub(p, p0), e) / ee : 0.0;
+    t = fmin(fmax(t, 0.0), 1.0);
+    return axpy(p0, t, e);
+}
+// a zero-area triangle is the union of its three edges: the closest of them, in the order ab, bc, ca (first wins ties)
+__device__ __noinline__ D3 closest_on_edges(const D3 p, const D3 a, const D3 b, const D3 c) {
+    D3 best = closest_on_segment(p, a, b);
+    double bd = dist2(p, best);
+    D3 k = closest_on_segment(p, b, c);
+    double kd = dist2(p, k);
+    if (kd < bd) { best = k; bd = kd; }
+    k = closest_on_segment(p, c, a);
+    kd = dist2(p, k);
+    if (kd < bd) best = k;
+    return best;
+}
+// Ericson's region test.  Degenerate: the cross product ab x ac is exactly zero, or (rounding of a nearly degenerate
+// triangle) the interior case finds no positive barycentric denominator.
+__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c) {
+    const D3 ab = sub(b, a), ac = sub(c, a);
+    if (ab.y * ac.z - ab.z * ac.y == 0.0 && ab.z * ac.x - ab.x * ac.z == 0.0 && ab.x * ac.y - ab.y * ac.x == 0.0)
+        return closest_on_edges(p, a, b, c);
+    const D3 ap = sub(p, a);
+    const double d1 = dot(ab, ap), d2 = dot(ac, ap);
+    if (d1 <= 0.0 && d2 <= 0.0) return a;
+    const D3 bp = sub(p, b);
+    const double d3 = dot(ab, bp), d4 = dot(ac, bp);
+    if (d3 >= 0.0 && d4 <= d3) return b;
+    const double vc = d1 * d4 - d3 * d2;
+    if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) return axpy(a, d1 / (d1 - d3), ab);
+    const D3 cp = sub(p, c);
+    const double d5 = dot(ab, cp), d6 = dot(ac, cp);
+    if (d6 >= 0.0 && d5 <= d6) return c;
+    const double vb = d5 * d2 - d1 * d6;
+    if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) return axpy(a, d2 / (d2 - d6), ac);
+    const double va = d3 * d6 - d5 * d4;
+    if (va <= 0.0 && (d4 - d3) >= 0.0 && (d5 - d6) >= 0.0) return axpy(b, (d4 - d3) / ((d4 - d3) + (d5 - d6)), sub(c, b));
+    const double s = va + vb + vc;
+    if (!(s > 0.0)) return closest_on_edges(p, a, b, c);
+    const double denom = 1.0 / s;
+    const double v = vb * denom, w = vc * denom;
+    return D3{(a.x + ab.x * v) + ac.x * w, (a.y + ab.y * v) + ac.y * w, (a.z + ab.z * v) + ac.z * w};
+}
+
+__device__ __forceinline__ bool finite4(const float4 v) { return fabsf(v.x) <= FLT_MAX && fabsf(v.y) <= FLT_MAX && fabsf(v.z) <= FLT_MAX; }
+
+// ---- the walk ------------------------------------------------------------------------------------------------------
+struct SurfaceArgs {
+    int64_t Q;
+    const void *qx, *qy, *qz;           // query coordinates (float or double): element i at q?[i * stride]
+    int64_t stride;
+    const int *perm;                    // resident points: sorted position -> caller's index (NULL: the identity)
+    const int *seed;                    // resident points: nearest-centroid slot of the last sweep, or -1 (NULL: none)
+    const Box *tb;
+    const int *parent;
+    const int2 *kids;
+    const int *leaf_of_slot;
+    const int4 *sfaces;
+    const float4 *posq;
+    int leaf0, leaf_level, n_nodes, F;
+    double *dist;                       // caller order; always written
+    int *face;                          // or NULL
+    double *closest;                    // or NULL
+};
+
+// One query per thread, stackless: first child and next sibling come from the tables the fit's search uses (tree.cu).
+struct SurfaceWalk {
+    const SurfaceArgs &a;
+    float x, y, z;                      // float32 rounding of the query: the box tests use it
+    float eq;                           // how far the float32 rounding can lie from the query (0 for float32 queries)
+    D3 p;                               // the query, exactly
+    double d2 = DBL_MAX * 2.0;          // best squared distance (+inf: none yet)
+    float ub = FLT_MAX * 2.0f;          // d2 rounded up, times the 1.1e-5 the float32 frames owe to orthonormality
+    int face = 0x7fffffff, slot = -1;
+
+    __device__ __forceinline__ SurfaceWalk(const SurfaceArgs &a_) : a(a_) {}
+    __device__ __forceinline__ void offer(double v, int f, int s) {
+        if (v < d2 || (v == d2 && f < face)) { d2 = v; face = f; slot = s; ub = __fmul_ru(__double2float_ru(v), 1.000011f); }
+    }
+    // lower bound of the squared distance from the query to anything in the node (sweep.cu: Traversal::test_node, with the
+    // gaps shrunk by eq), compared with the best so far; `link` = the node's first child | last-child bit
+    __device__ __forceinline__ bool open(int node, int &link) const {
+        NW_ASSERT(node >= 0 && node < a.n_nodes);
+        const Box *bp = &a.tb[node];
+        const float4 ba = __ldg(&bp->a), bb = __ldg(&bp->b), bd = __ldg(&bp->d);
+        link = __float_as_int(bd.z);
+        const float pn = fmaf(ba.x, x, fmaf(ba.z, y, bb.x * z));
+        const float p1 = fmaf(ba.y, x, fmaf(ba.w, y, bb.y * z));
+        const float g0 = fmaxf(fmaxf(bb.z - pn, pn - bd.x) - eq, 0.f), g1 = fmaxf(fmaxf(bb.w - p1, p1 - bd.y) - eq, 0.f);
+        const float s01 = __fmaf_rd(g1, g1, __fmul_rd(g0, g0));
+        if (!(s01 <= ub)) return false;
+        const float4 bc = __ldg(&bp->c);
+        const float p2 = fmaf(bc.x, x, fmaf(bc.y, y, bc.z * z));
+        const float g2 = fmaxf(fmaxf(bd.w - p2, p2 - bc.w) - eq, 0.f);
+        return __fmaf_rd(g2, g2, s01) <= ub;
+    }
+    __device__ __forceinline__ void leaf(int node) {
+        NW_ASSERT(node >= a.leaf0 && node < a.n_nodes);
+        const int2 k = __ldg(&a.kids[node]);
+        NW_ASSERT(k.x >= 0 && k.y >= 0 && k.x + k.y <= a.F);
+        for (int s = k.x; s < k.x + k.y; ++s) {
+            const int4 sf = __ldg(&a.sfaces[s]);
+            const float4 va = __ldg(&a.posq[sf.x]), vb = __ldg(&a.posq[sf.y]), vc = __ldg(&a.posq[sf.z]);
+            if (!(finite4(va) && finite4(vb) && finite4(vc))) continue;
+            offer(dist2(p, closest_on_triangle(p, d3(va), d3(vb), d3(vc))), sf.w, s);
+        }
+    }
+    __device__ __forceinline__ void subtree(int I) {
+        int node = I;
+        while (true) {
+            int link;
+            if (open(node, link)) {
+                if (node >= a.leaf0) leaf(node);
+                else { node = link & 0x7fffffff; continue; }
+            }
+            while (true) {
+                if (node == I) return;
+                if (link >= 0) { ++node; break; }
+                link = __ldg(&a.parent[node]);
+                node = link & 0x7fffffff;
+            }
+        }
+    }
+    // greedy descent to a first leaf for a query without a seed (sweep.cu: node_score)
+    __device__ __forceinline__ int greedy_leaf() const {
+        int node = 0;
+        while (node < a.leaf0) {
+            const int2 k = __ldg(&a.kids[node]);
+            int pick = k.x;
+            float bl = FLT_MAX * 2.0f;
+            for (int ch = k.x; ch < k.x + k.y; ++ch) {
+                const Box *bp = &a.tb[ch];
+                const float4 ba = __ldg(&bp->a), bb = __ldg(&bp->b), bc = __ldg(&bp->c), bd = __ldg(&bp->d);
+                float pn, p1, p2;
+                project_frame(ba, bb, bc, x, y, z, pn, p1, p2);
+                const float g0 = fmaxf(fmaxf(bb.z - pn, pn - bd.x), 0.f), g1 = fmaxf(fmaxf(bb.w - p1, p1 - bd.y), 0.f),
+                            g2 = fmaxf(fmaxf(bd.w - p2, p2 - bc.w), 0.f);
+                const float c0 = pn - 0.5f * (bb.z + bd.x), c1 = p1 - 0.5f * (bb.w + bd.y), c2 = p2 - 0.5f * (bd.w + bc.w);
+                const float l = (g0 * g0 + g1 * g1 + g2 * g2) + 1e-4f * (c0 * c0 + c1 * c1 + c2 * c2);
+                if (l < bl) { bl = l; pick = ch; }
+            }
+            node = pick;
+        }
+        return node;
+    }
+    // the leaf first, then at every level the sibling subtrees of the path to the root
+    __device__ __forceinline__ void from_leaf(int node) {
+        leaf(node);
+        for (int level = a.leaf_level; level >= 1; --level) {
+            const int p = __ldg(&a.parent[node]) & 0x7fffffff;
+            const int2 k = __ldg(&a.kids[p]);
+            for (int sib = k.x; sib < k.x + k.y; ++sib)
+                if (sib != node) subtree(sib);
+            node = p;
+        }
+    }
+};
+
+__device__ __forceinline__ float rn_f32(float v) { return v; }
+__device__ __forceinline__ float rn_f32(double v) { return __double2float_rn(v); }
+
+template <typename T>
+__global__ void __launch_bounds__(128) k_surface_nearest(const __grid_constant__ SurfaceArgs a) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= a.Q) return;
+    const T qx = ((const T *)a.qx)[i * a.stride], qy = ((const T *)a.qy)[i * a.stride], qz = ((const T *)a.qz)[i * a.stride];
+    const int64_t o = a.perm ? (int64_t)a.perm[i] : i;
+    SurfaceWalk w(a);
+    w.p = D3{(double)qx, (double)qy, (double)qz};
+    w.x = rn_f32(qx); w.y = rn_f32(qy); w.z = rn_f32(qz);
+    // |n . (q - q32)| <= |q - q32|_1 <= half an ulp per coordinate <= L1(q32) 2^-24: shrink every gap by twice that
+    w.eq = sizeof(T) == 8 ? fmaf(fabsf(w.x) + fabsf(w.y) + fabsf(w.z), 1.1920928955078125e-7f, FLT_MIN) : 0.f;
+    if (fabs(w.p.x) <= DBL_MAX && fabs(w.p.y) <= DBL_MAX && fabs(w.p.z) <= DBL_MAX) {
+        const int s = a.seed ? __ldg(&a.seed[i]) : -1;
+        w.from_leaf(s >= 0 && s < a.F ? a.leaf0 + __ldg(&a.leaf_of_slot[s]) : w.greedy_leaf());
+    }
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    D3 c = D3{nan, nan, nan};
+    if (w.slot >= 0) {
+        const int4 sf = __ldg(&a.sfaces[w.slot]);
+        c = closest_on_triangle(w.p, d3(__ldg(&a.posq[sf.x])), d3(__ldg(&a.posq[sf.y])), d3(__ldg(&a.posq[sf.z])));
+    }
+    a.dist[o] = w.slot >= 0 ? sqrt(w.d2) : nan;
+    if (a.face) a.face[o] = w.slot >= 0 ? w.face : -1;
+    if (a.closest) { a.closest[3 * o] = c.x; a.closest[3 * o + 1] = c.y; a.closest[3 * o + 2] = c.z; }
+}
+
+// ---- summary: max, mean and RMS of the distances, in a fixed order ------------------------------------------------------
+// Thread t of block b takes the entries b*256 + t + k*256*G in increasing k, then fixed trees; the result does not depend on
+// scheduling.  Non-finite distances (non-finite queries, or a mesh without one finite face) are left out.
+#define NW_SUM_BLOCKS 256
+__global__ void __launch_bounds__(256) k_dist_partials(const double *__restrict__ d, int64_t n, double *__restrict__ part) {
+    __shared__ double sh[4][256];
+    double mx = 0.0, s = 0.0, s2 = 0.0, cnt = 0.0;
+    for (int64_t i = blockIdx.x * 256 + threadIdx.x; i < n; i += 256 * (int64_t)gridDim.x) {
+        const double v = d[i];
+        if (v <= DBL_MAX) { mx = fmax(mx, v); s += v; s2 += v * v; cnt += 1.0; }
+    }
+    sh[0][threadIdx.x] = mx; sh[1][threadIdx.x] = s; sh[2][threadIdx.x] = s2; sh[3][threadIdx.x] = cnt;
+    __syncthreads();
+    for (int o = 128; o; o >>= 1) {
+        if (threadIdx.x < o) {
+            sh[0][threadIdx.x] = fmax(sh[0][threadIdx.x], sh[0][threadIdx.x + o]);
+            for (int k = 1; k < 4; ++k) sh[k][threadIdx.x] += sh[k][threadIdx.x + o];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x < 4) part[4 * blockIdx.x + threadIdx.x] = sh[threadIdx.x][0];
+}
+__global__ void __launch_bounds__(256) k_dist_summary(const double *__restrict__ part, double *__restrict__ out3) {
+    __shared__ double sh[4][NW_SUM_BLOCKS];
+    for (int k = 0; k < 4; ++k) sh[k][threadIdx.x] = part[4 * threadIdx.x + k];
+    __syncthreads();
+    for (int o = NW_SUM_BLOCKS / 2; o; o >>= 1) {
+        if (threadIdx.x < o) {
+            sh[0][threadIdx.x] = fmax(sh[0][threadIdx.x], sh[0][threadIdx.x + o]);
+            for (int k = 1; k < 4; ++k) sh[k][threadIdx.x] += sh[k][threadIdx.x + o];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        const double n = sh[3][0], nan = __longlong_as_double(0x7ff8000000000000LL);
+        out3[0] = n > 0.0 ? sh[0][0] : nan;
+        out3[1] = n > 0.0 ? sh[1][0] / n : nan;
+        out3[2] = n > 0.0 ? sqrt(sh[2][0] / n) : nan;
+    }
+}
+
+}  // namespace
+
+extern "C" int nw_surface_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *dist, int32_t *face, double *closest,
+                                   double summary[3]) {
+    if (!h) return NW_ERR_ARG;
+    NW_ARG(h->M > 0 && h->F > 0 && h->tl.n_levels > 1, "nw_surface_distance: no topology (call nw_set_topology first)");
+    NW_ARG(!h->points_mode, "nw_surface_distance: the handle holds point targets (nw_set_point_targets), not a mesh");
+    if (q) NW_ARG(Q >= 0 && Q < 2147483647LL, "nw_surface_distance: Q must be in [0, 2^31)");
+    else NW_ARG(Q == h->P && (h->px != nullptr || h->P == 0),
+                "nw_surface_distance: q == NULL measures the resident points; Q must equal their number (nw_set_points)");
+    NW_CUDA(cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    const int B = 256;
+    const TreeLevels &tl = h->tl;
+    const int leaf_level = tl.n_levels - 1, leaf0 = tl.off[leaf_level], total = leaf0 + tl.count[leaf_level];
+
+    // queries: the resident points (sorted SoA, results scattered to the caller's order through perm) or a copy of the caller's
+    const bool f64 = q ? q_is_f64 != 0 : h->px64 != nullptr;
+    SurfaceArgs a;
+    a.Q = Q;
+    if (q) {
+        const size_t bytes = (f64 ? 8 : 4) * 3 * (size_t)Q;
+        NW_CHECK(nw_alloc(h, &h->surf_q, std::max<size_t>(bytes, 8)));
+        NW_CHECK(nw_h2d(h, h->surf_q, q, bytes));
+        const size_t el = f64 ? 8 : 4;
+        a.qx = h->surf_q; a.qy = h->surf_q + el; a.qz = h->surf_q + 2 * el; a.stride = 3;
+        a.perm = nullptr; a.seed = nullptr;
+    } else {
+        if (f64) { a.qx = h->px64; a.qy = h->py64; a.qz = h->pz64; }
+        else { a.qx = h->px; a.qy = h->py; a.qz = h->pz; }
+        a.stride = 1;
+        a.perm = h->perm; a.seed = h->slot;
+    }
+
+    // slack of the call, then the triangle-bounded boxes at the current positions
+    NW_CHECK(nw_alloc(h, &h->surf_bits, (size_t)8));
+    NW_CUDA(cudaMemsetAsync(h->surf_bits, 0, sizeof(unsigned) * 6, s));
+    const float *pq = (const float *)h->posq;      // x, y, z of vertex v at pq[4 v + 0..2]
+    k_absmax3<float><<<std::min(nw_grid(h->M, B), 148 * 4), B, 0, s>>>(pq, pq + 1, pq + 2, h->M, 4, h->surf_bits);
+    NW_LAUNCH_CHECK();
+    if (Q > 0) {
+        if (f64) k_absmax3<double><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const double *)a.qx, (const double *)a.qy,
+                                                                                  (const double *)a.qz, Q, a.stride, h->surf_bits + 3);
+        else k_absmax3<float><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const float *)a.qx, (const float *)a.qy, (const float *)a.qz,
+                                                                            Q, a.stride, h->surf_bits + 3);
+        NW_LAUNCH_CHECK();
+    }
+    NW_CHECK(nw_alloc(h, &h->tboxes, (size_t)total));
+    k_tbox_init<<<nw_grid(total, B), B, 0, s>>>(h->boxes, total, h->tboxes);
+    NW_LAUNCH_CHECK();
+    k_tri_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->sfaces, h->posq, h->F, h->leaf_of_slot, leaf0, leaf_level, h->parent_g, h->tboxes);
+    NW_LAUNCH_CHECK();
+    k_tbox_decode<<<nw_grid(total - tl.off[1], B), B, 0, s>>>(h->tboxes, tl.off[1], total - tl.off[1], h->surf_bits);
+    NW_LAUNCH_CHECK();
+
+    // the search
+    const size_t nq = (size_t)std::max<int64_t>(Q, 1);
+    NW_CHECK(nw_alloc(h, &h->surf_dist, nq));
+    if (face) NW_CHECK(nw_alloc(h, &h->surf_face, nq));
+    if (closest) NW_CHECK(nw_alloc(h, &h->surf_closest, 3 * nq));
+    a.tb = h->tboxes; a.parent = h->parent_g; a.kids = h->kids; a.leaf_of_slot = h->leaf_of_slot; a.sfaces = h->sfaces; a.posq = h->posq;
+    a.leaf0 = leaf0; a.leaf_level = leaf_level; a.n_nodes = total; a.F = h->F;
+    a.dist = h->surf_dist; a.face = face ? h->surf_face : nullptr; a.closest = closest ? h->surf_closest : nullptr;
+    if (Q > 0) {
+        if (f64) k_surface_nearest<double><<<nw_grid(Q, 128), 128, 0, s>>>(a);
+        else k_surface_nearest<float><<<nw_grid(Q, 128), 128, 0, s>>>(a);
+        NW_LAUNCH_CHECK();
+    }
+    if (summary) {
+        NW_CHECK(nw_alloc(h, &h->surf_part, (size_t)4 * NW_SUM_BLOCKS + 4));
+        k_dist_partials<<<NW_SUM_BLOCKS, 256, 0, s>>>(h->surf_dist, Q, h->surf_part);
+        NW_LAUNCH_CHECK();
+        k_dist_summary<<<1, NW_SUM_BLOCKS, 0, s>>>(h->surf_part, h->surf_part + 4 * NW_SUM_BLOCKS);
+        NW_LAUNCH_CHECK();
+        NW_CUDA(cudaMemcpyAsync(summary, h->surf_part + 4 * NW_SUM_BLOCKS, sizeof(double) * 3, cudaMemcpyDeviceToHost, s));
+    }
+    if (Q > 0) {
+        if (dist) NW_CUDA(cudaMemcpyAsync(dist, h->surf_dist, sizeof(double) * Q, cudaMemcpyDeviceToHost, s));
+        if (face) NW_CUDA(cudaMemcpyAsync(face, h->surf_face, sizeof(int32_t) * Q, cudaMemcpyDeviceToHost, s));
+        if (closest) NW_CUDA(cudaMemcpyAsync(closest, h->surf_closest, sizeof(double) * 3 * Q, cudaMemcpyDeviceToHost, s));
+    }
+    NW_CUDA(cudaStreamSynchronize(s));
+    return NW_OK;
+}

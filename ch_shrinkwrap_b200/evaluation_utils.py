@@ -9,11 +9,19 @@ arguments and return values:
   searches in the solver's hierarchy (``nw_set_point_targets``); distances are the same float64 numbers.
 * ``nearest_point_distance(targets, queries)`` -- the building block, also used by the hole-punch candidate search.
 
+Not in the reference (its surface metrics compare sample clouds, so their answer depends on ``dx_min``):
+
+* ``surface_distance(mesh, points)`` -- exact distance from each point to the closed triangles of a mesh
+  (``nw_surface_distance``).
+* ``hausdorff_distance(mesh0, mesh1, dx_min)`` -- one-sided and symmetric Hausdorff and mean distances between two meshes,
+  from exact point-to-surface distances of each mesh's samples.
+
 No CPU fallback: these raise if libnanowrap.so or the GPU is missing.
 """
 from __future__ import annotations
 
 import ctypes
+from collections import namedtuple
 
 import numpy as np
 
@@ -76,6 +84,92 @@ def mesh_samples(mesh, dx_min=5, handle=None):
         if handle is None:
             h.close()
     return d
+
+
+def _surface_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False, want_summary=False):
+    """nw_surface_distance on handle `h`: queries None = the handle's `n_resident` resident points, else an (N,3) array.
+    Returns (dist, face, closest, summary), None for what was not asked for."""
+    if queries is None:
+        q, q64, Q = None, 0, int(n_resident)
+    else:
+        q, q64 = _xyz(queries)
+        Q = len(q)
+    dist = np.empty(Q, np.float64) if want_dist else None
+    face = np.empty(Q, np.int32) if want_face else None
+    closest = np.empty((Q, 3), np.float64) if want_closest else None
+    summary = np.empty(3, np.float64) if want_summary else None
+    h.call('nw_surface_distance', None if q is None else ctypes.c_void_p(q.ctypes.data), q64, Q, _lib.dptr(dist), _lib.iptr(face),
+           _lib.dptr(closest), _lib.dptr(summary))
+    return dist, face, closest, summary
+
+
+def _upload_surface(h, mesh):
+    """The mesh as the handle's topology (vertex positions as float32, faces = rows of ``mesh.faces``).  Normals and neighbour
+    tables do not enter the distance; a mesh without them gets zeros and -1 tables."""
+    pos = _lib.as_f32(mesh._vertices['position'])
+    faces = np.ascontiguousarray(mesh.faces, dtype=np.int32)
+    if len(pos) == 0 or len(faces) == 0:
+        raise ValueError('the mesh has no vertices or no faces')
+    nrm = getattr(mesh, 'vertex_normals', None)
+    nrm = np.zeros_like(pos) if nrm is None else _lib.as_f32(nrm)
+    nbr = np.full((len(pos), 20), -1, np.int32)
+    if 'neighbors' in (mesh._vertices.dtype.names or ()) and hasattr(mesh, '_halfedges'):
+        nb = np.asarray(mesh._vertices['neighbors'])
+        nbr = np.where(nb >= 0, np.asarray(mesh._halfedges['vertex'])[np.maximum(nb, 0)], -1).astype(np.int32)
+    h.call('nw_set_topology', _lib.fptr(pos), _lib.fptr(nrm), _lib.iptr(faces), _lib.iptr(nbr), None, len(pos), len(faces))
+
+
+def surface_distance(mesh, points, handle=None, return_face=False, return_closest=False):
+    """Exact Euclidean distance from each point to the closed triangles of `mesh` (float64, the points' order).
+
+    ``return_face``: also the row of ``mesh.faces`` of the nearest triangle (int32; exact fp64 ties go to the lowest row);
+    ``return_closest``: also the closest point on it ((N,3) float64).  Float32 points are used exactly, float64 points as
+    given.  A non-finite point gets NaN, face -1; faces with a non-finite corner are ignored.  Unlike the solver's nearest
+    face, which is the nearest face CENTROID (mesh_conj_grad.py:451-454), this is the distance to the surface itself."""
+    h = handle if handle is not None else _lib.Handle(0)
+    try:
+        _upload_surface(h, mesh)
+        dist, face, closest, _ = _surface_call(h, points, 0, True, return_face, return_closest)
+    finally:
+        if handle is None:
+            h.close()
+    if not (return_face or return_closest):
+        return dist
+    return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
+
+
+HausdorffResult = namedtuple('HausdorffResult', 'h01 h10 hausdorff mean01 mean10')
+
+
+def _surface_samples(mesh, dx_min, h):
+    pos = np.asarray(mesh._vertices['position'], np.float64)
+    if 'halfedge' in (mesh._vertices.dtype.names or ()):
+        pos = pos[mesh._vertices['halfedge'] != -1]                # a deleted vertex keeps its row
+    return np.concatenate([pos, mesh_samples(mesh, dx_min, h)], 0)
+
+
+def hausdorff_distance(mesh0, mesh1, dx_min=5, handle=None):
+    """Distances between two triangle meshes, both ways.
+
+    The samples of a mesh are its vertices plus ``mesh_samples(mesh, dx_min)`` (every triangle sampled on a dx_min grid in
+    its own plane).  ``h01`` is the largest exact distance from a sample of mesh0 to the surface of mesh1, ``mean01`` the
+    mean of those distances; ``h10`` and ``mean10`` the same the other way; ``hausdorff = max(h01, h10)``.
+
+    Each one-sided value is exact on its sample set, so it is a lower bound of the continuous one-sided Hausdorff distance
+    (the supremum over the whole surface) and converges to it as ``dx_min -> 0``.  The reductions run on the GPU in a fixed
+    order: repeated calls give identical numbers, and swapping the meshes swaps h01 / h10 and mean01 / mean10 exactly.
+    Returns a ``HausdorffResult(h01, h10, hausdorff, mean01, mean10)``."""
+    h = handle if handle is not None else _lib.Handle(0)
+    try:
+        s0, s1 = _surface_samples(mesh0, dx_min, h), _surface_samples(mesh1, dx_min, h)
+        _upload_surface(h, mesh1)
+        r01 = _surface_call(h, s0, want_dist=False, want_summary=True)[3]
+        _upload_surface(h, mesh0)
+        r10 = _surface_call(h, s1, want_dist=False, want_summary=True)[3]
+    finally:
+        if handle is None:
+            h.close()
+    return HausdorffResult(float(r01[0]), float(r10[0]), max(float(r01[0]), float(r10[0])), float(r01[1]), float(r10[1]))
 
 
 def points_from_mesh(mesh, dx_min=5, p=1.0, return_normals=False):

@@ -327,6 +327,18 @@ class ShrinkwrapMeshConjGrad(object):
         self._h.call('nw_point_influence', _lib.fptr(pi))
         return pi
 
+    def surface_distance(self, points=None, return_face=False, return_closest=False):
+        """Exact distance from each point to the mesh as it stands on the device (after ``search``, the fitted surface),
+        float64.  ``points=None``: the fit's own localisations, which are already resident (nothing is uploaded), in the order
+        they were given.  ``return_face`` / ``return_closest`` as ``evaluation_utils.surface_distance``.  This measures the
+        surface itself; the fit's weights keep using the nearest face centroid (mesh_conj_grad.py:451-454)."""
+        from .evaluation_utils import _surface_call
+        self._ensure_ready()
+        dist, face, closest, _ = _surface_call(self._h, points, self._session.P, True, return_face, return_closest)
+        if not (return_face or return_closest):
+            return dist
+        return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
+
     def _ncc(self):
         self._ensure_weights()
         fd = np.empty((self.M, 3), np.float64)

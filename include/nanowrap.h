@@ -171,6 +171,19 @@ int nw_holepunch_pair_candidate_faces(nw_ctx *h, const void *vertices, const voi
                                       int n_vertices, int n_faces, int n_halfedges, const int32_t *candidates,
                                       int n_candidates, int32_t *pairs);
 
+/* ---- exact point-to-surface distance (not part of the reference surface) ---------------------------------------
+ * Exact distance from each query to the handle's current triangle mesh (the topology of the last nw_set_topology*, at the
+ * current f -- after nw_search, the fitted surface).  q == NULL: the handle's own points (this rank's shard, caller order of
+ * nw_set_points; Q must equal their number).  Otherwise q is (Q,3) float32 (q_is_f64 = 0) or float64 (= 1).  Per query, in
+ * the caller's order: dist (Q) float64 Euclidean distance to the nearest closed triangle, face (Q) int32 its row of
+ * mesh.faces (exact fp64 ties -> lowest row), closest (Q,3) float64 the closest point on it.  summary = {max, mean, RMS} of
+ * dist from a fixed-order reduction on the device (bit-identical from call to call).  Faces with a non-finite corner are
+ * skipped; a non-finite query gets dist = NaN, face = -1 and is left out of summary.  Any output may be NULL.  Changes
+ * nothing that nw_search reads.  NW_ERR_ARG in points mode (nw_set_point_targets).  No collectives: each rank of a
+ * multi-rank handle measures its own shard. */
+int nw_surface_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *dist, int32_t *face, double *closest,
+                        double summary[3]);
+
 /* ---- measurement hooks (bench.py / profiling; not part of the reference surface) ------------------ */
 /* device-resident single-kernel launches on the handle's stream, for CUDA-event timing */
 int nw_bench_kernel(nw_ctx *h, const char *name, int reps, float *ms_per_launch);
