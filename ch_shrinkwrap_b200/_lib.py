@@ -52,6 +52,7 @@ SIGNATURES = {
     'nw_points_from_mesh': (c_int, [c_void_p, _f, _i, c_int, c_int, c_double, _d, c_int64, POINTER(c_int64)]),
     'nw_holepunch_pair_candidate_faces': (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, _i, c_int, _i]),
     'nw_surface_distance': (c_int, [c_void_p, c_void_p, c_int, c_int64, _d, _i, _d, _d]),
+    'nw_surface_signed_distance': (c_int, [c_void_p, c_void_p, c_int, c_int64, _d, _i, _d, _d]),
     'nw_bench_kernel': (c_int, [c_void_p, c_char_p, c_int, _f]),
     'nw_sync': (c_int, [c_void_p]),
     'nw_reset_seeds': (c_int, [c_void_p]),

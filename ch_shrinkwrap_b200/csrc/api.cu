@@ -52,6 +52,8 @@ extern "C" void nw_destroy(nw_ctx *h) {
     nw_free(&h->sfaces); nw_free(&h->cent); nw_free(&h->boxes); nw_free(&h->leaf_of_slot); nw_free(&h->node_f);
     nw_free(&h->tboxes); nw_free(&h->surf_q); nw_free(&h->surf_bits); nw_free(&h->surf_dist); nw_free(&h->surf_closest);
     nw_free(&h->surf_part); nw_free(&h->surf_face);
+    nw_free(&h->sgn_twin); nw_free(&h->sgn_voff); nw_free(&h->sgn_vface); nw_free(&h->sgn_k0); nw_free(&h->sgn_k1);
+    nw_free(&h->sgn_i0); nw_free(&h->sgn_i1); nw_free(&h->sgn_cnt); nw_free(&h->sgn_nv); nw_free(&h->sgn_vpart); nw_free(&h->sgn_bbox);
     nw_free(&h->acc); nw_free(&h->Sq); nw_free(&h->fdef);
     nw_free(&h->partials); nw_free(&h->st); nw_free(&h->hist);
     nw_free((char **)&h->cub_tmp); nw_free(&h->scratchM); nw_free(&h->scratchP);

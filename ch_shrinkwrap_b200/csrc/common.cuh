@@ -141,6 +141,20 @@ struct nw_ctx {
     unsigned *surf_bits = nullptr;               // per-axis max |coordinate| of vertices and queries (rounding slack of the call)
     double *surf_dist = nullptr, *surf_closest = nullptr, *surf_part = nullptr;
     int *surf_face = nullptr;
+    // nw_surface_signed_distance: edge and vertex tables of one topology (built on the first signed call), then per call the
+    // vertex pseudonormals and the signed volume
+    int64_t topo_gen = 0;                        // bumped by every nw_set_topology* and nw_set_point_targets (epoch moves more often)
+    int64_t sgn_gen = -1;                        // the topo_gen the tables below describe
+    int sgn_defects[5] = {0, 0, 0, 0, 0};        // boundary edges, edges on > 2 faces, co-directed edge pairs, faces repeating a
+                                                 // vertex, vertices whose faces form more than one fan
+    int *sgn_twin = nullptr;                     // 3F: the face across edge k (corner k -> k+1) of each face row, or -1
+    int *sgn_voff = nullptr, *sgn_vface = nullptr;   // vertex -> incident face rows in increasing order (CSR: M+1, 3F)
+    unsigned long long *sgn_k0 = nullptr, *sgn_k1 = nullptr;   // 3F sort keys
+    int *sgn_i0 = nullptr, *sgn_i1 = nullptr;    // 3F sort values
+    int *sgn_cnt = nullptr;                      // M+1 per-vertex counts, then the 5 defect counts
+    double *sgn_nv = nullptr;                    // 3M: angle-weighted vertex pseudonormals at the current positions
+    double *sgn_vpart = nullptr;                 // signed-volume partials, then the volume
+    unsigned *sgn_bbox = nullptr;                // ordered-uint min xyz, max xyz of the vertices the faces use
     // ---- solver vectors ----
     unsigned long long *acc = nullptr;           // (M,4) int64 fixed point: AH res xyz, AH 1
     float4 *Sq = nullptr;                        // search directions, interleaved: S_k of vertex v at Sq[3v + k] (48 B per vertex)

@@ -432,6 +432,7 @@ static int set_topology_impl(nw_ctx *h, const float *pos, const float *nrm, cons
     NW_CHECK(seg_end(h));
     h->M = M; h->F = F;
     h->epoch++;
+    h->topo_gen++;
     h->weights_valid = false;
     h->pin_fresh = false;
     h->points_mode = false;
@@ -668,6 +669,7 @@ extern "C" int nw_set_point_targets(nw_ctx *h, const void *xyz, int is_f64, int6
     const int n = (int)N, B = 256;
     h->M = n; h->F = n;
     h->epoch++;
+    h->topo_gen++;
     h->weights_valid = false; h->pin_fresh = false; h->feet_valid = false;
     h->points_mode = true;
     NW_CHECK(nw_alloc(h, &h->posq, (size_t)n)); NW_CHECK(nw_alloc(h, &h->nrmq, (size_t)n));

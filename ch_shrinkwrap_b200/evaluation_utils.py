@@ -13,6 +13,9 @@ Not in the reference (its surface metrics compare sample clouds, so their answer
 
 * ``surface_distance(mesh, points)`` -- exact distance from each point to the closed triangles of a mesh
   (``nw_surface_distance``).
+* ``surface_distance(mesh, points, signed=True)`` -- the same distance, negative inside a closed mesh and positive outside
+  (``nw_surface_signed_distance``: the angle-weighted pseudonormal of the nearest feature, oriented by the signed volume).
+* ``enclosed_volume(mesh)`` -- the volume a closed mesh encloses.
 * ``hausdorff_distance(mesh0, mesh1, dx_min)`` -- one-sided and symmetric Hausdorff and mean distances between two meshes,
   from exact point-to-surface distances of each mesh's samples.
 
@@ -103,6 +106,25 @@ def _surface_call(h, queries, n_resident=0, want_dist=True, want_face=False, wan
     return dist, face, closest, summary
 
 
+def _signed_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False):
+    """nw_surface_signed_distance on handle `h`, queries as in ``_surface_call``; ``queries`` of length 0 checks the mesh and
+    measures its volume only.  Returns (sdist, face, closest, volume), None for what was not asked for."""
+    if queries is None:
+        q, q64, Q = None, 0, int(n_resident)
+    else:
+        q, q64 = _xyz(queries)
+        Q = len(q)
+        if Q == 0:
+            q = np.zeros((1, 3), q.dtype)              # q must not be NULL: that would mean the resident points
+    sdist = np.empty(Q, np.float64) if want_dist else None
+    face = np.empty(Q, np.int32) if want_face else None
+    closest = np.empty((Q, 3), np.float64) if want_closest else None
+    volume = ctypes.c_double(0.0)
+    h.call('nw_surface_signed_distance', None if q is None else ctypes.c_void_p(q.ctypes.data), q64, Q, _lib.dptr(sdist),
+           _lib.iptr(face), _lib.dptr(closest), ctypes.byref(volume))
+    return sdist, face, closest, volume.value
+
+
 def _upload_surface(h, mesh):
     """The mesh as the handle's topology (vertex positions as float32, faces = rows of ``mesh.faces``).  Normals and neighbour
     tables do not enter the distance; a mesh without them gets zeros and -1 tables."""
@@ -119,8 +141,15 @@ def _upload_surface(h, mesh):
     h.call('nw_set_topology', _lib.fptr(pos), _lib.fptr(nrm), _lib.iptr(faces), _lib.iptr(nbr), None, len(pos), len(faces))
 
 
-def surface_distance(mesh, points, handle=None, return_face=False, return_closest=False):
+def surface_distance(mesh, points, handle=None, return_face=False, return_closest=False, signed=False):
     """Exact Euclidean distance from each point to the closed triangles of `mesh` (float64, the points' order).
+
+    ``signed=True``: negative inside the solid the mesh bounds, positive outside, 0 on the surface; NaN where the side is
+    undecidable (the offset from the closest point is orthogonal to the pseudonormal there).  The magnitude, face and closest
+    point are those of the unsigned call.  The side comes from the angle-weighted pseudonormal of the nearest face, edge or
+    vertex, and "inside" from the sign of the mesh's signed volume, so either winding gives the same answer.  The mesh must
+    be closed, edge-manifold and consistently oriented (ValueError with the defect counts otherwise); a mesh whose separate
+    components are oriented against each other is not supported.
 
     ``return_face``: also the row of ``mesh.faces`` of the nearest triangle (int32; exact fp64 ties go to the lowest row);
     ``return_closest``: also the closest point on it ((N,3) float64).  Float32 points are used exactly, float64 points as
@@ -129,13 +158,29 @@ def surface_distance(mesh, points, handle=None, return_face=False, return_closes
     h = handle if handle is not None else _lib.Handle(0)
     try:
         _upload_surface(h, mesh)
-        dist, face, closest, _ = _surface_call(h, points, 0, True, return_face, return_closest)
+        if signed:
+            dist, face, closest, _ = _signed_call(h, points, 0, True, return_face, return_closest)
+        else:
+            dist, face, closest, _ = _surface_call(h, points, 0, True, return_face, return_closest)
     finally:
         if handle is None:
             h.close()
     if not (return_face or return_closest):
         return dist
     return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
+
+
+def enclosed_volume(mesh, handle=None):
+    """The volume enclosed by a closed, edge-manifold, consistently oriented mesh (float64, either winding): the absolute
+    value of the signed volume sum_f dot(a - o, (b - o) x (c - o)) / 6 over the faces (a, b, c), reduced on the GPU in a
+    fixed order.  Raises ValueError for a mesh that does not bound a solid, as ``surface_distance(signed=True)`` does."""
+    h = handle if handle is not None else _lib.Handle(0)
+    try:
+        _upload_surface(h, mesh)
+        return _signed_call(h, np.zeros((0, 3), np.float32), want_dist=False)[3]
+    finally:
+        if handle is None:
+            h.close()
 
 
 HausdorffResult = namedtuple('HausdorffResult', 'h01 h10 hausdorff mean01 mean10')

@@ -180,13 +180,14 @@ class ShrinkwrapMeshMixin:
         s0 = self._S0
         return np.sqrt((s0 * s0).sum(1))
 
-    def point_surface_distance(self, points=None, return_face=False, return_closest=False):
+    def point_surface_distance(self, points=None, return_face=False, return_closest=False, signed=False):
         """Exact distance from each localisation to the fitted surface (float64); ``points=None``: the fit's own localisations
         (resident on the device).  Unlike ``point_dis``, which is per vertex and built from the fit's residuals, this is per
-        point and measures the closed triangles.  See ``ShrinkwrapMeshConjGrad.surface_distance``."""
+        point and measures the closed triangles.  ``signed=True``: negative inside the fitted surface, positive outside.  See
+        ``ShrinkwrapMeshConjGrad.surface_distance``."""
         if self.cg is None:
             raise RuntimeError('point_surface_distance: no fit on this mesh yet (self.cg is None)')
-        return self.cg.surface_distance(points, return_face=return_face, return_closest=return_closest)
+        return self.cg.surface_distance(points, return_face=return_face, return_closest=return_closest, signed=signed)
 
     @property
     def rms_point_sc(self):

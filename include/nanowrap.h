@@ -183,6 +183,18 @@ int nw_holepunch_pair_candidate_faces(nw_ctx *h, const void *vertices, const voi
  * multi-rank handle measures its own shard. */
 int nw_surface_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *dist, int32_t *face, double *closest,
                         double summary[3]);
+/* Signed distance to a closed mesh: the nearest-triangle search of nw_surface_distance (same queries, same face and closest,
+ * |sdist| = its dist), with sdist < 0 inside and > 0 outside.  The side is that of q - closest against the angle-weighted
+ * pseudonormal (Baerentzen & Aanaes 2005) of the feature the closest point lies on (face interior, edge, or vertex), times
+ * the sign of the mesh's signed volume, so it does not depend on the winding.  sdist = 0 on the surface; NaN where the side
+ * is undecidable (q - closest orthogonal to the pseudonormal) and for a non-finite query (face = -1).  volume = the enclosed
+ * volume |V| (fixed-order fp64 reduction).  The mesh must be closed, edge-manifold and consistently oriented (every edge on
+ * exactly two faces that traverse it in opposite directions, no face repeating a vertex, one fan of faces per vertex) and
+ * enclose a finite, non-zero volume; otherwise NW_ERR_ARG with the defect counts in nw_last_error.  A mesh whose components
+ * are oriented against each other is not supported: one global orientation decides inside.  Q == 0 with q != NULL checks
+ * the mesh and returns the volume only.  Any output may be NULL.  NW_ERR_ARG in points mode; no collectives. */
+int nw_surface_signed_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *sdist, int32_t *face,
+                               double *closest, double *volume);
 
 /* ---- measurement hooks (bench.py / profiling; not part of the reference surface) ------------------ */
 /* device-resident single-kernel launches on the handle's stream, for CUDA-event timing */

@@ -1,9 +1,11 @@
 """Exact point-to-surface distance at C3 (nw_surface_distance): call time for the 10^7 resident localisations against the fitted
-501 762-vertex mesh, and the two-way Hausdorff distance of two C3 fits.
+501 762-vertex mesh, and the two-way Hausdorff distance of two C3 fits.  With --signed, also the signed distance
+(nw_surface_signed_distance): a call with no queries just after an upload (twin table, vertex CSR, pseudonormals, volume) and
+repeated (pseudonormals and volume), and the 10^7 resident localisations signed and unsigned, alternating call by call.
 
 Every time is a host clock around calls that end in a stream synchronise (each nw_surface_distance call does), so it is
 device time plus the call's small host overhead: the median and the minimum of `reps` calls after two warm-up calls.
-  python tools/surface_probe.py [--reps 10] [--out FILE.json]"""
+  python tools/surface_probe.py [--reps 10] [--signed] [--out FILE.json]"""
 import argparse
 import ctypes
 import json
@@ -31,9 +33,56 @@ def timed(fn, reps):
     return {'median_ms': float(np.median(ts)), 'min_ms': float(np.min(ts)), 'reps': reps}
 
 
+def timed_alternating(fns, reps, setup=None):
+    """timed() of several calls, one of each in turn per repetition; `setup` (untimed) runs before every timed call."""
+    for _ in range(2):
+        for fn in fns.values():
+            if setup:
+                setup()
+            fn()
+    ts = {k: [] for k in fns}
+    for _ in range(reps):
+        for k, fn in fns.items():
+            if setup:
+                setup()
+            t0 = time.perf_counter()
+            fn()
+            ts[k].append(1e3 * (time.perf_counter() - t0))
+    return {k: {'median_ms': float(np.median(v)), 'min_ms': float(np.min(v)), 'reps': reps} for k, v in ts.items()}
+
+
+def signed_legs(h, fit, P, reps):
+    """nw_surface_signed_distance against nw_surface_distance on the fit's handle `h`; `fit` (the same mesh) on a second
+    handle for the calls that need a fresh upload."""
+    lib = eu._lib
+    summary, dist, sdist, vol = np.empty(3), np.empty(P), np.empty(P), ctypes.c_double()
+    one = np.zeros((1, 3), np.float32)
+    res = {}
+    aux = lib.Handle(0)
+    try:
+        q0 = lambda hh: hh.call('nw_surface_signed_distance', ctypes.c_void_p(one.ctypes.data), 0, 0, None, None, None,
+                                ctypes.byref(vol))
+        res['signed_q0_first_after_upload'] = timed_alternating({'call': lambda: q0(aux)}, reps,
+                                                                setup=lambda: eu._upload_surface(aux, fit))['call']
+        res['signed_q0_repeat'] = timed(lambda: q0(aux), reps)
+        res['volume_nm3'] = vol.value
+    finally:
+        aux.close()
+    res['resident_no_per_query_output'] = timed_alternating({
+        'unsigned_summary_only': lambda: h.call('nw_surface_distance', None, 0, P, None, None, None, lib.dptr(summary)),
+        'signed_volume_only': lambda: h.call('nw_surface_signed_distance', None, 0, P, None, None, None, ctypes.byref(vol))}, reps)
+    res['resident_distance_readback'] = timed_alternating({
+        'unsigned': lambda: h.call('nw_surface_distance', None, 0, P, lib.dptr(dist), None, None, None),
+        'signed': lambda: h.call('nw_surface_signed_distance', None, 0, P, lib.dptr(sdist), None, None, None)}, reps)
+    res['resident_inside_fraction'] = float((sdist < 0).mean())
+    res['resident_abs_signed_equals_unsigned'] = bool(np.array_equal(np.abs(sdist), dist))
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--reps', type=int, default=10)
+    ap.add_argument('--signed', action='store_true')
     ap.add_argument('--out', default=None)
     args = ap.parse_args()
     gpu = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
@@ -68,6 +117,8 @@ def main():
                                                               dx_min=5)
     res['hausdorff_repeat'] = timed(lambda: eu.hausdorff_distance(fit_a, fit_b, dx_min=5, handle=aux), 3)
     aux.close()
+    if args.signed:
+        res['signed'] = signed_legs(h, fit_b, P, args.reps)
     line = json.dumps(res)
     print(line)
     if args.out:
