@@ -1,6 +1,7 @@
 // common.cuh -- handle layout, error plumbing and small device helpers shared by all kernels.
 #pragma once
 #include <cuda_runtime.h>
+#include <cfloat>
 #include <stdint.h>
 #include <string>
 #include <unordered_map>
@@ -42,6 +43,60 @@ struct Box {
     __host__ __device__ __forceinline__ float lo(int k) const { return k == 0 ? b.z : k == 1 ? b.w : d.w; }
     __host__ __device__ __forceinline__ float hi(int k) const { return k == 0 ? d.x : k == 1 ? d.y : c.w; }
 };              // 64 B
+
+// Ordered-int encoding of floats: f2ord orders like the floats as signed ints, f2u as unsigned ints, so interval ends can be
+// merged with integer atomics and REDUX.  The box intervals hold f2ord bits while they are being measured.
+__device__ __forceinline__ int f2ord(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
+__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
+__device__ __forceinline__ unsigned f2u(float f) { return (unsigned)f2ord(f) ^ 0x80000000u; }
+__device__ __forceinline__ int u2ord(unsigned u) { return (int)(u ^ 0x80000000u); }
+#define NW_EMPTY_LO __int_as_float(f2ord(FLT_MAX))      // ordered-int encodings of an empty interval
+#define NW_EMPTY_HI __int_as_float(f2ord(-FLT_MAX))
+
+// One level of an extents pass (tree.cu: k_extents, surface.cu: k_tri_extents): a live lane's member, projected onto the
+// frame of boxes[node] by project(box, lo, hi), spans [lo, hi] per axis; finite == false contributes nothing.  Lanes that
+// share the node are reduced with REDUX first, then the run's first lane applies one ordered-int atomic min/max per quantity.
+template <typename Project>
+__device__ __forceinline__ void nw_merge_extents(Box *boxes, int node, bool live, bool finite, Project project) {
+    // lanes that share the node: the slots are sorted by key, so equal nodes are runs of consecutive lanes -- run heads
+    // from one shuffle and a ballot (match_any costs several times more)
+    const unsigned lane = threadIdx.x & 31;
+    const int prev = __shfl_up_sync(0xffffffffu, node, 1);
+    const unsigned heads = __ballot_sync(0xffffffffu, lane == 0 || prev != node || !live);
+    const unsigned upto = 0xffffffffu >> (31 - lane);                           // lanes 0..lane
+    const int first = 31 - __clz(heads & upto);
+    const unsigned above = heads & ~upto;
+    const unsigned grp = (above ? ((1u << (__ffs(above) - 1)) - 1u) : 0xffffffffu) & ~((1u << first) - 1u);
+    Box *b = &boxes[node];
+    float lo[3] = {0.f, 0.f, 0.f}, hi[3] = {0.f, 0.f, 0.f};
+    if (live) project(b, lo, hi);
+    unsigned mn[3], mx[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        mn[k] = __reduce_min_sync(grp, finite ? f2u(lo[k]) : 0xffffffffu);
+        mx[k] = __reduce_max_sync(grp, finite ? f2u(hi[k]) : 0u);
+    }
+    if (live && lane == (unsigned)first && mn[0] <= mx[0]) {
+        // the upper levels are hit by thousands of warps and all but the first few change nothing: look first
+        // (an L2 read; a stale value only costs a redundant atomic, the atomics themselves are monotone)
+        const float4 cb = __ldcg(&b->b), cd = __ldcg(&b->d);
+        const float ch2 = __ldcg(&b->c.w);
+        if (u2ord(mn[0]) < __float_as_int(cb.z)) atomicMin((int *)&b->b.z, u2ord(mn[0]));
+        if (u2ord(mx[0]) > __float_as_int(cd.x)) atomicMax((int *)&b->d.x, u2ord(mx[0]));
+        if (u2ord(mn[1]) < __float_as_int(cb.w)) atomicMin((int *)&b->b.w, u2ord(mn[1]));
+        if (u2ord(mx[1]) > __float_as_int(cd.y)) atomicMax((int *)&b->d.y, u2ord(mx[1]));
+        if (u2ord(mn[2]) < __float_as_int(cd.w)) atomicMin((int *)&b->d.w, u2ord(mn[2]));
+        if (u2ord(mx[2]) > __float_as_int(ch2)) atomicMax((int *)&b->c.w, u2ord(mx[2]));
+    }
+}
+
+// the merged ordered-int intervals of a box -> floats, each end moved out by w (field by field: a loop over Box::lo(k) /
+// hi(k) compiles to six scalar loads and stores instead of 128- and 64-bit ones)
+__device__ __forceinline__ void nw_decode_box(Box *b, float w) {
+    b->b.z = ord2f(__float_as_int(b->b.z)) - w; b->d.x = ord2f(__float_as_int(b->d.x)) + w;
+    b->b.w = ord2f(__float_as_int(b->b.w)) - w; b->d.y = ord2f(__float_as_int(b->d.y)) + w;
+    b->d.w = ord2f(__float_as_int(b->d.w)) - w; b->c.w = ord2f(__float_as_int(b->c.w)) + w;
+}
 
 // orthonormal completion of a unit vector (Duff et al. 2017, branchless): returns t1; t2 = n x t1 everywhere.
 // Used identically when boxes are built and when they are tested.

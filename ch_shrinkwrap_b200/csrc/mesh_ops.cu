@@ -15,9 +15,6 @@ namespace {
 
 __device__ __forceinline__ double pow2d(int e) { return __longlong_as_double((long long)(1023 + e) << 52); }
 
-__device__ __forceinline__ int f2ord(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
-__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
-
 // bounding box of the vertices: block reduction + ordered-int atomics into st->bbox (reset by k_shift_final)
 __global__ void __launch_bounds__(256) k_shift_partial(const float4 *__restrict__ pos, int M, SolverState *st) {
     if (st->stop) return;

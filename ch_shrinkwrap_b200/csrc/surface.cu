@@ -10,14 +10,15 @@
 // Exactness: every candidate face's distance is evaluated in fp64 (corners widened exactly from float32, queries in
 // float32 widened exactly or in float64) by one fixed sequence of operations, Ericson's closest-point region test
 // (Real-Time Collision Detection, 5.1.5).  This file is compiled with -fmad=false so that the compiler performs exactly the
-// written operations: tests/surface_oracle.py (closest_point_triangle) restates them in numpy and gets the same bits.
+// written operations: tests/surface_oracle.py (closest_point_region) restates them in numpy and gets the same bits.
 // Ties of the fp64 squared distance go to the lowest face index.  The box test only prunes: its float32 lower bound is
 // made conservative by the rounding slack of the call (below), so it can never discard the true minimum.
 //
-// nw_surface_signed_distance runs the same search, then k_surface_sign re-runs the region test on the winning face (same
-// bits of the closest point) and takes the side of q - c against the angle-weighted pseudonormal of that feature (face,
-// edge or vertex; Baerentzen & Aanaes 2005), oriented by the sign of the mesh's signed volume.  Its edge and vertex tables
-// are built once per topology (signed_tables), lazily, so nw_set_topology* does no extra work.
+// nw_surface_signed_distance runs the same search, then k_surface_sign re-runs the region test on the winning face with
+// closest_on_triangle<true>, which also names the feature the closest point lies on (same bits of the point), and takes the
+// side of q - c against the angle-weighted pseudonormal of that feature (face, edge or vertex; Baerentzen & Aanaes 2005),
+// oriented by the sign of the mesh's signed volume.  Its edge and vertex tables are built once per topology
+// (signed_tables), lazily, so nw_set_topology* does no extra work.
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -25,13 +26,6 @@
 #include "common.cuh"
 
 namespace {
-
-__device__ __forceinline__ int f2ord(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
-__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
-__device__ __forceinline__ unsigned f2u(float f) { return (unsigned)f2ord(f) ^ 0x80000000u; }      // order-preserving float -> unsigned
-__device__ __forceinline__ int u2ord(unsigned u) { return (int)(u ^ 0x80000000u); }
-#define NW_EMPTY_LO __int_as_float(f2ord(FLT_MAX))      // ordered-int encodings of an empty interval
-#define NW_EMPTY_HI __int_as_float(f2ord(-FLT_MAX))
 
 // projection onto a node frame as the box stores it (t2 = c.xyz): the operations of the search's node test (sweep.cu)
 __device__ __forceinline__ void project_frame(const float4 a, const float4 b, const float4 c, float x, float y, float z, float &pn,
@@ -82,8 +76,8 @@ __global__ void k_tbox_init(const Box *__restrict__ boxes, int n, Box *__restric
 }
 
 // k_extents (tree.cu) with the three corners of each face in place of its centroid: every face projects its corners onto the
-// frame of every ancestor; lanes of a warp that share the node are reduced first, then one ordered-int atomic per quantity.
-// A face with a non-finite corner contributes nothing (the query kernel skips it too).
+// frame of every ancestor (common.cuh: nw_merge_extents).  A face with a non-finite corner contributes nothing (the query
+// kernel skips it too).
 __global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sfaces, const float4 *__restrict__ pos, int F,
                                                      const int *__restrict__ leaf_of_slot, int leaf0, int leaf_level,
                                                      const int *__restrict__ parent_g, Box *__restrict__ boxes) {
@@ -97,17 +91,8 @@ __global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sf
         for (int k = 0; k < 3; ++k) finite = finite && fabsf(v[k].x) <= FLT_MAX && fabsf(v[k].y) <= FLT_MAX && fabsf(v[k].z) <= FLT_MAX;
     }
     int node = live ? leaf0 + leaf_of_slot[i] : 0;
-    const unsigned lane = threadIdx.x & 31;
     for (int l = leaf_level; l >= 1; --l) {
-        const int prev = __shfl_up_sync(0xffffffffu, node, 1);
-        const unsigned heads = __ballot_sync(0xffffffffu, lane == 0 || prev != node || !live);
-        const unsigned upto = 0xffffffffu >> (31 - lane);
-        const int first = 31 - __clz(heads & upto);
-        const unsigned above = heads & ~upto;
-        const unsigned grp = (above ? ((1u << (__ffs(above) - 1)) - 1u) : 0xffffffffu) & ~((1u << first) - 1u);
-        Box *b = &boxes[node];
-        float lo[3] = {0.f, 0.f, 0.f}, hi[3] = {0.f, 0.f, 0.f};
-        if (live) {
+        nw_merge_extents(boxes, node, live, finite, [&](const Box *b, float (&lo)[3], float (&hi)[3]) {
             const float4 ba = b->a, bb = b->b, bc = b->c;
             project_frame(ba, bb, bc, v[0].x, v[0].y, v[0].z, lo[0], lo[1], lo[2]);
             hi[0] = lo[0]; hi[1] = lo[1]; hi[2] = lo[2];
@@ -116,23 +101,7 @@ __global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sf
                 project_frame(ba, bb, bc, v[c].x, v[c].y, v[c].z, p[0], p[1], p[2]);
                 for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], p[k]); hi[k] = fmaxf(hi[k], p[k]); }
             }
-        }
-        unsigned mn[3], mx[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            mn[k] = __reduce_min_sync(grp, finite ? f2u(lo[k]) : 0xffffffffu);
-            mx[k] = __reduce_max_sync(grp, finite ? f2u(hi[k]) : 0u);
-        }
-        if (live && lane == (unsigned)first && mn[0] <= mx[0]) {
-            const float4 cb = __ldcg(&b->b), cd = __ldcg(&b->d);
-            const float ch2 = __ldcg(&b->c.w);
-            if (u2ord(mn[0]) < __float_as_int(cb.z)) atomicMin((int *)&b->b.z, u2ord(mn[0]));
-            if (u2ord(mx[0]) > __float_as_int(cd.x)) atomicMax((int *)&b->d.x, u2ord(mx[0]));
-            if (u2ord(mn[1]) < __float_as_int(cb.w)) atomicMin((int *)&b->b.w, u2ord(mn[1]));
-            if (u2ord(mx[1]) > __float_as_int(cd.y)) atomicMax((int *)&b->d.y, u2ord(mx[1]));
-            if (u2ord(mn[2]) < __float_as_int(cd.w)) atomicMin((int *)&b->d.w, u2ord(mn[2]));
-            if (u2ord(mx[2]) > __float_as_int(ch2)) atomicMax((int *)&b->c.w, u2ord(mx[2]));
-        }
+        });
         if (live) node = parent_g[node] & 0x7fffffff;
     }
 }
@@ -141,11 +110,7 @@ __global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sf
 __global__ void k_tbox_decode(Box *__restrict__ tb, int first, int count, const unsigned *__restrict__ bits6) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
-    const float w = call_slack(bits6);
-    Box *b = &tb[first + i];
-    b->b.z = ord2f(__float_as_int(b->b.z)) - w; b->d.x = ord2f(__float_as_int(b->d.x)) + w;
-    b->b.w = ord2f(__float_as_int(b->b.w)) - w; b->d.y = ord2f(__float_as_int(b->d.y)) + w;
-    b->d.w = ord2f(__float_as_int(b->d.w)) - w; b->c.w = ord2f(__float_as_int(b->c.w)) + w;
+    nw_decode_box(&tb[first + i], call_slack(bits6));
 }
 
 // ---- exact point-to-triangle distance (fp64, fixed operation order; restated in tests/surface_oracle.py) -------------------
@@ -156,82 +121,41 @@ __device__ __forceinline__ double dot(const D3 a, const D3 b) { return (a.x * b.
 __device__ __forceinline__ D3 axpy(const D3 a, const double t, const D3 e) { return D3{a.x + t * e.x, a.y + t * e.y, a.z + t * e.z}; }
 __device__ __forceinline__ double dist2(const D3 p, const D3 c) { const D3 d = sub(p, c); return dot(d, d); }
 
-__device__ __forceinline__ D3 closest_on_segment(const D3 p, const D3 p0, const D3 p1) {
+// R: also name the feature the closest point lies on (nw_surface_signed_distance), in r.  Region codes: 0 the interior,
+// 1 + k corner k, 4 + k the edge from corner k to corner k + 1 (mod 3).  The operations, and so the points, do not depend on R.
+#define NW_REGION_CORNER(k) (1 + (k))
+#define NW_REGION_EDGE(k) (4 + (k))
+// the segment p0 -> p1 as edge k of a triangle
+template <bool R>
+__device__ __forceinline__ D3 closest_on_segment(const D3 p, const D3 p0, const D3 p1, const int k, int &r) {
     const D3 e = sub(p1, p0);
     const double ee = dot(e, e);
     double t = ee > 0.0 ? dot(sub(p, p0), e) / ee : 0.0;
     t = fmin(fmax(t, 0.0), 1.0);
+    if (R) r = t == 0.0 ? NW_REGION_CORNER(k) : t == 1.0 ? NW_REGION_CORNER((k + 1) % 3) : NW_REGION_EDGE(k);
     return axpy(p0, t, e);
 }
 // a zero-area triangle is the union of its three edges: the closest of them, in the order ab, bc, ca (first wins ties)
-__device__ __noinline__ D3 closest_on_edges(const D3 p, const D3 a, const D3 b, const D3 c) {
-    D3 best = closest_on_segment(p, a, b);
+template <bool R>
+__device__ __noinline__ D3 closest_on_edges(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
+    int rk;
+    D3 best = closest_on_segment<R>(p, a, b, 0, r);
     double bd = dist2(p, best);
-    D3 k = closest_on_segment(p, b, c);
+    D3 k = closest_on_segment<R>(p, b, c, 1, rk);
     double kd = dist2(p, k);
-    if (kd < bd) { best = k; bd = kd; }
-    k = closest_on_segment(p, c, a);
+    if (kd < bd) { best = k; bd = kd; if (R) r = rk; }
+    k = closest_on_segment<R>(p, c, a, 2, rk);
     kd = dist2(p, k);
-    if (kd < bd) best = k;
+    if (kd < bd) { best = k; if (R) r = rk; }
     return best;
 }
 // Ericson's region test.  Degenerate: the cross product ab x ac is exactly zero, or (rounding of a nearly degenerate
 // triangle) the interior case finds no positive barycentric denominator.
-__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c) {
+template <bool R>
+__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
     const D3 ab = sub(b, a), ac = sub(c, a);
     if (ab.y * ac.z - ab.z * ac.y == 0.0 && ab.z * ac.x - ab.x * ac.z == 0.0 && ab.x * ac.y - ab.y * ac.x == 0.0)
-        return closest_on_edges(p, a, b, c);
-    const D3 ap = sub(p, a);
-    const double d1 = dot(ab, ap), d2 = dot(ac, ap);
-    if (d1 <= 0.0 && d2 <= 0.0) return a;
-    const D3 bp = sub(p, b);
-    const double d3 = dot(ab, bp), d4 = dot(ac, bp);
-    if (d3 >= 0.0 && d4 <= d3) return b;
-    const double vc = d1 * d4 - d3 * d2;
-    if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) return axpy(a, d1 / (d1 - d3), ab);
-    const D3 cp = sub(p, c);
-    const double d5 = dot(ab, cp), d6 = dot(ac, cp);
-    if (d6 >= 0.0 && d5 <= d6) return c;
-    const double vb = d5 * d2 - d1 * d6;
-    if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) return axpy(a, d2 / (d2 - d6), ac);
-    const double va = d3 * d6 - d5 * d4;
-    if (va <= 0.0 && (d4 - d3) >= 0.0 && (d5 - d6) >= 0.0) return axpy(b, (d4 - d3) / ((d4 - d3) + (d5 - d6)), sub(c, b));
-    const double s = va + vb + vc;
-    if (!(s > 0.0)) return closest_on_edges(p, a, b, c);
-    const double denom = 1.0 / s;
-    const double v = vb * denom, w = vc * denom;
-    return D3{(a.x + ab.x * v) + ac.x * w, (a.y + ab.y * v) + ac.y * w, (a.z + ab.z * v) + ac.z * w};
-}
-
-// ---- the same routine, also naming the feature the closest point lies on (nw_surface_signed_distance) ------------------
-// Region codes: 0 the interior, 1 + k corner k, 4 + k the edge from corner k to corner k + 1 (mod 3).  The operations are
-// those of closest_on_segment / closest_on_edges / closest_on_triangle, so the points are the same bits.
-#define NW_REGION_CORNER(k) (1 + (k))
-#define NW_REGION_EDGE(k) (4 + (k))
-__device__ __forceinline__ D3 segment_region(const D3 p, const D3 p0, const D3 p1, const int k, int &r) {
-    const D3 e = sub(p1, p0);
-    const double ee = dot(e, e);
-    double t = ee > 0.0 ? dot(sub(p, p0), e) / ee : 0.0;
-    t = fmin(fmax(t, 0.0), 1.0);
-    r = t == 0.0 ? NW_REGION_CORNER(k) : t == 1.0 ? NW_REGION_CORNER((k + 1) % 3) : NW_REGION_EDGE(k);
-    return axpy(p0, t, e);
-}
-__device__ __noinline__ D3 edges_region(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
-    int rk;
-    D3 best = segment_region(p, a, b, 0, r);
-    double bd = dist2(p, best);
-    D3 k = segment_region(p, b, c, 1, rk);
-    double kd = dist2(p, k);
-    if (kd < bd) { best = k; bd = kd; r = rk; }
-    k = segment_region(p, c, a, 2, rk);
-    kd = dist2(p, k);
-    if (kd < bd) { best = k; r = rk; }
-    return best;
-}
-__device__ __forceinline__ D3 triangle_region(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
-    const D3 ab = sub(b, a), ac = sub(c, a);
-    if (ab.y * ac.z - ab.z * ac.y == 0.0 && ab.z * ac.x - ab.x * ac.z == 0.0 && ab.x * ac.y - ab.y * ac.x == 0.0)
-        return edges_region(p, a, b, c, r);
+        return closest_on_edges<R>(p, a, b, c, r);
     const D3 ap = sub(p, a);
     const double d1 = dot(ab, ap), d2 = dot(ac, ap);
     if (d1 <= 0.0 && d2 <= 0.0) { r = NW_REGION_CORNER(0); return a; }
@@ -251,11 +175,15 @@ __device__ __forceinline__ D3 triangle_region(const D3 p, const D3 a, const D3 b
         return axpy(b, (d4 - d3) / ((d4 - d3) + (d5 - d6)), sub(c, b));
     }
     const double s = va + vb + vc;
-    if (!(s > 0.0)) return edges_region(p, a, b, c, r);
+    if (!(s > 0.0)) return closest_on_edges<R>(p, a, b, c, r);
     const double denom = 1.0 / s;
     const double v = vb * denom, w = vc * denom;
     r = 0;
     return D3{(a.x + ab.x * v) + ac.x * w, (a.y + ab.y * v) + ac.y * w, (a.z + ab.z * v) + ac.z * w};
+}
+__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c) {
+    int r;
+    return closest_on_triangle<false>(p, a, b, c, r);
 }
 
 // the operations of the degenerate test above: cross(b - a, c - a) of a face in row order
@@ -601,7 +529,7 @@ __global__ void __launch_bounds__(128) k_surface_sign(const __grid_constant__ Si
     const int cv[3] = {a.faces[3 * f], a.faces[3 * f + 1], a.faces[3 * f + 2]};
     const D3 x[3] = {d3(a.posq[cv[0]]), d3(a.posq[cv[1]]), d3(a.posq[cv[2]])};
     int r;
-    const D3 c = triangle_region(p, x[0], x[1], x[2], r);
+    const D3 c = closest_on_triangle<true>(p, x[0], x[1], x[2], r);
     D3 N;
     if (r == 0) {
         N = cross(sub(x[1], x[0]), sub(x[2], x[0]));

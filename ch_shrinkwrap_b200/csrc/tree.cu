@@ -130,11 +130,6 @@ __global__ void k_sorted_faces(const int *__restrict__ faces, const int *__restr
     fcells[i] = cells[f];
 }
 
-__device__ __forceinline__ int f2ord(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
-__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
-__device__ __forceinline__ unsigned f2u(float f) { return (unsigned)f2ord(f) ^ 0x80000000u; }      // order-preserving float -> unsigned
-__device__ __forceinline__ int u2ord(unsigned u) { return (int)(u ^ 0x80000000u); }
-
 __device__ __forceinline__ void project3(const float3 n, const float4 c, float &pn, float &p1, float &p2) {
     const float3 t1 = nw_tangent_of(n.x, n.y, n.z);
     const float3 t2 = make_float3(n.y * t1.z - n.z * t1.y, n.z * t1.x - n.x * t1.z, n.x * t1.y - n.y * t1.x);
@@ -142,8 +137,6 @@ __device__ __forceinline__ void project3(const float3 n, const float4 c, float &
     p1 = fmaf(t1.x, c.x, fmaf(t1.y, c.y, t1.z * c.z));
     p2 = fmaf(t2.x, c.x, fmaf(t2.y, c.y, t2.z * c.z));
 }
-#define NW_EMPTY_LO __int_as_float(f2ord(FLT_MAX))      // ordered-int encodings of an empty interval
-#define NW_EMPTY_HI __int_as_float(f2ord(-FLT_MAX))
 
 // ======================================================================================================================
 // The hierarchy is the OCTREE OF OCCUPIED HILBERT CELLS: a level-k node is the set of centroids that share the first 3k
@@ -301,8 +294,7 @@ __global__ void k_reset_extents(Box *__restrict__ boxes, int first, int count) {
     b->b.z = NW_EMPTY_LO; b->b.w = NW_EMPTY_LO; b->d.w = NW_EMPTY_LO; b->d.x = NW_EMPTY_HI; b->d.y = NW_EMPTY_HI; b->c.w = NW_EMPTY_HI;
 }
 
-// every iteration: each centroid projects onto the frame of every ancestor; lanes of a warp that
-// share the node are reduced with REDUX first, then one ordered-int atomic min/max per quantity
+// every iteration: each centroid projects onto the frame of every ancestor (common.cuh: nw_merge_extents)
 __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent, int F, const int *__restrict__ leaf_of_slot,
                                                  int leaf0, int leaf_level, const int *__restrict__ parent_g, Box *__restrict__ boxes) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -310,41 +302,12 @@ __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent
     const float4 c = live ? cent[i] : make_float4(0.f, 0.f, 0.f, 0.f);
     const bool finite = live && (c.x == c.x) && (c.y == c.y) && (c.z == c.z);
     int node = live ? leaf0 + leaf_of_slot[i] : 0;
-    const unsigned lane = threadIdx.x & 31;
     for (int l = leaf_level; l >= 1; --l) {
-        // lanes that share the node: the slots are sorted by key, so equal nodes are runs of consecutive lanes -- run
-        // heads from one shuffle and a ballot (match_any costs several times more)
-        const int prev = __shfl_up_sync(0xffffffffu, node, 1);
-        const unsigned heads = __ballot_sync(0xffffffffu, lane == 0 || prev != node || !live);
-        const unsigned upto = 0xffffffffu >> (31 - lane);                       // lanes 0..lane
-        const int first = 31 - __clz(heads & upto);
-        const unsigned above = heads & ~upto;
-        const unsigned grp = (above ? ((1u << (__ffs(above) - 1)) - 1u) : 0xffffffffu) & ~((1u << first) - 1u);
-        Box *b = &boxes[node];
-        float p[3] = {0.f, 0.f, 0.f};
-        if (live) {
+        nw_merge_extents(boxes, node, live, finite, [&](const Box *b, float (&lo)[3], float (&hi)[3]) {
             const float4 ba = b->a;
-            project3(make_float3(ba.x, ba.z, b->b.x), c, p[0], p[1], p[2]);
-        }
-        unsigned mn[3], mx[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            const unsigned lo = finite ? f2u(p[k]) : 0xffffffffu, hi = finite ? f2u(p[k]) : 0u;
-            mn[k] = __reduce_min_sync(grp, lo);
-            mx[k] = __reduce_max_sync(grp, hi);
-        }
-        if (live && lane == (unsigned)first && mn[0] <= mx[0]) {
-            // the upper levels are hit by thousands of warps and all but the first few change nothing: look first
-            // (an L2 read; a stale value only costs a redundant atomic, the atomics themselves are monotone)
-            const float4 cb = __ldcg(&b->b), cd = __ldcg(&b->d);
-            const float ch2 = __ldcg(&b->c.w);
-            if (u2ord(mn[0]) < __float_as_int(cb.z)) atomicMin((int *)&b->b.z, u2ord(mn[0]));
-            if (u2ord(mx[0]) > __float_as_int(cd.x)) atomicMax((int *)&b->d.x, u2ord(mx[0]));
-            if (u2ord(mn[1]) < __float_as_int(cb.w)) atomicMin((int *)&b->b.w, u2ord(mn[1]));
-            if (u2ord(mx[1]) > __float_as_int(cd.y)) atomicMax((int *)&b->d.y, u2ord(mx[1]));
-            if (u2ord(mn[2]) < __float_as_int(cd.w)) atomicMin((int *)&b->d.w, u2ord(mn[2]));
-            if (u2ord(mx[2]) > __float_as_int(ch2)) atomicMax((int *)&b->c.w, u2ord(mx[2]));
-        }
+            project3(make_float3(ba.x, ba.z, b->b.x), c, lo[0], lo[1], lo[2]);
+            hi[0] = lo[0]; hi[1] = lo[1]; hi[2] = lo[2];
+        });
         if (live) node = parent_g[node] & 0x7fffffff;
     }
 }
@@ -354,11 +317,7 @@ __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent
 __global__ void k_box_decode(Box *__restrict__ boxes, int first, int count, const SolverState *__restrict__ st) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
-    const float w = st->coord_l1 * 1.9073486328125e-6f;
-    Box *b = &boxes[first + i];
-    b->b.z = ord2f(__float_as_int(b->b.z)) - w; b->d.x = ord2f(__float_as_int(b->d.x)) + w;
-    b->b.w = ord2f(__float_as_int(b->b.w)) - w; b->d.y = ord2f(__float_as_int(b->d.y)) + w;
-    b->d.w = ord2f(__float_as_int(b->d.w)) - w; b->c.w = ord2f(__float_as_int(b->c.w)) + w;
+    nw_decode_box(&boxes[first + i], st->coord_l1 * 1.9073486328125e-6f);
 }
 
 #define NW_NMOM 3        // floats per node of the build scratch (area-weighted normal sum)

@@ -89,26 +89,12 @@ def mesh_samples(mesh, dx_min=5, handle=None):
     return d
 
 
-def _surface_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False, want_summary=False):
-    """nw_surface_distance on handle `h`: queries None = the handle's `n_resident` resident points, else an (N,3) array.
-    Returns (dist, face, closest, summary), None for what was not asked for."""
-    if queries is None:
-        q, q64, Q = None, 0, int(n_resident)
-    else:
-        q, q64 = _xyz(queries)
-        Q = len(q)
-    dist = np.empty(Q, np.float64) if want_dist else None
-    face = np.empty(Q, np.int32) if want_face else None
-    closest = np.empty((Q, 3), np.float64) if want_closest else None
-    summary = np.empty(3, np.float64) if want_summary else None
-    h.call('nw_surface_distance', None if q is None else ctypes.c_void_p(q.ctypes.data), q64, Q, _lib.dptr(dist), _lib.iptr(face),
-           _lib.dptr(closest), _lib.dptr(summary))
-    return dist, face, closest, summary
-
-
-def _signed_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False):
-    """nw_surface_signed_distance on handle `h`, queries as in ``_surface_call``; ``queries`` of length 0 checks the mesh and
-    measures its volume only.  Returns (sdist, face, closest, volume), None for what was not asked for."""
+def _surface_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False, want_summary=False,
+                  signed=False):
+    """nw_surface_distance, or with ``signed`` nw_surface_signed_distance, on handle `h`: queries None = the handle's
+    `n_resident` resident points, else an (N,3) array.  Returns (dist, face, closest, extra), None for what was not asked
+    for; extra is the summary (max, mean, RMS) of the unsigned call (``want_summary``), the enclosed volume of the signed
+    one.  A signed call with a length-0 ``queries`` checks the mesh and measures its volume only."""
     if queries is None:
         q, q64, Q = None, 0, int(n_resident)
     else:
@@ -116,13 +102,31 @@ def _signed_call(h, queries, n_resident=0, want_dist=True, want_face=False, want
         Q = len(q)
         if Q == 0:
             q = np.zeros((1, 3), q.dtype)              # q must not be NULL: that would mean the resident points
-    sdist = np.empty(Q, np.float64) if want_dist else None
+    qp = None if q is None else ctypes.c_void_p(q.ctypes.data)
+    dist = np.empty(Q, np.float64) if want_dist else None
     face = np.empty(Q, np.int32) if want_face else None
     closest = np.empty((Q, 3), np.float64) if want_closest else None
-    volume = ctypes.c_double(0.0)
-    h.call('nw_surface_signed_distance', None if q is None else ctypes.c_void_p(q.ctypes.data), q64, Q, _lib.dptr(sdist),
-           _lib.iptr(face), _lib.dptr(closest), ctypes.byref(volume))
-    return sdist, face, closest, volume.value
+    if signed:
+        volume = ctypes.c_double(0.0)
+        h.call('nw_surface_signed_distance', qp, q64, Q, _lib.dptr(dist), _lib.iptr(face), _lib.dptr(closest),
+               ctypes.byref(volume))
+        return dist, face, closest, volume.value
+    summary = np.empty(3, np.float64) if want_summary else None
+    h.call('nw_surface_distance', qp, q64, Q, _lib.dptr(dist), _lib.iptr(face), _lib.dptr(closest), _lib.dptr(summary))
+    return dist, face, closest, summary
+
+
+def _signed_call(h, queries, n_resident=0, want_dist=True, want_face=False, want_closest=False):
+    """``_surface_call(..., signed=True)``: (sdist, face, closest, volume)."""
+    return _surface_call(h, queries, n_resident, want_dist, want_face, want_closest, signed=True)
+
+
+def _surface_distances(h, queries, n_resident, signed, return_face, return_closest):
+    """The return value of the ``surface_distance`` methods: dist, or (dist[, face][, closest])."""
+    dist, face, closest, _ = _surface_call(h, queries, n_resident, True, return_face, return_closest, signed=signed)
+    if not (return_face or return_closest):
+        return dist
+    return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
 
 
 def _upload_surface(h, mesh):
@@ -158,16 +162,10 @@ def surface_distance(mesh, points, handle=None, return_face=False, return_closes
     h = handle if handle is not None else _lib.Handle(0)
     try:
         _upload_surface(h, mesh)
-        if signed:
-            dist, face, closest, _ = _signed_call(h, points, 0, True, return_face, return_closest)
-        else:
-            dist, face, closest, _ = _surface_call(h, points, 0, True, return_face, return_closest)
+        return _surface_distances(h, points, 0, signed, return_face, return_closest)
     finally:
         if handle is None:
             h.close()
-    if not (return_face or return_closest):
-        return dist
-    return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
 
 
 def enclosed_volume(mesh, handle=None):

@@ -332,13 +332,9 @@ class ShrinkwrapMeshConjGrad(object):
         float64.  ``points=None``: the fit's own localisations, which are already resident (nothing is uploaded), in the order
         they were given.  ``return_face`` / ``return_closest`` / ``signed`` as ``evaluation_utils.surface_distance``.  This
         measures the surface itself; the fit's weights keep using the nearest face centroid (mesh_conj_grad.py:451-454)."""
-        from .evaluation_utils import _signed_call, _surface_call
+        from .evaluation_utils import _surface_distances
         self._ensure_ready()
-        call = _signed_call if signed else _surface_call
-        dist, face, closest, _ = call(self._h, points, self._session.P, True, return_face, return_closest)
-        if not (return_face or return_closest):
-            return dist
-        return (dist,) + ((face,) if return_face else ()) + ((closest,) if return_closest else ())
+        return _surface_distances(self._h, points, self._session.P, signed, return_face, return_closest)
 
     def _ncc(self):
         self._ensure_weights()

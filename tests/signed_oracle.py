@@ -1,9 +1,9 @@
 """CPU restatement of nw_surface_signed_distance (ch_shrinkwrap_b200/csrc/surface.cu), test infrastructure only.
 
-The region of the winning face by the operations of surface_oracle.closest_point_triangle, the twin table, the vertex ->
-face CSR and the defect counts by plain numpy, the vertex pseudonormals with np.arctan2, the sign and the signed volume in
-the device's reduction order.  The independent truth is the generalised winding number (solid angles by van Oosterom &
-Strackee), brute force over all faces, plus a few small closed test solids."""
+The region of the winning face from surface_oracle.closest_point_region, the twin table, the vertex -> face CSR and the
+defect counts by plain numpy, the vertex pseudonormals with np.arctan2, the sign and the signed volume in the device's
+reduction order.  The independent truth is the generalised winding number (solid angles by van Oosterom & Strackee), brute
+force over all faces, plus a few small closed test solids."""
 from __future__ import annotations
 
 import math
@@ -11,8 +11,7 @@ import math
 import numpy as np
 
 import surface_oracle as orc
-
-CORNER, EDGE = 1, 4                      # region codes: 0 interior, CORNER + k corner k, EDGE + k the edge corner k -> k + 1
+from surface_oracle import CORNER, EDGE
 
 
 def _cross(u, v):
@@ -22,57 +21,10 @@ def _cross(u, v):
 
 def _unit_normal(a, b, c):
     cr = _cross(b - a, c - a)
-    l2 = orc._dot(cr, cr)
+    l2 = orc.dot(cr, cr)
     with np.errstate(divide='ignore', invalid='ignore'):
         n = cr / np.sqrt(l2)[:, None]
     return np.where((l2 > 0.0)[:, None], n, 0.0)
-
-
-def _segment_region(p, p0, p1, k):
-    e = p1 - p0
-    ee = orc._dot(e, e)
-    with np.errstate(divide='ignore', invalid='ignore'):
-        t = np.where(ee > 0.0, orc._dot(p - p0, e) / ee, 0.0)
-    t = np.fmin(np.fmax(t, 0.0), 1.0)
-    return np.where(t == 0.0, CORNER + k, np.where(t == 1.0, CORNER + (k + 1) % 3, EDGE + k))
-
-
-def _edges_region(p, a, b, c):
-    best = orc._closest_on_segment(p, a, b)
-    bd = orc._dist2(p, best)
-    r = _segment_region(p, a, b, 0)
-    for k, (u, v) in ((1, (b, c)), (2, (c, a))):
-        x = orc._closest_on_segment(p, u, v)
-        kd = orc._dist2(p, x)
-        m = kd < bd
-        best = np.where(m[:, None], x, best)
-        bd = np.where(m, kd, bd)
-        r = np.where(m, _segment_region(p, u, v, k), r)
-    return r
-
-
-def triangle_region(p, a, b, c):
-    """(closest point, region code) row by row: closest_point_triangle's precedence of regions, same bits."""
-    ab, ac = b - a, c - a
-    degenerate = ((ab[:, 1] * ac[:, 2] - ab[:, 2] * ac[:, 1] == 0.0) & (ab[:, 2] * ac[:, 0] - ab[:, 0] * ac[:, 2] == 0.0)
-                  & (ab[:, 0] * ac[:, 1] - ab[:, 1] * ac[:, 0] == 0.0))
-    ap, bp, cp = p - a, p - b, p - c
-    d1, d2 = orc._dot(ab, ap), orc._dot(ac, ap)
-    d3, d4 = orc._dot(ab, bp), orc._dot(ac, bp)
-    d5, d6 = orc._dot(ab, cp), orc._dot(ac, cp)
-    vc = d1 * d4 - d3 * d2
-    vb = d5 * d2 - d1 * d6
-    va = d3 * d6 - d5 * d4
-    s = va + vb + vc
-    edges = _edges_region(p, a, b, c)
-    r = np.where(s > 0.0, 0, edges)
-    r = np.where((va <= 0.0) & ((d4 - d3) >= 0.0) & ((d5 - d6) >= 0.0), EDGE + 1, r)
-    r = np.where((vb <= 0.0) & (d2 >= 0.0) & (d6 <= 0.0), EDGE + 2, r)
-    r = np.where((d6 >= 0.0) & (d5 <= d6), CORNER + 2, r)
-    r = np.where((vc <= 0.0) & (d1 >= 0.0) & (d3 <= 0.0), EDGE + 0, r)
-    r = np.where((d3 >= 0.0) & (d4 <= d3), CORNER + 1, r)
-    r = np.where((d1 <= 0.0) & (d2 <= 0.0), CORNER + 0, r)
-    return orc.closest_point_triangle(p, a, b, c), np.where(degenerate, edges, r)
 
 
 def tables(faces, M, fans=True):
@@ -133,7 +85,7 @@ def pseudonormals(vertices, faces, voff, vface):
     p, a, b = pick(0), pick(1), pick(2)
     uu, ww = a - p, b - p
     uw = _cross(uu, ww)
-    th = np.arctan2(np.sqrt(orc._dot(uw, uw)), orc._dot(uu, ww))
+    th = np.arctan2(np.sqrt(orc.dot(uw, uw)), orc.dot(uu, ww))
     contrib = th[:, None] * nf
     N = np.zeros((M, 3))
     for j in range(int(cnt.max(initial=0))):         # in the device's order: entry j of every vertex that has one
@@ -151,7 +103,7 @@ def volume_terms(vertices, faces):
     o = ((used.min(0) + used.max(0)) * np.float32(0.5)).astype(np.float64)
     v = v32.astype(np.float64)
     a, b, c = v[f[:, 0]] - o, v[f[:, 1]] - o, v[f[:, 2]] - o
-    return orc._dot(a, _cross(b, c)) / 6.0
+    return orc.dot(a, _cross(b, c)) / 6.0
 
 
 def fixed_order_sum(terms, blocks=256, threads=256):
@@ -191,7 +143,7 @@ def signed_distance(points, vertices, faces):
     v = v32.astype(np.float64)
     fr = f[face[ok]]
     x = [v[fr[:, j]] for j in range(3)]
-    c, r = triangle_region(q[ok], *x)
+    c, r = orc.closest_point_region(q[ok], *x)
     N = _cross(x[1] - x[0], x[2] - x[0])
     corner = (r >= CORNER) & (r < EDGE)
     N[corner] = N_v[fr[corner, r[corner] - CORNER]]
@@ -207,12 +159,12 @@ def signed_distance(points, vertices, faces):
         lower = (fi < g)[:, None]
         N[edge] = np.where(lower, nf, ng) + np.where(lower, ng, nf)
     qc = q[ok] - c
-    s = orc._dot(qc, N)
+    s = orc.dot(qc, N)
     sd = np.full(len(q), np.nan)
     sd[ok] = np.where(d[ok] == 0.0, 0.0, np.where(s == 0.0, np.nan, np.where((s > 0.0) == (V > 0.0), d[ok], -d[ok])))
     margin = np.full(len(q), np.nan)
     with np.errstate(divide='ignore', invalid='ignore'):
-        margin[ok] = np.abs(s) / (np.sqrt(orc._dot(qc, qc)) * np.sqrt(orc._dot(N, N)))
+        margin[ok] = np.abs(s) / (np.sqrt(orc.dot(qc, qc)) * np.sqrt(orc.dot(N, N)))
     region = np.full(len(q), -1)
     region[ok] = r
     return sd, face, closest, abs(V), margin, region
@@ -225,9 +177,9 @@ def face_normal_side(points, vertices, faces, face):
     v = v32.astype(np.float64)
     f = np.asarray(faces, np.int64)[face]
     x = [v[f[:, j]] for j in range(3)]
-    c, _ = triangle_region(q, *x)
+    c = orc.closest_point_triangle(q, *x)
     V = math.fsum(volume_terms(v32, faces))
-    return np.sign(orc._dot(q - c, _cross(x[1] - x[0], x[2] - x[0]))) * np.sign(V)
+    return np.sign(orc.dot(q - c, _cross(x[1] - x[0], x[2] - x[0]))) * np.sign(V)
 
 
 def winding_number(points, vertices, faces, chunk=1 << 22):
@@ -260,7 +212,7 @@ def _outward(v, f):
     v64 = v.astype(np.float64)
     ctr = v64.mean(0)
     a, b, c = v64[f[:, 0]], v64[f[:, 1]], v64[f[:, 2]]
-    flip = orc._dot(_cross(b - a, c - a), (a + b + c) / 3.0 - ctr) < 0.0
+    flip = orc.dot(_cross(b - a, c - a), (a + b + c) / 3.0 - ctr) < 0.0
     f = f.copy()
     f[flip] = f[flip][:, [0, 2, 1]]
     return f

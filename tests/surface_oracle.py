@@ -1,56 +1,62 @@
 """CPU restatement of nw_surface_distance (ch_shrinkwrap_b200/csrc/surface.cu), test infrastructure only.
 
 The library's exact point-to-triangle routine restated in numpy, operation for operation in fp64 (the library compiles it
-with -fmad=false), so that distances, closest points and faces compare bit for bit; plus a brute-force nearest face with the
-same tie rule.  Not a reference feature, so it lives beside the tests rather than in the reference oracle (oracle/)."""
+with -fmad=false), so that distances, closest points and faces compare bit for bit; with the region code of the closest
+point, which the signed distance (signed_oracle.py) reads.  Plus a brute-force nearest face with the same tie rule.  Not a
+reference feature, so it lives beside the tests rather than in the reference oracle (oracle/)."""
 from __future__ import annotations
 
 import numpy as np
 import scipy.spatial
 
 
-def _dot(u, v):
+CORNER, EDGE = 1, 4                      # region codes: 0 interior, CORNER + k corner k, EDGE + k the edge corner k -> k + 1
+
+
+def dot(u, v):
     return (u[:, 0] * v[:, 0] + u[:, 1] * v[:, 1]) + u[:, 2] * v[:, 2]
 
 
 def _dist2(p, c):
     d = p - c
-    return _dot(d, d)
+    return dot(d, d)
 
 
-def _closest_on_segment(p, p0, p1):
+def _closest_on_segment(p, p0, p1, k):
+    """(closest point, region code) on the segment p0 -> p1, taken as edge k of a triangle."""
     e = p1 - p0
-    ee = _dot(e, e)
+    ee = dot(e, e)
     with np.errstate(divide='ignore', invalid='ignore'):
-        t = np.where(ee > 0.0, _dot(p - p0, e) / ee, 0.0)
+        t = np.where(ee > 0.0, dot(p - p0, e) / ee, 0.0)
     t = np.fmin(np.fmax(t, 0.0), 1.0)
-    return p0 + t[:, None] * e
+    return p0 + t[:, None] * e, np.where(t == 0.0, CORNER + k, np.where(t == 1.0, CORNER + (k + 1) % 3, EDGE + k))
 
 
 def _closest_on_edges(p, a, b, c):
     """A zero-area triangle is the union of its edges: the closest of ab, bc, ca (the first wins ties)."""
-    best = _closest_on_segment(p, a, b)
+    best, r = _closest_on_segment(p, a, b, 0)
     bd = _dist2(p, best)
-    for u, v in ((b, c), (c, a)):
-        k = _closest_on_segment(p, u, v)
-        kd = _dist2(p, k)
+    for k, (u, v) in ((1, (b, c)), (2, (c, a))):
+        x, rk = _closest_on_segment(p, u, v, k)
+        kd = _dist2(p, x)
         m = kd < bd
-        best = np.where(m[:, None], k, best)
+        best = np.where(m[:, None], x, best)
         bd = np.where(m, kd, bd)
-    return best
+        r = np.where(m, rk, r)
+    return best, r
 
 
-def closest_point_triangle(p, a, b, c):
-    """Closest point on the closed triangle (a, b, c) to p, row by row, float64 (N,3) arrays: Ericson's region test
-    (Real-Time Collision Detection 5.1.5).  Degenerate: ab x ac is exactly zero, or the interior case finds no positive
-    barycentric denominator; then the closest of the three edges as segments."""
+def closest_point_region(p, a, b, c):
+    """(closest point, region code) on the closed triangle (a, b, c) to p, row by row, float64 (N,3) arrays: Ericson's
+    region test (Real-Time Collision Detection 5.1.5).  Degenerate: ab x ac is exactly zero, or the interior case finds no
+    positive barycentric denominator; then the closest of the three edges as segments."""
     ab, ac = b - a, c - a
     degenerate = ((ab[:, 1] * ac[:, 2] - ab[:, 2] * ac[:, 1] == 0.0) & (ab[:, 2] * ac[:, 0] - ab[:, 0] * ac[:, 2] == 0.0)
                   & (ab[:, 0] * ac[:, 1] - ab[:, 1] * ac[:, 0] == 0.0))
     ap, bp, cp = p - a, p - b, p - c
-    d1, d2 = _dot(ab, ap), _dot(ac, ap)
-    d3, d4 = _dot(ab, bp), _dot(ac, bp)
-    d5, d6 = _dot(ab, cp), _dot(ac, cp)
+    d1, d2 = dot(ab, ap), dot(ac, ap)
+    d3, d4 = dot(ab, bp), dot(ac, bp)
+    d5, d6 = dot(ab, cp), dot(ac, cp)
     vc = d1 * d4 - d3 * d2
     vb = d5 * d2 - d1 * d6
     va = d3 * d6 - d5 * d4
@@ -62,16 +68,22 @@ def closest_point_triangle(p, a, b, c):
         denom = 1.0 / s
         v, w = vb * denom, vc * denom
         inner = (a + ab * v[:, None]) + ac * w[:, None]
-    edges = _closest_on_edges(p, a, b, c)
+    edges, edges_r = _closest_on_edges(p, a, b, c)
+    out, r = np.where((s > 0.0)[:, None], inner, edges), np.where(s > 0.0, 0, edges_r)
     # the regions in reverse order of precedence, so that the first that holds is the one left standing
-    out = np.where((s > 0.0)[:, None], inner, edges)
-    out = np.where(((va <= 0.0) & ((d4 - d3) >= 0.0) & ((d5 - d6) >= 0.0))[:, None], on_bc, out)
-    out = np.where(((vb <= 0.0) & (d2 >= 0.0) & (d6 <= 0.0))[:, None], on_ac, out)
-    out = np.where(((d6 >= 0.0) & (d5 <= d6))[:, None], c, out)
-    out = np.where(((vc <= 0.0) & (d1 >= 0.0) & (d3 <= 0.0))[:, None], on_ab, out)
-    out = np.where(((d3 >= 0.0) & (d4 <= d3))[:, None], b, out)
-    out = np.where(((d1 <= 0.0) & (d2 <= 0.0))[:, None], a, out)
-    return np.where(degenerate[:, None], edges, out)
+    for holds, x, code in (((va <= 0.0) & ((d4 - d3) >= 0.0) & ((d5 - d6) >= 0.0), on_bc, EDGE + 1),
+                           ((vb <= 0.0) & (d2 >= 0.0) & (d6 <= 0.0), on_ac, EDGE + 2),
+                           ((d6 >= 0.0) & (d5 <= d6), c, CORNER + 2),
+                           ((vc <= 0.0) & (d1 >= 0.0) & (d3 <= 0.0), on_ab, EDGE + 0),
+                           ((d3 >= 0.0) & (d4 <= d3), b, CORNER + 1),
+                           ((d1 <= 0.0) & (d2 <= 0.0), a, CORNER + 0)):
+        out, r = np.where(holds[:, None], x, out), np.where(holds, code, r)
+    return np.where(degenerate[:, None], edges, out), np.where(degenerate, edges_r, r)
+
+
+def closest_point_triangle(p, a, b, c):
+    """The closest point of ``closest_point_region``."""
+    return closest_point_region(p, a, b, c)[0]
 
 
 def surface_nearest(points, vertices, faces, chunk=1 << 21):
