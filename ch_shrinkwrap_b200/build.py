@@ -11,10 +11,10 @@ CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libnanowrap.so')
 ARCH = ['-gencode', 'arch=compute_100a,code=sm_100a']
 COMMON = ['-O3', '-std=c++17', '-lineinfo', '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr'] + os.environ.get('NW_EXTRA_FLAGS', '').split()
-# curvature.cu, quality.cu and surface.cu need one IEEE operation per source operation (see their headers)
+# curvature.cu, quality.cu, surface.cu and intersect.cu need one IEEE operation per source operation (see their headers)
 SOURCES = {'api.cu': [], 'points.cu': [], 'tree.cu': [], 'sweep.cu': [], 'mesh_ops.cu': [], 'comm.cu': [],
            'ring.cu': [], 'benchhook.cu': [], 'xfer.cu': [], 'curvature.cu': ['-fmad=false'], 'quality.cu': ['-fmad=false'],
-           'surface.cu': ['-fmad=false']}
+           'surface.cu': ['-fmad=false'], 'intersect.cu': ['-fmad=false']}
 
 
 def _nvcc():

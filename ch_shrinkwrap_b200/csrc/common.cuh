@@ -98,6 +98,23 @@ __device__ __forceinline__ void nw_decode_box(Box *b, float w) {
     b->d.w = ord2f(__float_as_int(b->d.w)) - w; b->c.w = ord2f(__float_as_int(b->c.w)) + w;
 }
 
+// projection onto a node frame as the box stores it (t2 = c.xyz): the operations of the search's node test (sweep.cu)
+__device__ __forceinline__ void project_frame(const float4 a, const float4 b, const float4 c, float x, float y, float z, float &pn,
+                                              float &p1, float &p2) {
+    pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
+    p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
+    p2 = fmaf(c.x, x, fmaf(c.y, y, c.z * z));
+}
+
+// The slack of the triangle-bounded boxes (surface.cu: nw_surface_boxes): 2^-19 x the L1 bound of everything that is
+// projected (the vertices, bits 0..2, and the queries, bits 3..5; zero without queries) -- the rule of tree.cu's k_box_decode,
+// whose coord_l1 covers the fit's vertices and points only.  Queries given explicitly can lie much farther out than either.
+__device__ __forceinline__ float call_slack(const unsigned *__restrict__ bits6) {
+    float l1 = 0.f;
+    for (int k = 0; k < 3; ++k) l1 += fmaxf(__uint_as_float(bits6[k]), __uint_as_float(bits6[3 + k]));
+    return l1 * 1.9073486328125e-6f;
+}
+
 // orthonormal completion of a unit vector (Duff et al. 2017, branchless): returns t1; t2 = n x t1 everywhere.
 // Used identically when boxes are built and when they are tested.
 __host__ __device__ __forceinline__ float3 nw_tangent_of(const float nx, const float ny, const float nz) {
@@ -210,6 +227,12 @@ struct nw_ctx {
     double *sgn_nv = nullptr;                    // 3M: angle-weighted vertex pseudonormals at the current positions
     double *sgn_vpart = nullptr;                 // signed-volume partials, then the volume
     unsigned *sgn_bbox = nullptr;                // ordered-uint min xyz, max xyz of the vertices the faces use
+    // ---- nw_self_intersections (intersect.cu): only that call (and tboxes / surf_bits, see above) touches these ----
+    uint8_t *sx_flag = nullptr;                  // per sorted slot: 0 tested, 1 degenerate, 2 a non-finite corner
+    int *sx_last = nullptr;                      // per global node id: its last slot
+    unsigned long long *sx_keys = nullptr, *sx_sorted = nullptr;   // (f << 32) | g of every pair found, then sorted
+    unsigned long long *sx_cnt = nullptr;        // pairs found, then the 4 statistics of nw_self_intersections
+    int2 *sx_pairs = nullptr;                    // the sorted pairs as (f, g)
     // ---- solver vectors ----
     unsigned long long *acc = nullptr;           // (M,4) int64 fixed point: AH res xyz, AH 1
     float4 *Sq = nullptr;                        // search directions, interleaved: S_k of vertex v at Sq[3v + k] (48 B per vertex)
@@ -368,3 +391,7 @@ int nw_allreduce_scalars(nw_ctx *h);
 int nw_comm_agree(nw_ctx *h);
 int nw_set_acc_shifts(nw_ctx *h);
 int nw_curvature_relaunch(nw_ctx *h);
+int nw_mesh_check(nw_ctx *h, const std::string &who);   // surface.cu: a mesh topology is loaded (not point targets)
+// surface.cu: h->surf_bits (the slack of the call: the vertices, and Q queries q?[i * stride] when Q > 0) and h->tboxes (the
+// triangle-bounded boxes at the current positions)
+int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, int64_t Q, int64_t stride, bool f64);

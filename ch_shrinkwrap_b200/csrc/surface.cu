@@ -19,6 +19,10 @@
 // side of q - c against the angle-weighted pseudonormal of that feature (face, edge or vertex; Baerentzen & Aanaes 2005),
 // oriented by the sign of the mesh's signed volume.  Its edge and vertex tables are built once per topology
 // (signed_tables), lazily, so nw_set_topology* does no extra work.
+//
+// The slack and the triangle-bounded boxes are built by nw_surface_boxes, which nw_self_intersections (intersect.cu) calls
+// too: its broad phase walks the same boxes with a face instead of a query.  Distances and inside/outside answers assume an
+// embedded mesh; nw_self_intersections is the check for faces that cross or touch.
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -27,15 +31,7 @@
 
 namespace {
 
-// projection onto a node frame as the box stores it (t2 = c.xyz): the operations of the search's node test (sweep.cu)
-__device__ __forceinline__ void project_frame(const float4 a, const float4 b, const float4 c, float x, float y, float z, float &pn,
-                                              float &p1, float &p2) {
-    pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
-    p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
-    p2 = fmaf(c.x, x, fmaf(c.y, y, c.z * z));
-}
-
-// ---- rounding slack of the call -----------------------------------------------------------------------------------
+// ---- rounding slack of the call (common.cuh: call_slack) -----------------------------------------------------------
 // per-axis max |coordinate| over the finite values, as the bits of non-negative floats (which order like unsigned ints)
 __device__ __forceinline__ float abs_up(float v) { return fabsf(v); }
 __device__ __forceinline__ float abs_up(double v) { return __double2float_ru(fabs(v)); }
@@ -51,14 +47,6 @@ __global__ void __launch_bounds__(256) k_absmax3(const T *__restrict__ x, const 
         const unsigned r = __reduce_max_sync(0xffffffffu, __float_as_uint(m[k]));
         if ((threadIdx.x & 31) == 0 && r) atomicMax(out3 + k, r);
     }
-}
-// The slack of the box test: 2^-19 x the L1 bound of everything that is projected (the vertices, bits 0..2, and the queries,
-// bits 3..5) -- the rule of tree.cu's k_box_decode, whose coord_l1 covers the fit's vertices and points only.  Queries given
-// explicitly can lie much farther out than either.
-__device__ __forceinline__ float call_slack(const unsigned *__restrict__ bits6) {
-    float l1 = 0.f;
-    for (int k = 0; k < 3; ++k) l1 += fmaxf(__uint_as_float(bits6[k]), __uint_as_float(bits6[3 + k]));
-    return l1 * 1.9073486328125e-6f;
 }
 
 // ---- triangle-bounded boxes ------------------------------------------------------------------------------------------
@@ -550,14 +538,49 @@ __global__ void __launch_bounds__(128) k_surface_sign(const __grid_constant__ Si
 
 }  // namespace
 
+// the handle holds a mesh: the rule of every call that measures the mesh itself (this file, intersect.cu)
+int nw_mesh_check(nw_ctx *h, const std::string &w) {
+    NW_ARG(h->M > 0 && h->F > 0 && h->tl.n_levels > 1, w + ": no topology (call nw_set_topology first)");
+    NW_ARG(!h->points_mode, w + ": the handle holds point targets (nw_set_point_targets), not a mesh");
+    return NW_OK;
+}
+
 // arguments shared by both entry points
 static int surface_check(nw_ctx *h, const char *who, const void *q, int64_t Q) {
     const std::string w(who);
-    NW_ARG(h->M > 0 && h->F > 0 && h->tl.n_levels > 1, w + ": no topology (call nw_set_topology first)");
-    NW_ARG(!h->points_mode, w + ": the handle holds point targets (nw_set_point_targets), not a mesh");
+    NW_CHECK(nw_mesh_check(h, w));
     if (q) NW_ARG(Q >= 0 && Q < 2147483647LL, w + ": Q must be in [0, 2^31)");
     else NW_ARG(Q == h->P && (h->px != nullptr || h->P == 0),
                 w + ": q == NULL measures the resident points; Q must equal their number (nw_set_points)");
+    return NW_OK;
+}
+
+// The slack of the call, then the triangle-bounded boxes at the current positions.  Q == 0: the vertices' slack alone
+// (nw_self_intersections has no queries).
+int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, int64_t Q, int64_t stride, bool f64) {
+    cudaStream_t s = h->stream;
+    const int B = 256;
+    const TreeLevels &tl = h->tl;
+    const int leaf_level = tl.n_levels - 1, leaf0 = tl.off[leaf_level], total = leaf0 + tl.count[leaf_level];
+    NW_CHECK(nw_alloc(h, &h->surf_bits, (size_t)8));
+    NW_CUDA(cudaMemsetAsync(h->surf_bits, 0, sizeof(unsigned) * 6, s));
+    const float *pq = (const float *)h->posq;      // x, y, z of vertex v at pq[4 v + 0..2]
+    k_absmax3<float><<<std::min(nw_grid(h->M, B), 148 * 4), B, 0, s>>>(pq, pq + 1, pq + 2, h->M, 4, h->surf_bits);
+    NW_LAUNCH_CHECK();
+    if (Q > 0) {
+        if (f64) k_absmax3<double><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const double *)qx, (const double *)qy,
+                                                                                  (const double *)qz, Q, stride, h->surf_bits + 3);
+        else k_absmax3<float><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const float *)qx, (const float *)qy, (const float *)qz,
+                                                                            Q, stride, h->surf_bits + 3);
+        NW_LAUNCH_CHECK();
+    }
+    NW_CHECK(nw_alloc(h, &h->tboxes, (size_t)total));
+    k_tbox_init<<<nw_grid(total, B), B, 0, s>>>(h->boxes, total, h->tboxes);
+    NW_LAUNCH_CHECK();
+    k_tri_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->sfaces, h->posq, h->F, h->leaf_of_slot, leaf0, leaf_level, h->parent_g, h->tboxes);
+    NW_LAUNCH_CHECK();
+    k_tbox_decode<<<nw_grid(total - tl.off[1], B), B, 0, s>>>(h->tboxes, tl.off[1], total - tl.off[1], h->surf_bits);
+    NW_LAUNCH_CHECK();
     return NW_OK;
 }
 
@@ -566,7 +589,6 @@ static int surface_check(nw_ctx *h, const char *who, const void *q, int64_t Q) {
 static int surface_walk(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, bool want_face, bool want_closest, SurfaceArgs &a,
                         bool &f64) {
     cudaStream_t s = h->stream;
-    const int B = 256;
     const TreeLevels &tl = h->tl;
     const int leaf_level = tl.n_levels - 1, leaf0 = tl.off[leaf_level], total = leaf0 + tl.count[leaf_level];
 
@@ -587,26 +609,7 @@ static int surface_walk(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, bool 
         a.perm = h->perm; a.seed = h->slot;
     }
 
-    // slack of the call, then the triangle-bounded boxes at the current positions
-    NW_CHECK(nw_alloc(h, &h->surf_bits, (size_t)8));
-    NW_CUDA(cudaMemsetAsync(h->surf_bits, 0, sizeof(unsigned) * 6, s));
-    const float *pq = (const float *)h->posq;      // x, y, z of vertex v at pq[4 v + 0..2]
-    k_absmax3<float><<<std::min(nw_grid(h->M, B), 148 * 4), B, 0, s>>>(pq, pq + 1, pq + 2, h->M, 4, h->surf_bits);
-    NW_LAUNCH_CHECK();
-    if (Q > 0) {
-        if (f64) k_absmax3<double><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const double *)a.qx, (const double *)a.qy,
-                                                                                  (const double *)a.qz, Q, a.stride, h->surf_bits + 3);
-        else k_absmax3<float><<<std::min(nw_grid(Q, B), 148 * 4), B, 0, s>>>((const float *)a.qx, (const float *)a.qy, (const float *)a.qz,
-                                                                            Q, a.stride, h->surf_bits + 3);
-        NW_LAUNCH_CHECK();
-    }
-    NW_CHECK(nw_alloc(h, &h->tboxes, (size_t)total));
-    k_tbox_init<<<nw_grid(total, B), B, 0, s>>>(h->boxes, total, h->tboxes);
-    NW_LAUNCH_CHECK();
-    k_tri_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->sfaces, h->posq, h->F, h->leaf_of_slot, leaf0, leaf_level, h->parent_g, h->tboxes);
-    NW_LAUNCH_CHECK();
-    k_tbox_decode<<<nw_grid(total - tl.off[1], B), B, 0, s>>>(h->tboxes, tl.off[1], total - tl.off[1], h->surf_bits);
-    NW_LAUNCH_CHECK();
+    NW_CHECK(nw_surface_boxes(h, a.qx, a.qy, a.qz, Q, a.stride, f64));
 
     // the search
     const size_t nq = (size_t)std::max<int64_t>(Q, 1);

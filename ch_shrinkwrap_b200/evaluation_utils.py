@@ -16,6 +16,8 @@ Not in the reference (its surface metrics compare sample clouds, so their answer
 * ``surface_distance(mesh, points, signed=True)`` -- the same distance, negative inside a closed mesh and positive outside
   (``nw_surface_signed_distance``: the angle-weighted pseudonormal of the nearest feature, oriented by the signed volume).
 * ``enclosed_volume(mesh)`` -- the volume a closed mesh encloses.
+* ``self_intersections(mesh)`` -- the pairs of faces that cross or touch beyond their shared vertices and edges, exactly
+  (``nw_self_intersections``); none means the mesh is embedded, which the two calls above assume.
 * ``hausdorff_distance(mesh0, mesh1, dx_min)`` -- one-sided and symmetric Hausdorff and mean distances between two meshes,
   from exact point-to-surface distances of each mesh's samples.
 
@@ -153,7 +155,8 @@ def surface_distance(mesh, points, handle=None, return_face=False, return_closes
     point are those of the unsigned call.  The side comes from the angle-weighted pseudonormal of the nearest face, edge or
     vertex, and "inside" from the sign of the mesh's signed volume, so either winding gives the same answer.  The mesh must
     be closed, edge-manifold and consistently oriented (ValueError with the defect counts otherwise); a mesh whose separate
-    components are oriented against each other is not supported.
+    components are oriented against each other is not supported.  It must also be embedded: on a mesh whose faces cross or
+    fold over each other the signs are meaningless, and no check here sees that; ``self_intersections`` does.
 
     ``return_face``: also the row of ``mesh.faces`` of the nearest triangle (int32; exact fp64 ties go to the lowest row);
     ``return_closest``: also the closest point on it ((N,3) float64).  Float32 points are used exactly, float64 points as
@@ -171,11 +174,52 @@ def surface_distance(mesh, points, handle=None, return_face=False, return_closes
 def enclosed_volume(mesh, handle=None):
     """The volume enclosed by a closed, edge-manifold, consistently oriented mesh (float64, either winding): the absolute
     value of the signed volume sum_f dot(a - o, (b - o) x (c - o)) / 6 over the faces (a, b, c), reduced on the GPU in a
-    fixed order.  Raises ValueError for a mesh that does not bound a solid, as ``surface_distance(signed=True)`` does."""
+    fixed order.  Raises ValueError for a mesh that does not bound a solid, as ``surface_distance(signed=True)`` does.  A
+    self-intersecting mesh passes those checks and gets a meaningless volume; ``self_intersections`` is the check."""
     h = handle if handle is not None else _lib.Handle(0)
     try:
         _upload_surface(h, mesh)
         return _signed_call(h, np.zeros((0, 3), np.float32), want_dist=False)[3]
+    finally:
+        if handle is None:
+            h.close()
+
+
+IntersectionStats = namedtuple('IntersectionStats', 'candidates exact degenerate non_finite')
+
+
+def _self_intersections(h, return_stats=False, capacity=1024):
+    """nw_self_intersections on handle `h`: (n, 2) int32 face-row pairs f < g sorted by (f, g)[, IntersectionStats].  Calls
+    again with the exact capacity only when the first guess was too small."""
+    n = ctypes.c_int64(0)
+    stats = np.zeros(4, np.int64)
+    sp = stats.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
+    pairs = np.empty((capacity, 2), np.int32)
+    h.call('nw_self_intersections', _lib.iptr(pairs), capacity, ctypes.byref(n), sp)
+    if n.value > capacity:
+        pairs = np.empty((n.value, 2), np.int32)
+        h.call('nw_self_intersections', _lib.iptr(pairs), n.value, ctypes.byref(n), sp)
+    pairs = np.ascontiguousarray(pairs[:n.value])
+    return (pairs, IntersectionStats(*(int(x) for x in stats))) if return_stats else pairs
+
+
+def self_intersections(mesh, handle=None, return_stats=False):
+    """The pairs of faces of `mesh` that intersect: an (n, 2) int32 array of rows of ``mesh.faces``, f < g, sorted by (f, g).
+
+    Two faces intersect when their closed triangles share a point that their shared vertex indices do not explain: faces with
+    no common vertex must not touch at all; faces sharing one vertex must meet only there; faces sharing an edge are reported
+    when they are coplanar and fold over each other; faces with the same three vertices always.  Degenerate faces (collinear
+    corners, a repeated vertex included) and faces with a non-finite corner are not tested.  The answer is exact for the
+    float32 positions (every decision is the exactly evaluated sign of an orientation determinant), so it does not depend on
+    the winding, the order of the faces or a power-of-two scale.  The mesh need not be closed or manifold.
+
+    ``return_stats``: also an ``IntersectionStats(candidates, exact, degenerate, non_finite)``: the face pairs whose boxes
+    overlapped, the orientation signs that needed the exact stage, and the faces left out.  An empty result means the mesh is
+    embedded, which ``surface_distance(signed=True)`` and ``enclosed_volume`` assume."""
+    h = handle if handle is not None else _lib.Handle(0)
+    try:
+        _upload_surface(h, mesh)
+        return _self_intersections(h, return_stats)
     finally:
         if handle is None:
             h.close()

@@ -189,6 +189,13 @@ class ShrinkwrapMeshMixin:
             raise RuntimeError('point_surface_distance: no fit on this mesh yet (self.cg is None)')
         return self.cg.surface_distance(points, return_face=return_face, return_closest=return_closest, signed=signed)
 
+    def self_intersections(self, return_stats=False):
+        """The pairs of faces of the fitted surface that cross or touch beyond their shared vertices and edges ((n, 2) int32
+        rows of ``faces``); see ``evaluation_utils.self_intersections``.  Runs on the fit's handle, nothing is uploaded."""
+        if self.cg is None:
+            raise RuntimeError('self_intersections: no fit on this mesh yet (self.cg is None)')
+        return self.cg.self_intersections(return_stats=return_stats)
+
     @property
     def rms_point_sc(self):
         res = self.cg.res

@@ -336,6 +336,13 @@ class ShrinkwrapMeshConjGrad(object):
         self._ensure_ready()
         return _surface_distances(self._h, points, self._session.P, signed, return_face, return_closest)
 
+    def self_intersections(self, return_stats=False):
+        """The intersecting face pairs of the mesh as it stands on the device (after ``search``, the fitted surface), with
+        nothing uploaded: see ``evaluation_utils.self_intersections``.  The fit's own state is not touched."""
+        from .evaluation_utils import _self_intersections
+        self._ensure_ready()
+        return _self_intersections(self._h, return_stats)
+
     def _ncc(self):
         self._ensure_weights()
         fd = np.empty((self.M, 3), np.float64)

@@ -195,6 +195,18 @@ int nw_surface_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, doubl
  * the mesh and returns the volume only.  Any output may be NULL.  NW_ERR_ARG in points mode; no collectives. */
 int nw_surface_signed_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *sdist, int32_t *face,
                                double *closest, double *volume);
+/* Self-intersections of the handle's current mesh (the topology of the last nw_set_topology*, at the current f -- after
+ * nw_search, the fitted surface).  Faces f < g (rows of mesh.faces) are reported when their closed triangles share a point
+ * that their shared vertex indices do not explain: with none shared, any common point (touching counts); with one shared
+ * vertex s, the edge of either face opposite s meets the other closed face; with a shared edge, the opposite corners are
+ * coplanar with it and strictly on the same side (a fold-over); with three, always.  Degenerate faces (exactly collinear
+ * corners, a repeated vertex included) and faces with a non-finite corner are not tested.  Exact (every decision is the sign
+ * of orient3d / orient2d of the float32 positions), sorted by (f, g), independent of scheduling.  *n_pairs = the number of
+ * pairs; the first min(n, capacity) go to pairs (capacity x 2 int32); pairs may be NULL with capacity 0 (count only).
+ * stats (or NULL) = {candidate pairs that passed the box test, predicate evaluations the fp64 filter left to the exact
+ * stage, degenerate faces, faces with a non-finite corner}.  The signed distance and the enclosed volume assume no such
+ * pair.  Changes nothing that nw_search reads.  NW_ERR_ARG in points mode or without a topology; no collectives. */
+int nw_self_intersections(nw_ctx *h, int32_t *pairs, int64_t capacity, int64_t *n_pairs, int64_t stats[4]);
 
 /* ---- measurement hooks (bench.py / profiling; not part of the reference surface) ------------------ */
 /* device-resident single-kernel launches on the handle's stream, for CUDA-event timing */
