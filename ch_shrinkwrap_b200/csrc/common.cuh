@@ -31,7 +31,7 @@
 
 struct Box {
     float4 a;   // n.x t1.x | n.y t1.y            the search decides most nodes from a, b, d alone (normal + first tangent axis,
-    float4 b;   // n.z t1.z | n-min t1-min        sweep.cu: test_node) and loads c only for the rest; the two axes are interleaved
+    float4 b;   // n.z t1.z | n-min t1-min        sweep.cu: Traversal::open) and loads c only for the rest; the two axes are interleaved
     float4 c;   // t2.x t2.y t2.z | t2-max        so that each (n, t1) pair is an aligned register pair (packed FFMA2 experiment)
     float4 d;   // n-max t1-max | first child (leaf: first slot) | (node is a last child) << 31, as int bits | t2-min
     __host__ __device__ __forceinline__ float3 normal() const { return make_float3(a.x, a.z, b.x); }
@@ -43,6 +43,10 @@ struct Box {
     __host__ __device__ __forceinline__ float lo(int k) const { return k == 0 ? b.z : k == 1 ? b.w : d.w; }
     __host__ __device__ __forceinline__ float hi(int k) const { return k == 0 ? d.x : k == 1 ? d.y : c.w; }
 };              // 64 B
+
+// The node links tree.cu writes (k_level_tables): Box::d.z = first child (leaf: first slot) | (node is a last child) << 31,
+// parent_g[g] = parent | (the parent is a last child) << 31.  A negative link carries the last-child bit; this is its node.
+__host__ __device__ __forceinline__ int nw_link_node(int link) { return link & 0x7fffffff; }
 
 // Ordered-int encoding of floats: f2ord orders like the floats as signed ints, f2u as unsigned ints, so interval ends can be
 // merged with integer atomics and REDUX.  The box intervals hold f2ord bits while they are being measured.
@@ -128,6 +132,63 @@ struct TreeLevels {
     int count[NW_MAX_LEVELS];     // nodes per level
     int off[NW_MAX_LEVELS];       // global id of the first node of the level: levels are stored back to back, root = 0
 };
+
+// The octree tables a search walks (tree.cu), over one array of boxes: the fit's (h->boxes, intervals over the centroids) or
+// the triangle-bounded ones (h->tboxes, over the face corners).  Nodes are addressed by ONE global id (levels stored back to
+// back, root = 0, leaves = [leaf0, n_nodes)), so a step needs no per-level offset lookups.  Filled by nw_octree_view.
+struct OctreeView {
+    const Box *__restrict__ boxes;
+    const int *__restrict__ parent;     // global id of the parent | (the parent is the last child of its parent) << 31
+    const int2 *__restrict__ kids;      // inner node: {global id of the first child, children}; leaf: {first slot, members}
+    const int *__restrict__ leaf_of_slot;   // index of the leaf WITHIN the leaf level
+    int leaf0, leaf_level;              // global id of the first leaf; its level (= number of climb steps to the root)
+    int n_nodes, n_slots;               // sizes of boxes[] and of the slot arrays
+};
+
+// Greedy-descent score of a box for the float32 query (x, y, z): the squared gaps, with the squared distance to the box
+// centre as a tie-breaker (several overlapping boxes can contain the query and all have gap 0).  It only steers a descent
+// to a first leaf and never decides a result.
+__device__ __forceinline__ float node_score(const Box *__restrict__ bp, float x, float y, float z) {
+    const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), c = __ldg(&bp->c), d = __ldg(&bp->d);
+    float pn, p1, p2;
+    project_frame(a, b, c, x, y, z, pn, p1, p2);
+    const float g0 = fmaxf(fmaxf(b.z - pn, pn - d.x), 0.f), g1 = fmaxf(fmaxf(b.w - p1, p1 - d.y), 0.f),
+                g2 = fmaxf(fmaxf(d.w - p2, p2 - c.w), 0.f);
+    const float c0 = pn - 0.5f * (b.z + d.x), c1 = p1 - 0.5f * (b.w + d.y), c2 = p2 - 0.5f * (d.w + c.w);
+    return (g0 * g0 + g1 * g1 + g2 * g2) + 1e-4f * (c0 * c0 + c1 * c1 + c2 * c2);
+}
+
+// Depth-first walk of the subtree rooted at node I, without a stack: first child and next sibling come from the node's own
+// link (Box::d.z), the way up from the parent table.  Children are visited in index (= Hilbert) order.  v is an OctreeView,
+// or the fit's TreeView (sweep.cu), which holds the same fields in a layout of its own.  The visitor w gives
+//   bool tick()                  true: stop now (a node budget; constexpr false where there is none)
+//   bool open(int node, int &link)   its node test; it also sets link = the node's Box::d.z bits
+//   void leaf(int node)          the members of an opened leaf
+template <typename W, typename V>
+__device__ __forceinline__ void nw_walk_subtree(W &w, const V &v, int I) {
+    int node = I;
+    while (true) {
+        int link;
+        if (w.tick()) return;
+        NW_ASSERT(node >= 0 && node < v.n_nodes);
+        if (w.open(node, link)) {
+            if (node >= v.leaf0) w.leaf(node);
+            else {
+                node = nw_link_node(link);
+                // (measured at C3 and rejected: an L1 prefetch of all children here, CCTL.PF1 by lanes 0..7 -- the fit's warm
+                // sweep went from 2.17 to 2.53 ms and the first sweep of a fit, whose longest packet runs 16 k steps at
+                // ~1000 cycles each while the average SM is done after 60 % of the launch, did not get shorter)
+                continue;
+            }
+        }
+        while (true) {
+            if (node == I) return;
+            if (link >= 0) { ++node; break; }          // not the last child: next sibling
+            link = __ldg(&v.parent[node]);
+            node = nw_link_node(link);
+        }
+    }
+}
 
 // Scalars produced and consumed on the device inside one search() call.
 struct SolverState {
@@ -286,6 +347,18 @@ struct nw_ctx {
     int rank = 0, nranks = 1;
     int comm_status = 0;                         // error latched inside a collective sequence (nw_comm_agree)
 };
+
+// The handle's octree over `boxes` (h->boxes or h->tboxes); a handle without a tree yet gives an empty one.
+static inline OctreeView nw_octree_view(const nw_ctx *h, const Box *boxes) {
+    const TreeLevels &tl = h->tl;
+    OctreeView v;
+    v.boxes = boxes; v.parent = h->parent_g; v.kids = h->kids; v.leaf_of_slot = h->leaf_of_slot;
+    v.leaf_level = tl.n_levels - 1;
+    v.leaf0 = tl.n_levels > 0 ? tl.off[tl.n_levels - 1] : 0;
+    v.n_nodes = tl.n_levels > 0 ? v.leaf0 + tl.count[tl.n_levels - 1] : 0;
+    v.n_slots = h->F;
+    return v;
+}
 
 #define NW_CUDA(call)                                                                      \
     do {                                                                                   \

@@ -12,7 +12,7 @@
 // tested, only counted.
 //
 // Broad phase (k_self_pairs): one thread per sorted face slot walks the triangle-bounded boxes of nw_surface_boxes (the
-// octree of the fit's search, intervals over face corners, surface.cu) with SurfaceWalk::subtree's stackless walk.  A node
+// octree of the fit's search, intervals over face corners, surface.cu) with the stackless walk nw_walk_subtree.  A node
 // is opened when its (widened) intervals overlap those of the face's three corners projected onto its frame with the
 // operations of k_tri_extents, widened by the same slack: a common point projects into both, so the test only prunes.
 // Each pair is visited once, by its lower slot: a node whose slots all lie at or below the thread's own (node slot ranges are
@@ -291,7 +291,7 @@ __global__ void __launch_bounds__(256) k_self_prep(const int4 *__restrict__ sfac
     if (i != k.x + k.y - 1) return;
     last[node] = i;
     while (node != 0) {
-        const int p = parent_g[node] & 0x7fffffff;
+        const int p = nw_link_node(parent_g[node]);
         k = kids[p];
         if (k.x + k.y - 1 != node) break;
         last[p] = i;
@@ -301,15 +301,12 @@ __global__ void __launch_bounds__(256) k_self_prep(const int4 *__restrict__ sfac
 
 // ---- the walk ----------------------------------------------------------------------------------------------------------
 struct SelfArgs {
-    const Box *tb;
-    const int *parent;
-    const int2 *kids;
+    OctreeView oct;                     // over h->tboxes
     const int *last;
     const int4 *sfaces;
     const float4 *pos;
     const uint8_t *flag;
     const unsigned *bits;               // the slack of the call (nw_surface_boxes)
-    int leaf0, n_nodes, F;
     u64 *keys;                          // (f << 32) | g, f < g
     u64 cap;
     u64 *cnt;                           // [0] pairs found, [1] candidates, [2] exact-stage calls
@@ -325,10 +322,10 @@ struct SelfWalk {
     u64 cand = 0, n = 0;
 
     __device__ __forceinline__ SelfWalk(const SelfArgs &a_) : a(a_) {}
+    __device__ __forceinline__ bool tick() const { return false; }
     // the node's intervals overlap those of the face's corners on its frame, each side widened by the slack
     __device__ __forceinline__ bool open(int node, int &link) const {
-        NW_ASSERT(node >= 0 && node < a.n_nodes);
-        const Box *bp = &a.tb[node];
+        const Box *bp = &a.oct.boxes[node];
         const float4 bd = __ldg(&bp->d);
         link = __float_as_int(bd.z);
         if (__ldg(&a.last[node]) <= i) return false;
@@ -344,9 +341,9 @@ struct SelfWalk {
         return l[0] - w <= bd.x && h[0] + w >= bb.z && l[1] - w <= bd.y && h[1] + w >= bb.w && l[2] - w <= bc.w && h[2] + w >= bd.w;
     }
     __device__ __forceinline__ void leaf(int node) {
-        NW_ASSERT(node >= a.leaf0 && node < a.n_nodes);
-        const int2 k = __ldg(&a.kids[node]);
-        NW_ASSERT(k.x >= 0 && k.y >= 0 && k.x + k.y <= a.F);
+        NW_ASSERT(node >= a.oct.leaf0 && node < a.oct.n_nodes);
+        const int2 k = __ldg(&a.oct.kids[node]);
+        NW_ASSERT(k.x >= 0 && k.y >= 0 && k.x + k.y <= a.oct.n_slots);
         for (int s = max(k.x, i + 1); s < k.x + k.y; ++s) {
             if (__ldg(&a.flag[s])) continue;
             const int4 sf = __ldg(&a.sfaces[s]);
@@ -363,33 +360,16 @@ struct SelfWalk {
             if (j < a.cap) a.keys[j] = ((u64)(unsigned)min(face, sf.w) << 32) | (unsigned)max(face, sf.w);
         }
     }
-    // SurfaceWalk::subtree
-    __device__ __forceinline__ void subtree(int I) {
-        int node = I;
-        while (true) {
-            int link;
-            if (open(node, link)) {
-                if (node >= a.leaf0) leaf(node);
-                else { node = link & 0x7fffffff; continue; }
-            }
-            while (true) {
-                if (node == I) return;
-                if (link >= 0) { ++node; break; }
-                link = __ldg(&a.parent[node]);
-                node = link & 0x7fffffff;
-            }
-        }
-    }
     // the root's children in turn (the root has no box: the intervals are measured from level 1 down)
     __device__ __forceinline__ void walk() {
-        const int2 k = __ldg(&a.kids[0]);
-        for (int c = k.x; c < k.x + k.y; ++c) subtree(c);
+        const int2 k = __ldg(&a.oct.kids[0]);
+        for (int c = k.x; c < k.x + k.y; ++c) nw_walk_subtree(*this, a.oct, c);
     }
 };
 
 __global__ void __launch_bounds__(128) k_self_pairs(const __grid_constant__ SelfArgs a) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.F || __ldg(&a.flag[i])) return;
+    if (i >= a.oct.n_slots || __ldg(&a.flag[i])) return;
     SelfWalk w(a);
     w.i = i;
     const int4 sf = __ldg(&a.sfaces[i]);
@@ -419,23 +399,22 @@ extern "C" int nw_self_intersections(nw_ctx *h, int32_t *pairs, int64_t capacity
     NW_ARG(capacity >= 0 && (pairs != nullptr || capacity == 0), "nw_self_intersections: pairs may be NULL only with capacity 0");
     NW_CUDA(cudaSetDevice(h->device));
     cudaStream_t s = h->stream;
-    const TreeLevels &tl = h->tl;
-    const int leaf0 = tl.off[tl.n_levels - 1], total = leaf0 + tl.count[tl.n_levels - 1], F = h->F;
+    const int F = h->F;
 
     NW_CHECK(nw_surface_boxes(h, nullptr, nullptr, nullptr, 0, 1, false));
+    SelfArgs a;
+    a.oct = nw_octree_view(h, h->tboxes);
     NW_CHECK(nw_alloc(h, &h->sx_flag, (size_t)F));
-    NW_CHECK(nw_alloc(h, &h->sx_last, (size_t)total));
+    NW_CHECK(nw_alloc(h, &h->sx_last, (size_t)a.oct.n_nodes));
     NW_CHECK(nw_alloc(h, &h->sx_cnt, (size_t)5));
     NW_CUDA(cudaMemsetAsync(h->sx_cnt, 0, sizeof(u64) * 5, s));
-    k_self_prep<<<nw_grid(F, 256), 256, 0, s>>>(h->sfaces, h->posq, F, h->leaf_of_slot, leaf0, h->parent_g, h->kids, h->sx_flag,
+    k_self_prep<<<nw_grid(F, 256), 256, 0, s>>>(h->sfaces, h->posq, F, h->leaf_of_slot, a.oct.leaf0, h->parent_g, h->kids, h->sx_flag,
                                                 h->sx_last, h->sx_cnt);
     NW_LAUNCH_CHECK();
 
     // pairs into a grow-only buffer; one more pass when it was too small (the set found is the same every time)
     if (!h->sx_keys) NW_CHECK(nw_alloc(h, &h->sx_keys, (size_t)65536));
-    SelfArgs a;
-    a.tb = h->tboxes; a.parent = h->parent_g; a.kids = h->kids; a.last = h->sx_last; a.sfaces = h->sfaces; a.pos = h->posq;
-    a.flag = h->sx_flag; a.bits = h->surf_bits; a.leaf0 = leaf0; a.n_nodes = total; a.F = F;
+    a.last = h->sx_last; a.sfaces = h->sfaces; a.pos = h->posq; a.flag = h->sx_flag; a.bits = h->surf_bits;
     a.keys = h->sx_keys; a.cap = h->caps[(void *)&h->sx_keys] / sizeof(u64); a.cnt = h->sx_cnt;
     k_self_pairs<<<nw_grid(F, 128), 128, 0, s>>>(a);
     NW_LAUNCH_CHECK();

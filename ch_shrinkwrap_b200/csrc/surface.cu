@@ -90,7 +90,7 @@ __global__ void __launch_bounds__(256) k_tri_extents(const int4 *__restrict__ sf
                 for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], p[k]); hi[k] = fmaxf(hi[k], p[k]); }
             }
         });
-        if (live) node = parent_g[node] & 0x7fffffff;
+        if (live) node = nw_link_node(parent_g[node]);
     }
 }
 
@@ -194,19 +194,15 @@ struct SurfaceArgs {
     int64_t stride;
     const int *perm;                    // resident points: sorted position -> caller's index (NULL: the identity)
     const int *seed;                    // resident points: nearest-centroid slot of the last sweep, or -1 (NULL: none)
-    const Box *tb;
-    const int *parent;
-    const int2 *kids;
-    const int *leaf_of_slot;
+    OctreeView oct;                     // over h->tboxes
     const int4 *sfaces;
     const float4 *posq;
-    int leaf0, leaf_level, n_nodes, F;
     double *dist;                       // caller order; always written
     int *face;                          // or NULL
     double *closest;                    // or NULL
 };
 
-// One query per thread, stackless: first child and next sibling come from the tables the fit's search uses (tree.cu).
+// One query per thread, stackless (common.cuh: nw_walk_subtree) over the tables the fit's search uses (tree.cu).
 struct SurfaceWalk {
     const SurfaceArgs &a;
     float x, y, z;                      // float32 rounding of the query: the box tests use it
@@ -214,17 +210,17 @@ struct SurfaceWalk {
     D3 p;                               // the query, exactly
     double d2 = DBL_MAX * 2.0;          // best squared distance (+inf: none yet)
     float ub = FLT_MAX * 2.0f;          // d2 rounded up, times the 1.1e-5 the float32 frames owe to orthonormality
-    int face = 0x7fffffff, slot = -1;
+    int face = 0x7fffffff, slot = -1;   // (not sweep.cu's Nearest: its field order, slot then face, changes this kernel's registers)
 
     __device__ __forceinline__ SurfaceWalk(const SurfaceArgs &a_) : a(a_) {}
     __device__ __forceinline__ void offer(double v, int f, int s) {
         if (v < d2 || (v == d2 && f < face)) { d2 = v; face = f; slot = s; ub = __fmul_ru(__double2float_ru(v), 1.000011f); }
     }
-    // lower bound of the squared distance from the query to anything in the node (sweep.cu: Traversal::test_node, with the
-    // gaps shrunk by eq), compared with the best so far; `link` = the node's first child | last-child bit
+    __device__ __forceinline__ bool tick() const { return false; }
+    // lower bound of the squared distance from the query to anything in the node (sweep.cu: Traversal::open, with the
+    // gaps shrunk by eq), compared with the best so far
     __device__ __forceinline__ bool open(int node, int &link) const {
-        NW_ASSERT(node >= 0 && node < a.n_nodes);
-        const Box *bp = &a.tb[node];
+        const Box *bp = &a.oct.boxes[node];
         const float4 ba = __ldg(&bp->a), bb = __ldg(&bp->b), bd = __ldg(&bp->d);
         link = __float_as_int(bd.z);
         const float pn = fmaf(ba.x, x, fmaf(ba.z, y, bb.x * z));
@@ -238,9 +234,9 @@ struct SurfaceWalk {
         return __fmaf_rd(g2, g2, s01) <= ub;
     }
     __device__ __forceinline__ void leaf(int node) {
-        NW_ASSERT(node >= a.leaf0 && node < a.n_nodes);
-        const int2 k = __ldg(&a.kids[node]);
-        NW_ASSERT(k.x >= 0 && k.y >= 0 && k.x + k.y <= a.F);
+        NW_ASSERT(node >= a.oct.leaf0 && node < a.oct.n_nodes);
+        const int2 k = __ldg(&a.oct.kids[node]);
+        NW_ASSERT(k.x >= 0 && k.y >= 0 && k.x + k.y <= a.oct.n_slots);
         for (int s = k.x; s < k.x + k.y; ++s) {
             const int4 sf = __ldg(&a.sfaces[s]);
             const float4 va = __ldg(&a.posq[sf.x]), vb = __ldg(&a.posq[sf.y]), vc = __ldg(&a.posq[sf.z]);
@@ -248,38 +244,15 @@ struct SurfaceWalk {
             offer(dist2(p, closest_on_triangle(p, d3(va), d3(vb), d3(vc))), sf.w, s);
         }
     }
-    __device__ __forceinline__ void subtree(int I) {
-        int node = I;
-        while (true) {
-            int link;
-            if (open(node, link)) {
-                if (node >= a.leaf0) leaf(node);
-                else { node = link & 0x7fffffff; continue; }
-            }
-            while (true) {
-                if (node == I) return;
-                if (link >= 0) { ++node; break; }
-                link = __ldg(&a.parent[node]);
-                node = link & 0x7fffffff;
-            }
-        }
-    }
-    // greedy descent to a first leaf for a query without a seed (sweep.cu: node_score)
+    // greedy descent to a first leaf for a query without a seed
     __device__ __forceinline__ int greedy_leaf() const {
         int node = 0;
-        while (node < a.leaf0) {
-            const int2 k = __ldg(&a.kids[node]);
+        while (node < a.oct.leaf0) {
+            const int2 k = __ldg(&a.oct.kids[node]);
             int pick = k.x;
             float bl = FLT_MAX * 2.0f;
             for (int ch = k.x; ch < k.x + k.y; ++ch) {
-                const Box *bp = &a.tb[ch];
-                const float4 ba = __ldg(&bp->a), bb = __ldg(&bp->b), bc = __ldg(&bp->c), bd = __ldg(&bp->d);
-                float pn, p1, p2;
-                project_frame(ba, bb, bc, x, y, z, pn, p1, p2);
-                const float g0 = fmaxf(fmaxf(bb.z - pn, pn - bd.x), 0.f), g1 = fmaxf(fmaxf(bb.w - p1, p1 - bd.y), 0.f),
-                            g2 = fmaxf(fmaxf(bd.w - p2, p2 - bc.w), 0.f);
-                const float c0 = pn - 0.5f * (bb.z + bd.x), c1 = p1 - 0.5f * (bb.w + bd.y), c2 = p2 - 0.5f * (bd.w + bc.w);
-                const float l = (g0 * g0 + g1 * g1 + g2 * g2) + 1e-4f * (c0 * c0 + c1 * c1 + c2 * c2);
+                const float l = node_score(&a.oct.boxes[ch], x, y, z);
                 if (l < bl) { bl = l; pick = ch; }
             }
             node = pick;
@@ -289,11 +262,11 @@ struct SurfaceWalk {
     // the leaf first, then at every level the sibling subtrees of the path to the root
     __device__ __forceinline__ void from_leaf(int node) {
         leaf(node);
-        for (int level = a.leaf_level; level >= 1; --level) {
-            const int p = __ldg(&a.parent[node]) & 0x7fffffff;
-            const int2 k = __ldg(&a.kids[p]);
+        for (int level = a.oct.leaf_level; level >= 1; --level) {
+            const int p = nw_link_node(__ldg(&a.oct.parent[node]));
+            const int2 k = __ldg(&a.oct.kids[p]);
             for (int sib = k.x; sib < k.x + k.y; ++sib)
-                if (sib != node) subtree(sib);
+                if (sib != node) nw_walk_subtree(*this, a.oct, sib);
             node = p;
         }
     }
@@ -315,7 +288,7 @@ __global__ void __launch_bounds__(128) k_surface_nearest(const __grid_constant__
     w.eq = sizeof(T) == 8 ? fmaf(fabsf(w.x) + fabsf(w.y) + fabsf(w.z), 1.1920928955078125e-7f, FLT_MIN) : 0.f;
     if (fabs(w.p.x) <= DBL_MAX && fabs(w.p.y) <= DBL_MAX && fabs(w.p.z) <= DBL_MAX) {
         const int s = a.seed ? __ldg(&a.seed[i]) : -1;
-        w.from_leaf(s >= 0 && s < a.F ? a.leaf0 + __ldg(&a.leaf_of_slot[s]) : w.greedy_leaf());
+        w.from_leaf(s >= 0 && s < a.oct.n_slots ? a.oct.leaf0 + __ldg(&a.oct.leaf_of_slot[s]) : w.greedy_leaf());
     }
     const double nan = __longlong_as_double(0x7ff8000000000000LL);
     D3 c = D3{nan, nan, nan};
@@ -560,8 +533,8 @@ static int surface_check(nw_ctx *h, const char *who, const void *q, int64_t Q) {
 int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, int64_t Q, int64_t stride, bool f64) {
     cudaStream_t s = h->stream;
     const int B = 256;
-    const TreeLevels &tl = h->tl;
-    const int leaf_level = tl.n_levels - 1, leaf0 = tl.off[leaf_level], total = leaf0 + tl.count[leaf_level];
+    const OctreeView v = nw_octree_view(h, h->boxes);      // the sizes of the fit's tree, whose frames and links tboxes copies
+    const int first = h->tl.off[1];
     NW_CHECK(nw_alloc(h, &h->surf_bits, (size_t)8));
     NW_CUDA(cudaMemsetAsync(h->surf_bits, 0, sizeof(unsigned) * 6, s));
     const float *pq = (const float *)h->posq;      // x, y, z of vertex v at pq[4 v + 0..2]
@@ -574,12 +547,12 @@ int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, 
                                                                             Q, stride, h->surf_bits + 3);
         NW_LAUNCH_CHECK();
     }
-    NW_CHECK(nw_alloc(h, &h->tboxes, (size_t)total));
-    k_tbox_init<<<nw_grid(total, B), B, 0, s>>>(h->boxes, total, h->tboxes);
+    NW_CHECK(nw_alloc(h, &h->tboxes, (size_t)v.n_nodes));
+    k_tbox_init<<<nw_grid(v.n_nodes, B), B, 0, s>>>(h->boxes, v.n_nodes, h->tboxes);
     NW_LAUNCH_CHECK();
-    k_tri_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->sfaces, h->posq, h->F, h->leaf_of_slot, leaf0, leaf_level, h->parent_g, h->tboxes);
+    k_tri_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->sfaces, h->posq, h->F, h->leaf_of_slot, v.leaf0, v.leaf_level, h->parent_g, h->tboxes);
     NW_LAUNCH_CHECK();
-    k_tbox_decode<<<nw_grid(total - tl.off[1], B), B, 0, s>>>(h->tboxes, tl.off[1], total - tl.off[1], h->surf_bits);
+    k_tbox_decode<<<nw_grid(v.n_nodes - first, B), B, 0, s>>>(h->tboxes, first, v.n_nodes - first, h->surf_bits);
     NW_LAUNCH_CHECK();
     return NW_OK;
 }
@@ -589,8 +562,6 @@ int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, 
 static int surface_walk(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, bool want_face, bool want_closest, SurfaceArgs &a,
                         bool &f64) {
     cudaStream_t s = h->stream;
-    const TreeLevels &tl = h->tl;
-    const int leaf_level = tl.n_levels - 1, leaf0 = tl.off[leaf_level], total = leaf0 + tl.count[leaf_level];
 
     // queries: the resident points (sorted SoA, results scattered to the caller's order through perm) or a copy of the caller's
     f64 = q ? q_is_f64 != 0 : h->px64 != nullptr;
@@ -616,8 +587,7 @@ static int surface_walk(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, bool 
     NW_CHECK(nw_alloc(h, &h->surf_dist, nq));
     if (want_face) NW_CHECK(nw_alloc(h, &h->surf_face, nq));
     if (want_closest) NW_CHECK(nw_alloc(h, &h->surf_closest, 3 * nq));
-    a.tb = h->tboxes; a.parent = h->parent_g; a.kids = h->kids; a.leaf_of_slot = h->leaf_of_slot; a.sfaces = h->sfaces; a.posq = h->posq;
-    a.leaf0 = leaf0; a.leaf_level = leaf_level; a.n_nodes = total; a.F = h->F;
+    a.oct = nw_octree_view(h, h->tboxes); a.sfaces = h->sfaces; a.posq = h->posq;
     a.dist = h->surf_dist; a.face = want_face ? h->surf_face : nullptr; a.closest = want_closest ? h->surf_closest : nullptr;
     if (Q > 0) {
         if (f64) k_surface_nearest<double><<<nw_grid(Q, 128), 128, 0, s>>>(a);

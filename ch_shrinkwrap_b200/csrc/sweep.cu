@@ -81,6 +81,12 @@ struct Nearest {
     double d2;
     float ub;      // d2 rounded up to float: prune bound for the float32 lower bounds
     int slot, face;
+    // no candidate yet: +inf, so that the first offer wins
+    static __device__ __forceinline__ Nearest none() {
+        Nearest n;
+        n.d2 = DBL_MAX * 2.0; n.ub = FLT_MAX * 2.0f; n.slot = -1; n.face = 0x7fffffff;
+        return n;
+    }
     __device__ __forceinline__ void offer(double v, int s, int f) {
         // strict minimum; exact fp64 ties -> lowest face index (contract of SURVEY 7.3)
         // ub carries the relative 1.1e-5 that the box tests owe to the float32 orthonormality of the node frames (it used to
@@ -94,7 +100,7 @@ struct Nearest {
 // both the query's and the members' evaluation, DESIGN.md "exactness") and the squares by a relative 1e-5 (axes are
 // orthonormal only to float32 accuracy).  A node is skipped only if this bound exceeds the best exact fp64 distance,
 // so skipping can never change the answer.
-// (The walk itself uses the two-stage form of this test, Traversal::test_node.  Each 128-bit load of a node quarter also
+// (The walk itself uses the two-stage form of this test, Traversal::open.  Each 128-bit load of a node quarter also
 // costs two moves of the warp-uniform node address into the vector registers it is about to overwrite; an opaque per-thread
 // copy of the address does not change that allocation at 32 registers, and 256-bit loads do not pay either: DESIGN.md.)
 template <typename Q>
@@ -112,37 +118,24 @@ __device__ __forceinline__ float node_lb(const Q &q, const Box *__restrict__ bp)
     return __fmul_rd(lb, 0.99999f);
 }
 
-// greedy-descent score: the bound, with the squared distance to the box centre as a tie-breaker (several overlapping
-// boxes can contain the query and all have bound 0)
-template <typename Q>
-__device__ __forceinline__ float node_score(const Q &q, const Box *__restrict__ bp) {
-    const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), c = __ldg(&bp->c), d = __ldg(&bp->d);
-    const float x = q.fx(), y = q.fy(), z = q.fz();
-    const float pn = fmaf(a.x, x, fmaf(a.z, y, b.x * z));
-    const float p1 = fmaf(a.y, x, fmaf(a.w, y, b.y * z));
-    const float p2 = fmaf(c.x, x, fmaf(c.y, y, c.z * z));
-    const float g0 = fmaxf(fmaxf(b.z - pn, pn - d.x), 0.f), g1 = fmaxf(fmaxf(b.w - p1, p1 - d.y), 0.f),
-                g2 = fmaxf(fmaxf(d.w - p2, p2 - c.w), 0.f);
-    const float c0 = pn - 0.5f * (b.z + d.x), c1 = p1 - 0.5f * (b.w + d.y), c2 = p2 - 0.5f * (d.w + c.w);
-    return (g0 * g0 + g1 * g1 + g2 * g2) + 1e-4f * (c0 * c0 + c1 * c1 + c2 * c2);
-}
-
-// Stackless search of the octree of occupied Hilbert cells (tree.cu).  All state is scalar and held BY VALUE so that it
-// stays in registers (a per-thread stack array, or references to the caller's query, made the compiler spill the whole
-// object to local memory and reload it inside every node test).  Nodes are addressed by ONE global id (levels stored
-// back to back, root = 0, leaves = [leaf0, n_nodes)), so a step needs no per-level offset lookups.
+// Stackless search of the octree of occupied Hilbert cells (tree.cu, common.cuh: nw_walk_subtree).  All state is scalar
+// and held BY VALUE so that it stays in registers (a per-thread stack array, or references to the caller's query, made the
+// compiler spill the whole object to local memory and reload it inside every node test).
+// The tree fields are those of an OctreeView over h->boxes (make_args copies them from nw_octree_view), interleaved with
+// the centroid search's own: k_sweep1 reads this struct from its parameters, and holding an OctreeView instead reorders
+// those loads and the kernel's register assignment.
 struct TreeView {
     const float4 *__restrict__ cent;
     const double *__restrict__ cent64;  // NULL, or (points mode, float64 targets) the exact coordinates per slot: cent[] only prunes
     const Box *__restrict__ boxes;
-    const int *__restrict__ parent;     // global id of the parent | (the parent is the last child of its parent) << 31
-    const int2 *__restrict__ kids;      // inner node: {global id of the first child, children}; leaf: {first slot, centroids}
-    const int *__restrict__ leaf_of_slot;   // index of the leaf WITHIN the leaf level
+    const int *__restrict__ parent;
+    const int2 *__restrict__ kids;
+    const int *__restrict__ leaf_of_slot;
     const unsigned *__restrict__ fcells;   // grid cell (x | y << 10 | z << 20) each sorted centroid was keyed into at upload
     float3 grid_lo;                        // the 1024^3 grid of those keys: g = (p - grid_lo) * grid_inv
     float grid_inv, grid_cellw;            // cells per nm, nm per cell (0 when the mesh has no extent)
-    int leaf0, leaf_level;                 // global id of the first leaf; its level (= number of climb steps to the root)
-    int n_nodes, n_slots;                  // sizes of boxes[] / cent[] (bounds assertions only)
+    int leaf0, leaf_level;
+    int n_nodes, n_slots;
 };
 
 //
@@ -234,15 +227,14 @@ struct Traversal {
             } else if (q.lb_box(c, c) <= best.ub) { if constexpr (COUNT) ++n_exact; best.offer(q.d2(c), s, __float_as_int(c.w)); }
         }
     }
-    // Depth-first search of the subtree rooted at node I.  First child and next sibling come from two small integer
-    // tables, so no per-thread stack is needed.  Children are visited in index (= Hilbert) order: with a seed the bound
-    // is already (nearly) exact, so nearest-first ordering would buy nothing.
-    // The node test of the walk: node_lb() in two stages.  Normal axis + first tangent axis need three of the node's four
-    // 16-byte quarters; if that partial sum (a lower bound of the full one: the third square only adds) already rules the
-    // node out for every lane, the fourth quarter is never loaded and the third axis never evaluated.  Otherwise the full
-    // bound is formed from the same partial sum: the same nodes are opened as with a one-stage test.
-    __device__ __forceinline__ bool test_node(const Box *__restrict__ bp, int &link) {
-        NW_ASSERT(bp >= tv.boxes && bp < tv.boxes + tv.n_nodes);
+    // The node test of the walk (nw_walk_subtree; children in Hilbert order: with a seed the bound is already (nearly)
+    // exact, so nearest-first ordering would buy nothing): node_lb() in two stages.  Normal axis + first tangent axis need
+    // three of the node's four 16-byte quarters; if that partial sum (a lower bound of the full one: the third square only
+    // adds) already rules the node out for every lane, the fourth quarter is never loaded and the third axis never
+    // evaluated.  Otherwise the full bound is formed from the same partial sum: the same nodes are opened as with a
+    // one-stage test.
+    __device__ __forceinline__ bool open(int node, int &link) {
+        const Box *__restrict__ bp = &tv.boxes[node];
         const float4 a = __ldg(&bp->a), b = __ldg(&bp->b), d = __ldg(&bp->d);
         const float x = q.fx(), y = q.fy(), z = q.fz();
         link = __float_as_int(d.z);
@@ -257,34 +249,10 @@ struct Traversal {
         const float g2 = fmaxf(fmaxf(d.w - p2, p2 - c.w), 0.f);
         return any(__fmaf_rd(g2, g2, s01) <= best.ub);
     }
-    __device__ __forceinline__ void dfs_subtree(int I) {
-        int node = I;
-        while (true) {
-            int link;                                      // first child | (node is a last child) << 31, stored in the node itself
-            if (tick()) return;
-            const bool pass = test_node(&tv.boxes[node], link);
-            if (pass) {
-                if (node >= tv.leaf0) leaf(node);
-                else {
-                    node = link & 0x7fffffff;
-                    // (measured at C3 and rejected: an L1 prefetch of all children here, CCTL.PF1 by lanes 0..7 -- the warm
-                    // sweep went from 2.17 to 2.53 ms and the first sweep of a fit, whose longest packet runs 16 k steps at
-                    // ~1000 cycles each while the average SM is done after 60 % of the launch, did not get shorter)
-                    continue;
-                }
-            }
-            while (true) {
-                if (node == I) return;
-                if (link >= 0) { ++node; break; }          // not the last child: next sibling
-                link = __ldg(&tv.parent[node]);            // parent | (parent is a last child) << 31
-                node = link & 0x7fffffff;
-            }
-        }
-    }
     // Packet prefilter for the climb: all (<= 8) siblings of a level are bounded in ONE step -- lane j evaluates sibling j
     // against the packet centre, which settles it for every lane (set_packet_centre).  Survivors are then searched with
-    // every lane's own, tighter bound (dfs_subtree).  Measured at C3: using the same prefilter for the children inside
-    // dfs_subtree (survivor masks per level in registers) cut the steps from 82 to 65 per point but cost 16 registers
+    // every lane's own, tighter bound (nw_walk_subtree).  Measured at C3: using the same prefilter for the children inside
+    // the subtree walk (survivor masks per level in registers) cut the steps from 82 to 65 per point but cost 16 registers
     // and ran 8 % slower; relying on the packet bound ALONE is hopeless (warps that straddle a jump of the Hilbert curve
     // have a large radius: 80-190 ms instead of 3).
     __device__ __forceinline__ float packet_reach() const {
@@ -308,14 +276,14 @@ struct Traversal {
         const int shared = shared_levels(cell);
         for (int level = tv.leaf_level; level >= 1; --level) {
             if (all(!active || (level <= shared && cube_clear(level)))) return;
-            const int p = __ldg(&tv.parent[node]) & 0x7fffffff;
+            const int p = nw_link_node(__ldg(&tv.parent[node]));
             const int2 k = __ldg(&tv.kids[p]);
             if constexpr (PACKET) {
                 unsigned todo = family_mask(k.x, k.y, node) & 0xffu;           // an octree node has <= 8 children
-                while (todo) { const int j = __ffs(todo) - 1; todo &= todo - 1; dfs_subtree(k.x + j); }
+                while (todo) { const int j = __ffs(todo) - 1; todo &= todo - 1; nw_walk_subtree(*this, tv, k.x + j); }
             } else {
                 for (int sib = k.x; sib < k.x + k.y; ++sib)
-                    if (sib != node) dfs_subtree(sib);
+                    if (sib != node) nw_walk_subtree(*this, tv, sib);
             }
             node = p;
         }
@@ -330,7 +298,7 @@ struct Traversal {
             const int2 k = __ldg(&tv.kids[node]);
             float bl = FLT_MAX * 2.0f;
             for (int ch = k.x; ch < k.x + k.y; ++ch) {
-                float l = node_score(q, &tv.boxes[ch]);
+                float l = node_score(&tv.boxes[ch], q.fx(), q.fy(), q.fz());
                 if constexpr (PACKET) l = __shfl_sync(0xffffffffu, l, lead);
                 if constexpr (COUNT) ++n_tests;
                 if (l < bl) { bl = l; node = ch; }
@@ -574,8 +542,7 @@ __global__ void __launch_bounds__(128) k_seed_leaders(const __grid_constant__ Sw
     const int64_t t = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     const int64_t i = t * stride;
     if (i >= a.P || a.slot[i] >= 0) return;
-    Nearest best;
-    best.d2 = DBL_MAX * 2.0; best.ub = FLT_MAX * 2.0f; best.slot = -1; best.face = 0x7fffffff;
+    Nearest best = Nearest::none();
     const float x = a.px[i], y = a.py[i], z = a.pz[i];
     const float eps = (fabsf(x) + fabsf(y) + fabsf(z) + a.st->coord_l1) * 9.5367431640625e-7f;
     typename std::conditional<F64, QueryF64, QueryF32>::type q;
@@ -634,8 +601,7 @@ __global__ void __launch_bounds__(128) k_seed_from_feet(const __grid_constant__ 
         const int mid = (lo + hi) >> 1;
         if (__ldg(&fkeys[mid]) < key) lo = mid + 1; else hi = mid;
     }
-    Nearest best;
-    best.d2 = DBL_MAX * 2.0; best.ub = FLT_MAX * 2.0f; best.slot = -1; best.face = 0x7fffffff;
+    Nearest best = Nearest::none();
     const float eps = (fabsf(x) + fabsf(y) + fabsf(z) + a.st->coord_l1) * 9.5367431640625e-7f;
     QueryF32 q;
     q.x = x; q.y = y; q.z = z;
@@ -670,11 +636,7 @@ __global__ void __launch_bounds__(128, F64 ? 12 : 16) k_sweep1(const __grid_cons
         xd = x; yd = y; zd = z;
         if (F64) { xd = a.px64[i]; yd = a.py64[i]; zd = a.pz64[i]; }
     }
-    Nearest best;
-    best.d2 = DBL_MAX * 2.0;   // +inf
-    best.ub = FLT_MAX * 2.0f;
-    best.slot = -1;
-    best.face = 0x7fffffff;
+    Nearest best = Nearest::none();
     // cold start: only the first point of every block of 128 was searched from the root (k_seed_leaders); the warps that
     // do not hold it climb from its face too (it may already have been replaced by that point's final answer: just as good)
     const int64_t i0 = (entry & 0x0fffffff) * (int64_t)blockDim.x;
@@ -974,9 +936,9 @@ static Sweep1Args make_args(nw_ctx *h) {
     a.slot = h->slot;
     a.w0 = h->w0; a.w1 = h->w1; a.w2 = h->w2; a.rx = h->rx; a.ry = h->ry; a.rz = h->rz;
     a.posq = h->posq; a.sfaces = h->sfaces; a.F = h->F;
-    a.tv.cent = h->cent; a.tv.cent64 = h->points_mode ? h->cent64 : nullptr; a.tv.boxes = h->boxes; a.tv.parent = h->parent_g; a.tv.kids = h->kids; a.tv.leaf_of_slot = h->leaf_of_slot;
-    a.tv.leaf_level = h->tl.n_levels - 1; a.tv.leaf0 = h->tl.n_levels > 0 ? h->tl.off[h->tl.n_levels - 1] : 0;
-    a.tv.n_nodes = h->tl.n_levels > 0 ? h->tl.off[h->tl.n_levels - 1] + h->tl.count[h->tl.n_levels - 1] : 0; a.tv.n_slots = h->F;
+    const OctreeView o = nw_octree_view(h, h->boxes);
+    a.tv.cent = h->cent; a.tv.cent64 = h->points_mode ? h->cent64 : nullptr; a.tv.boxes = o.boxes; a.tv.parent = o.parent; a.tv.kids = o.kids;
+    a.tv.leaf_of_slot = o.leaf_of_slot; a.tv.leaf0 = o.leaf0; a.tv.leaf_level = o.leaf_level; a.tv.n_nodes = o.n_nodes; a.tv.n_slots = o.n_slots;
     a.tv.fcells = h->fcells; a.tv.grid_lo = make_float3(h->key_lo[0], h->key_lo[1], h->key_lo[2]); a.tv.grid_inv = h->key_inv;
     a.tv.grid_cellw = h->key_inv > 0.f ? 1.f / h->key_inv : 0.f;
     a.acc = h->acc; a.st = h->st;

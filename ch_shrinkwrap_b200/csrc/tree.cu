@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(256) k_extents(const float4 *__restrict__ cent
             project3(make_float3(ba.x, ba.z, b->b.x), c, lo[0], lo[1], lo[2]);
             hi[0] = lo[0]; hi[1] = lo[1]; hi[2] = lo[2];
         });
-        if (live) node = parent_g[node] & 0x7fffffff;
+        if (live) node = nw_link_node(parent_g[node]);
     }
 }
 // ordered-int -> float for the extents written by k_extents.  The intervals are widened by the rounding slack of the
@@ -476,12 +476,11 @@ static int scan_inclusive(nw_ctx *h, const int *in, int *out, int n) {
 static int extents_pass(nw_ctx *h) {
     cudaStream_t s = h->stream;
     const int B = 256;
-    const TreeLevels &tl = h->tl;
-    const int first = tl.off[1], count = tl.off[tl.n_levels - 1] + tl.count[tl.n_levels - 1] - first;
+    const OctreeView v = nw_octree_view(h, h->boxes);
+    const int first = h->tl.off[1], count = v.n_nodes - first;
     k_reset_extents<<<nw_grid(count, B), B, 0, s>>>(h->boxes, first, count);
     NW_LAUNCH_CHECK();
-    k_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->cent, h->F, h->leaf_of_slot, tl.off[tl.n_levels - 1], tl.n_levels - 1, h->parent_g,
-                                             h->boxes);
+    k_extents<<<nw_grid(h->F, B), B, 0, s>>>(h->cent, h->F, h->leaf_of_slot, v.leaf0, v.leaf_level, h->parent_g, h->boxes);
     NW_LAUNCH_CHECK();
     k_box_decode<<<nw_grid(count, B), B, 0, s>>>(h->boxes, first, count, h->st);
     NW_LAUNCH_CHECK();
