@@ -11,10 +11,11 @@ CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libnanowrap.so')
 ARCH = ['-gencode', 'arch=compute_100a,code=sm_100a']
 COMMON = ['-O3', '-std=c++17', '-lineinfo', '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr'] + os.environ.get('NW_EXTRA_FLAGS', '').split()
-# curvature.cu, quality.cu, surface.cu and intersect.cu need one IEEE operation per source operation (see their headers)
+# curvature.cu, quality.cu, surface.cu, hausdorff.cu and intersect.cu need one IEEE operation per source operation (see their headers)
 SOURCES = {'api.cu': [], 'points.cu': [], 'tree.cu': [], 'sweep.cu': [], 'mesh_ops.cu': [], 'comm.cu': [],
            'ring.cu': [], 'benchhook.cu': [], 'xfer.cu': [], 'curvature.cu': ['-fmad=false'], 'quality.cu': ['-fmad=false'],
-           'surface.cu': ['-fmad=false'], 'intersect.cu': ['-fmad=false']}
+           'surface.cu': ['-fmad=false'], 'hausdorff.cu': ['-fmad=false'],
+           'intersect.cu': ['-fmad=false']}
 
 
 def _nvcc():
@@ -27,7 +28,7 @@ def _nvcc():
 def build(force=False, verbose=False):
     nvcc = _nvcc()
     srcs = [os.path.join(CSRC, s) for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
-    deps = srcs + [os.path.join(CSRC, 'common.cuh'), os.path.join(HERE, '..', 'include', 'nanowrap.h')]
+    deps = srcs + [os.path.join(CSRC, 'common.cuh'), os.path.join(CSRC, 'closest.cuh'), os.path.join(HERE, '..', 'include', 'nanowrap.h')]
     if not force and os.path.exists(LIB) and all(os.path.getmtime(d) <= os.path.getmtime(LIB) for d in deps):
         return LIB
     objdir = os.path.join(HERE, 'build')

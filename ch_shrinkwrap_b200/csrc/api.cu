@@ -55,6 +55,9 @@ extern "C" void nw_destroy(nw_ctx *h) {
     nw_free(&h->sgn_twin); nw_free(&h->sgn_voff); nw_free(&h->sgn_vface); nw_free(&h->sgn_k0); nw_free(&h->sgn_k1);
     nw_free(&h->sgn_i0); nw_free(&h->sgn_i1); nw_free(&h->sgn_cnt); nw_free(&h->sgn_nv); nw_free(&h->sgn_vpart); nw_free(&h->sgn_bbox);
     nw_free(&h->sx_flag); nw_free(&h->sx_last); nw_free(&h->sx_keys); nw_free(&h->sx_sorted); nw_free(&h->sx_cnt); nw_free(&h->sx_pairs);
+    nw_free(&h->hb_pos); nw_free(&h->hb_faces); nw_free(&h->hb_vface); nw_free(&h->hb_flag); nw_free(&h->hb_idx); nw_free(&h->hb_slot);
+    nw_free(&h->hb_ent[0]); nw_free(&h->hb_ent[1]); nw_free(&h->hb_q); nw_free(&h->hb_qd); nw_free(&h->hb_qf); nw_free(&h->hb_qs);
+    nw_free(&h->hb_qa); nw_free(&h->hb_st);
     nw_free(&h->acc); nw_free(&h->Sq); nw_free(&h->fdef);
     nw_free(&h->partials); nw_free(&h->st); nw_free(&h->hist);
     nw_free((char **)&h->cub_tmp); nw_free(&h->scratchM); nw_free(&h->scratchP);

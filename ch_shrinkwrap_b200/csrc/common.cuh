@@ -294,6 +294,16 @@ struct nw_ctx {
     unsigned long long *sx_keys = nullptr, *sx_sorted = nullptr;   // (f << 32) | g of every pair found, then sorted
     unsigned long long *sx_cnt = nullptr;        // pairs found, then the 4 statistics of nw_self_intersections
     int2 *sx_pairs = nullptr;                    // the sorted pairs as (f, g)
+    // ---- nw_hausdorff_bounds (hausdorff.cu): only that call (and tboxes / surf_bits, see above) touches these ----
+    float *hb_pos = nullptr;                     // 3M: positions of the mesh passed in (A)
+    int *hb_faces = nullptr;                     // 3F: its face rows
+    int *hb_vface = nullptr;                     // M: lowest finite face row of A that uses the vertex (else 0x7f7f7f7f)
+    int *hb_flag = nullptr, *hb_idx = nullptr;   // per vertex / entry + 1: 0-1 flags and their exclusive scan
+    int *hb_slot = nullptr;                      // F of the handle's mesh: face row -> sorted slot (inverse of sfaces[.].w)
+    char *hb_ent[2] = {nullptr, nullptr};        // the triangles of the current and the next level (hausdorff.cu: HbEntry)
+    double *hb_q = nullptr, *hb_qd = nullptr;    // the level's point queries (x, y, z), their distances
+    int *hb_qf = nullptr, *hb_qs = nullptr, *hb_qa = nullptr;   // their nearest face rows, seed slots, face rows of A
+    char *hb_st = nullptr;                       // running bounds and counters (hausdorff.cu: HbState)
     // ---- solver vectors ----
     unsigned long long *acc = nullptr;           // (M,4) int64 fixed point: AH res xyz, AH 1
     float4 *Sq = nullptr;                        // search directions, interleaved: S_k of vertex v at Sq[3v + k] (48 B per vertex)
@@ -468,3 +478,5 @@ int nw_mesh_check(nw_ctx *h, const std::string &who);   // surface.cu: a mesh to
 // surface.cu: h->surf_bits (the slack of the call: the vertices, and Q queries q?[i * stride] when Q > 0) and h->tboxes (the
 // triangle-bounded boxes at the current positions)
 int nw_surface_boxes(nw_ctx *h, const void *qx, const void *qy, const void *qz, int64_t Q, int64_t stride, bool f64);
+// surface.cu: k_surface_nearest<double> over those boxes for Q interleaved float64 points, seeded at slots (or seed == NULL)
+int nw_surface_walk_f64(nw_ctx *h, const double *q, int64_t Q, const int *seed, double *dist, int *face);

@@ -23,11 +23,16 @@
 // The slack and the triangle-bounded boxes are built by nw_surface_boxes, which nw_self_intersections (intersect.cu) calls
 // too: its broad phase walks the same boxes with a face instead of a query.  Distances and inside/outside answers assume an
 // embedded mesh; nw_self_intersections is the check for faces that cross or touch.
+//
+// The region test lives in closest.cuh, which hausdorff.cu (nw_hausdorff_bounds) includes too; that call walks its points
+// through nw_surface_walk_f64 below.  Its kernels have a file of their own because adding kernels to this one changed the
+// register allocation of k_surface_nearest.
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cub/cub.cuh>
 #include "common.cuh"
+#include "closest.cuh"
 
 namespace {
 
@@ -101,80 +106,7 @@ __global__ void k_tbox_decode(Box *__restrict__ tb, int first, int count, const 
     nw_decode_box(&tb[first + i], call_slack(bits6));
 }
 
-// ---- exact point-to-triangle distance (fp64, fixed operation order; restated in tests/surface_oracle.py) -------------------
-struct D3 { double x, y, z; };
-__device__ __forceinline__ D3 d3(const float4 v) { return D3{(double)v.x, (double)v.y, (double)v.z}; }
-__device__ __forceinline__ D3 sub(const D3 a, const D3 b) { return D3{a.x - b.x, a.y - b.y, a.z - b.z}; }
-__device__ __forceinline__ double dot(const D3 a, const D3 b) { return (a.x * b.x + a.y * b.y) + a.z * b.z; }
-__device__ __forceinline__ D3 axpy(const D3 a, const double t, const D3 e) { return D3{a.x + t * e.x, a.y + t * e.y, a.z + t * e.z}; }
-__device__ __forceinline__ double dist2(const D3 p, const D3 c) { const D3 d = sub(p, c); return dot(d, d); }
-
-// R: also name the feature the closest point lies on (nw_surface_signed_distance), in r.  Region codes: 0 the interior,
-// 1 + k corner k, 4 + k the edge from corner k to corner k + 1 (mod 3).  The operations, and so the points, do not depend on R.
-#define NW_REGION_CORNER(k) (1 + (k))
-#define NW_REGION_EDGE(k) (4 + (k))
-// the segment p0 -> p1 as edge k of a triangle
-template <bool R>
-__device__ __forceinline__ D3 closest_on_segment(const D3 p, const D3 p0, const D3 p1, const int k, int &r) {
-    const D3 e = sub(p1, p0);
-    const double ee = dot(e, e);
-    double t = ee > 0.0 ? dot(sub(p, p0), e) / ee : 0.0;
-    t = fmin(fmax(t, 0.0), 1.0);
-    if (R) r = t == 0.0 ? NW_REGION_CORNER(k) : t == 1.0 ? NW_REGION_CORNER((k + 1) % 3) : NW_REGION_EDGE(k);
-    return axpy(p0, t, e);
-}
-// a zero-area triangle is the union of its three edges: the closest of them, in the order ab, bc, ca (first wins ties)
-template <bool R>
-__device__ __noinline__ D3 closest_on_edges(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
-    int rk;
-    D3 best = closest_on_segment<R>(p, a, b, 0, r);
-    double bd = dist2(p, best);
-    D3 k = closest_on_segment<R>(p, b, c, 1, rk);
-    double kd = dist2(p, k);
-    if (kd < bd) { best = k; bd = kd; if (R) r = rk; }
-    k = closest_on_segment<R>(p, c, a, 2, rk);
-    kd = dist2(p, k);
-    if (kd < bd) { best = k; if (R) r = rk; }
-    return best;
-}
-// Ericson's region test.  Degenerate: the cross product ab x ac is exactly zero, or (rounding of a nearly degenerate
-// triangle) the interior case finds no positive barycentric denominator.
-template <bool R>
-__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c, int &r) {
-    const D3 ab = sub(b, a), ac = sub(c, a);
-    if (ab.y * ac.z - ab.z * ac.y == 0.0 && ab.z * ac.x - ab.x * ac.z == 0.0 && ab.x * ac.y - ab.y * ac.x == 0.0)
-        return closest_on_edges<R>(p, a, b, c, r);
-    const D3 ap = sub(p, a);
-    const double d1 = dot(ab, ap), d2 = dot(ac, ap);
-    if (d1 <= 0.0 && d2 <= 0.0) { r = NW_REGION_CORNER(0); return a; }
-    const D3 bp = sub(p, b);
-    const double d3 = dot(ab, bp), d4 = dot(ac, bp);
-    if (d3 >= 0.0 && d4 <= d3) { r = NW_REGION_CORNER(1); return b; }
-    const double vc = d1 * d4 - d3 * d2;
-    if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) { r = NW_REGION_EDGE(0); return axpy(a, d1 / (d1 - d3), ab); }
-    const D3 cp = sub(p, c);
-    const double d5 = dot(ab, cp), d6 = dot(ac, cp);
-    if (d6 >= 0.0 && d5 <= d6) { r = NW_REGION_CORNER(2); return c; }
-    const double vb = d5 * d2 - d1 * d6;
-    if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) { r = NW_REGION_EDGE(2); return axpy(a, d2 / (d2 - d6), ac); }
-    const double va = d3 * d6 - d5 * d4;
-    if (va <= 0.0 && (d4 - d3) >= 0.0 && (d5 - d6) >= 0.0) {
-        r = NW_REGION_EDGE(1);
-        return axpy(b, (d4 - d3) / ((d4 - d3) + (d5 - d6)), sub(c, b));
-    }
-    const double s = va + vb + vc;
-    if (!(s > 0.0)) return closest_on_edges<R>(p, a, b, c, r);
-    const double denom = 1.0 / s;
-    const double v = vb * denom, w = vc * denom;
-    r = 0;
-    return D3{(a.x + ab.x * v) + ac.x * w, (a.y + ab.y * v) + ac.y * w, (a.z + ab.z * v) + ac.z * w};
-}
-__device__ __forceinline__ D3 closest_on_triangle(const D3 p, const D3 a, const D3 b, const D3 c) {
-    int r;
-    return closest_on_triangle<false>(p, a, b, c, r);
-}
-
-// the operations of the degenerate test above: cross(b - a, c - a) of a face in row order
+// the operations of closest_on_triangle's degenerate test (closest.cuh): cross(b - a, c - a) of a face in row order
 __device__ __forceinline__ D3 cross(const D3 u, const D3 v) { return D3{u.y * v.z - u.z * v.y, u.z * v.x - u.x * v.z, u.x * v.y - u.y * v.x}; }
 // unit normal cr / |cr|; a zero-area face has none and contributes zero
 __device__ __forceinline__ D3 unit_normal(const D3 a, const D3 b, const D3 c) {
@@ -184,8 +116,6 @@ __device__ __forceinline__ D3 unit_normal(const D3 a, const D3 b, const D3 c) {
     const double l = sqrt(l2);
     return D3{cr.x / l, cr.y / l, cr.z / l};
 }
-
-__device__ __forceinline__ bool finite4(const float4 v) { return fabsf(v.x) <= FLT_MAX && fabsf(v.y) <= FLT_MAX && fabsf(v.z) <= FLT_MAX; }
 
 // ---- the walk ------------------------------------------------------------------------------------------------------
 struct SurfaceArgs {
@@ -597,6 +527,21 @@ static int surface_walk(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, bool 
     return NW_OK;
 }
 
+// nw_hausdorff_bounds (hausdorff.cu): Q float64 points q (x, y, z interleaved) walked over h->tboxes as nw_surface_boxes left
+// them; seed: a slot per point to start from, or NULL.  dist and face (face rows) per point, on the handle's stream.
+int nw_surface_walk_f64(nw_ctx *h, const double *q, int64_t Q, const int *seed, double *dist, int *face) {
+    SurfaceArgs a;
+    a.Q = Q; a.qx = q; a.qy = q + 1; a.qz = q + 2; a.stride = 3;
+    a.perm = nullptr; a.seed = seed;
+    a.oct = nw_octree_view(h, h->tboxes); a.sfaces = h->sfaces; a.posq = h->posq;
+    a.dist = dist; a.face = face; a.closest = nullptr;
+    if (Q > 0) {
+        k_surface_nearest<double><<<nw_grid(Q, 128), 128, 0, h->stream>>>(a);
+        NW_LAUNCH_CHECK();
+    }
+    return NW_OK;
+}
+
 extern "C" int nw_surface_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q, double *dist, int32_t *face, double *closest,
                                    double summary[3]) {
     if (!h) return NW_ERR_ARG;
@@ -727,3 +672,4 @@ extern "C" int nw_surface_signed_distance(nw_ctx *h, const void *q, int q_is_f64
     NW_CUDA(cudaStreamSynchronize(s));
     return NW_OK;
 }
+

@@ -207,6 +207,22 @@ int nw_surface_signed_distance(nw_ctx *h, const void *q, int q_is_f64, int64_t Q
  * stage, degenerate faces, faces with a non-finite corner}.  The signed distance and the enclosed volume assume no such
  * pair.  Changes nothing that nw_search reads.  NW_ERR_ARG in points mode or without a topology; no collectives. */
 int nw_self_intersections(nw_ctx *h, int32_t *pairs, int64_t capacity, int64_t *n_pairs, int64_t stats[4]);
+/* Certified bounds of the one-sided Hausdorff distance h(A -> B) = max over the points p of A's closed triangles of d_B(p),
+ * d_B the exact distance to B's closed triangles (nw_surface_distance).  A is passed in: pos (M,3) float32, faces (F,3)
+ * int32 rows; B is the handle's current mesh (after nw_search, the fitted surface).  bounds = {lower, upper} with
+ * lower - eps <= h(A -> B) <= upper, eps = 2^-40 x the L1 bound (sum over the axes of the largest |coordinate|) of A's used
+ * vertices and B's vertices.  lower is attained: it is the nw_surface_distance value, bit for bit, of witness (3 float64), a
+ * point of face row witness_faces[0] of A whose nearest face row of B is witness_faces[1].  A branch and bound over A's
+ * triangles: each is bounded through the convexity of the distance to single faces of B and the 1-Lipschitz distance,
+ * retired when its bound is within tol of lower, else split at its edge midpoints (the next level's point walks).  It
+ * stops when nothing is left (converged: upper - lower <= tol) or before a level that would take the total of point walks
+ * past max_queries (the bounds reached are still valid).  stats (or NULL) = {levels, triangles bounded, point walks, faces of
+ * A skipped for a non-finite corner, converged}.  Only vertices some finite face of A uses are measured.  NW_ERR_ARG for a
+ * face index outside [0, M), when A or B has no finite face, for tol < 0, for max_queries below the number of vertices A
+ * uses, and in points mode.  Deterministic (bit-identical from call to call); changes nothing that nw_search reads; no
+ * collectives.  Any output may be NULL. */
+int nw_hausdorff_bounds(nw_ctx *h, const float *pos, int M, const int32_t *faces, int F, double tol, int64_t max_queries,
+                        double bounds[2], double witness[3], int32_t witness_faces[2], int64_t stats[5]);
 
 /* ---- measurement hooks (bench.py / profiling; not part of the reference surface) ------------------ */
 /* device-resident single-kernel launches on the handle's stream, for CUDA-event timing */

@@ -2,10 +2,12 @@
 501 762-vertex mesh, and the two-way Hausdorff distance of two C3 fits.  With --signed, also the signed distance
 (nw_surface_signed_distance): a call with no queries just after an upload (twin table, vertex CSR, pseudonormals, volume) and
 repeated (pseudonormals and volume), and the 10^7 resident localisations signed and unsigned, alternating call by call.
+With --bounds, also the certified bounds of the Hausdorff distance between the two C3 fits (nw_hausdorff_bounds, both ways,
+tol = 0.01 nm) against the sampled hausdorff_distance at dx_min = 5, alternating call by call on one auxiliary handle.
 
 Every time is a host clock around calls that end in a stream synchronise (each nw_surface_distance call does), so it is
 device time plus the call's small host overhead: the median and the minimum of `reps` calls after two warm-up calls.
-  python tools/surface_probe.py [--reps 10] [--signed] [--out FILE.json]"""
+  python tools/surface_probe.py [--reps 10] [--signed] [--bounds] [--out FILE.json]"""
 import argparse
 import ctypes
 import json
@@ -79,10 +81,34 @@ def signed_legs(h, fit, P, reps):
     return res
 
 
+def bounds_legs(fit_a, fit_b, reps):
+    """hausdorff_bounds(fit_a, fit_b, tol=0.01) against hausdorff_distance(dx_min=5), alternating on one auxiliary handle."""
+    aux = eu._lib.Handle(0)
+    try:
+        r, s01, s10 = eu.hausdorff_bounds(fit_a, fit_b, tol=0.01, handle=aux, return_stats=True)
+        hd = eu.hausdorff_distance(fit_a, fit_b, dx_min=5, handle=aux)
+        res = {'tol': 0.01, 'lower01': r.lower01, 'upper01': r.upper01, 'lower10': r.lower10, 'upper10': r.upper10,
+               'converged': r.converged,
+               'witness01': [r.witness01[0].tolist(), r.witness01[1], r.witness01[2]],
+               'witness10': [r.witness10[0].tolist(), r.witness10[1], r.witness10[2]],
+               'stats_keys': ['levels', 'entries_bounded', 'point_walks', 'faces_skipped', 'converged'],
+               'stats01': [int(x) for x in s01], 'stats10': [int(x) for x in s10],
+               'hausdorff_distance_dx5': {'h01': hd.h01, 'h10': hd.h10},
+               'upper01_ge_6.21': r.upper01 >= 6.21, 'upper10_ge_71.17': r.upper10 >= 71.17,
+               'sampled_le_upper': hd.h01 <= r.upper01 and hd.h10 <= r.upper10}
+        res['times'] = timed_alternating({
+            'hausdorff_bounds_tol0.01': lambda: eu.hausdorff_bounds(fit_a, fit_b, tol=0.01, handle=aux),
+            'hausdorff_distance_dx5': lambda: eu.hausdorff_distance(fit_a, fit_b, dx_min=5, handle=aux)}, reps)
+    finally:
+        aux.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--reps', type=int, default=10)
     ap.add_argument('--signed', action='store_true')
+    ap.add_argument('--bounds', action='store_true')
     ap.add_argument('--out', default=None)
     args = ap.parse_args()
     gpu = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
@@ -119,6 +145,8 @@ def main():
     aux.close()
     if args.signed:
         res['signed'] = signed_legs(h, fit_b, P, args.reps)
+    if args.bounds:
+        res['bounds'] = bounds_legs(fit_a, fit_b, args.reps)
     line = json.dumps(res)
     print(line)
     if args.out:
