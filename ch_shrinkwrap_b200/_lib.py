@@ -55,6 +55,7 @@ SIGNATURES = {
     'nw_surface_signed_distance': (c_int, [c_void_p, c_void_p, c_int, c_int64, _d, _i, _d, _d]),
     'nw_self_intersections': (c_int, [c_void_p, _i, c_int64, POINTER(c_int64), POINTER(c_int64)]),
     'nw_hausdorff_bounds': (c_int, [c_void_p, _f, c_int, _i, c_int, c_double, c_int64, _d, _d, _i, POINTER(c_int64)]),
+    'nw_mean_distance_bounds': (c_int, [c_void_p, _f, c_int, _i, c_int, c_double, c_int64, _d, POINTER(c_int64)]),
     'nw_bench_kernel': (c_int, [c_void_p, c_char_p, c_int, _f]),
     'nw_sync': (c_int, [c_void_p]),
     'nw_reset_seeds': (c_int, [c_void_p]),

@@ -58,6 +58,7 @@ extern "C" void nw_destroy(nw_ctx *h) {
     nw_free(&h->hb_pos); nw_free(&h->hb_faces); nw_free(&h->hb_vface); nw_free(&h->hb_flag); nw_free(&h->hb_idx); nw_free(&h->hb_slot);
     nw_free(&h->hb_ent[0]); nw_free(&h->hb_ent[1]); nw_free(&h->hb_q); nw_free(&h->hb_qd); nw_free(&h->hb_qf); nw_free(&h->hb_qs);
     nw_free(&h->hb_qa); nw_free(&h->hb_st);
+    nw_free(&h->mb_area); nw_free(&h->mb_val); nw_free(&h->mb_part); nw_free(&h->mb_st);
     nw_free(&h->acc); nw_free(&h->Sq); nw_free(&h->fdef);
     nw_free(&h->partials); nw_free(&h->st); nw_free(&h->hist);
     nw_free((char **)&h->cub_tmp); nw_free(&h->scratchM); nw_free(&h->scratchP);

@@ -304,6 +304,11 @@ struct nw_ctx {
     double *hb_q = nullptr, *hb_qd = nullptr;    // the level's point queries (x, y, z), their distances
     int *hb_qf = nullptr, *hb_qs = nullptr, *hb_qa = nullptr;   // their nearest face rows, seed slots, face rows of A
     char *hb_st = nullptr;                       // running bounds and counters (hausdorff.cu: HbState)
+    // ---- nw_mean_distance_bounds (hausdorff.cu): only that call (and the hb_ buffers above, tboxes, surf_bits) touches these ----
+    double *mb_area = nullptr;                   // 4F: |T0| of every face of A: nearest, lower and upper bound (MbState)
+    double *mb_val = nullptr;                    // 4 per entry: [lo, hi] of the integrals of d_B and d_B^2 over it
+    double *mb_part = nullptr;                   // 8 NW_MB_BLOCKS: the blocks' fixed-order sums (all entries, retired ones)
+    char *mb_st = nullptr;                       // best brackets, retired totals and counters (hausdorff.cu: MbState)
     // ---- solver vectors ----
     unsigned long long *acc = nullptr;           // (M,4) int64 fixed point: AH res xyz, AH 1
     float4 *Sq = nullptr;                        // search directions, interleaved: S_k of vertex v at Sq[3v + k] (48 B per vertex)

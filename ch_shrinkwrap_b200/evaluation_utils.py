@@ -22,6 +22,8 @@ Not in the reference (its surface metrics compare sample clouds, so their answer
   from exact point-to-surface distances of each mesh's samples.
 * ``hausdorff_bounds(mesh0, mesh1, tol)`` -- certified bounds of the one-sided and symmetric Hausdorff distances, with the
   points that attain the lower bounds (``nw_hausdorff_bounds``).
+* ``mean_distance_bounds(mesh0, mesh1, tol)`` -- certified bounds of the area-weighted mean and RMS distances between two
+  meshes, both ways (``nw_mean_distance_bounds``): the continuous counterpart of ``average_squared_distance``.
 
 No CPU fallback: these raise if libnanowrap.so or the GPU is missing.
 """
@@ -246,7 +248,8 @@ def hausdorff_distance(mesh0, mesh1, dx_min=5, handle=None):
 
     Each one-sided value is exact on its sample set, so it is a lower bound of the continuous one-sided Hausdorff distance
     (the supremum over the whole surface) and converges to it as ``dx_min -> 0``; ``hausdorff_bounds`` brackets the
-    continuous value itself.  The reductions run on the GPU in a fixed
+    continuous value itself.  ``mean01`` and ``mean10`` weight every sample alike, not by area, and their error depends on
+    ``dx_min``; ``mean_distance_bounds`` brackets the area-weighted mean and RMS distances.  The reductions run on the GPU in a fixed
     order: repeated calls give identical numbers, and swapping the meshes swaps h01 / h10 and mean01 / mean10 exactly.
     Returns a ``HausdorffResult(h01, h10, hausdorff, mean01, mean10)``."""
     h = handle if handle is not None else _lib.Handle(0)
@@ -303,6 +306,53 @@ def hausdorff_bounds(mesh0, mesh1, tol=0.01, max_queries=HAUSDORFF_MAX_QUERIES, 
         if handle is None:
             h.close()
     r = HausdorffBounds(lo01, up01, lo10, up10, max(lo01, lo10), max(up01, up10), bool(st01[4] and st10[4]), w01, w10)
+    return (r, st01, st10) if return_stats else r
+
+
+MeanDistanceBounds = namedtuple('MeanDistanceBounds', 'mean01_lower mean01_upper rms01_lower rms01_upper mean10_lower '
+                                                     'mean10_upper rms10_lower rms10_upper area0 area1 converged')
+
+
+def _mean_distance_bounds(h, mesh, tol, max_queries):
+    """nw_mean_distance_bounds from `mesh` to the handle's mesh: (out (5,) float64, stats (7,) int64)."""
+    pos = _lib.as_f32(mesh._vertices['position'])
+    faces = np.ascontiguousarray(mesh.faces, dtype=np.int32)
+    out, stats = np.zeros(5), np.zeros(7, np.int64)
+    h.call('nw_mean_distance_bounds', _lib.fptr(pos), len(pos), _lib.iptr(faces), len(faces), float(tol), int(max_queries),
+           _lib.dptr(out), stats.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)))
+    return out, stats
+
+
+def mean_distance_bounds(mesh0, mesh1, tol=0.01, max_queries=HAUSDORFF_MAX_QUERIES, handle=None, return_stats=False):
+    """Certified bounds of the area-weighted mean and RMS distances between two triangle meshes, both ways.
+
+    mean01 = (1/|A|) x the integral over mesh0's finite faces A of d_1, the exact distance to mesh1's closed triangles (the
+    quantity ``surface_distance`` measures), and rms01 = sqrt((1/|A|) x the integral of d_1^2): the continuous counterparts
+    of the reference's ``average_squared_distance`` of two sample clouds, independent of any sampling step.  mean10 and
+    rms10 the same the other way.  ``mean01_lower - eps <= mean01 <= mean01_upper + eps`` and likewise for the other three,
+    eps = 2^-40 x the sum over the axes of the largest |coordinate| of both meshes' used vertices; ``area0`` and ``area1``
+    are the total areas of the finite faces.
+
+    The same branch and bound over the triangles as ``hausdorff_bounds``: each triangle's integrals are bracketed from above
+    by the convexity of the distance to single faces and from below by concavity and by support planes of every face of the
+    other mesh that can be nearest on it, so a triangle lying over the inside of one face is settled without a split.
+    ``converged`` when both gaps are at most ``tol`` (mesh units) both ways; a call that would pass ``max_queries`` point walks
+    in one direction stops early with valid, wider brackets.  Faces with a non-finite corner are skipped and counted, faces
+    of zero area counted.  Repeated calls give identical numbers, and swapping the meshes swaps the 01 and 10 fields.
+    ``return_stats``: also the two stats arrays (levels, triangles bounded, point walks, candidate faces evaluated, faces
+    skipped as non-finite, zero-area faces, converged) of ``nw_mean_distance_bounds``.  ValueError for a mesh with no finite
+    face or zero total area, a face index out of range, ``tol < 0`` or too small a ``max_queries``."""
+    h = handle if handle is not None else _lib.Handle(0)
+    try:
+        _upload_surface(h, mesh1)
+        o01, st01 = _mean_distance_bounds(h, mesh0, tol, max_queries)
+        _upload_surface(h, mesh0)
+        o10, st10 = _mean_distance_bounds(h, mesh1, tol, max_queries)
+    finally:
+        if handle is None:
+            h.close()
+    r = MeanDistanceBounds(*(float(x) for x in o01[1:]), *(float(x) for x in o10[1:]), float(o01[0]), float(o10[0]),
+                           bool(st01[6] and st10[6]))
     return (r, st01, st10) if return_stats else r
 
 

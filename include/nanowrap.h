@@ -223,6 +223,21 @@ int nw_self_intersections(nw_ctx *h, int32_t *pairs, int64_t capacity, int64_t *
  * collectives.  Any output may be NULL. */
 int nw_hausdorff_bounds(nw_ctx *h, const float *pos, int M, const int32_t *faces, int F, double tol, int64_t max_queries,
                         double bounds[2], double witness[3], int32_t witness_faces[2], int64_t stats[5]);
+/* Certified bounds of the area-weighted mean and RMS distance from A to B over A's finite faces: with |A| their total area,
+ * mean = (1/|A|) integral over A of d_B and rms = sqrt((1/|A|) integral over A of d_B^2), d_B as for nw_hausdorff_bounds
+ * (A passed in as there, B the handle's current mesh).  out = {|A|, mean_lo, mean_hi, rms_lo, rms_hi} with
+ * mean_lo - eps <= mean <= mean_hi + eps and the same for rms, eps = 2^-40 x the L1 bound of A's used vertices and B's
+ * vertices.  The same branch and bound over A's triangles as nw_hausdorff_bounds: each triangle's integrals are bracketed
+ * from below by concavity and by support planes of a complete set of candidate faces of B, from above by convexity, and the
+ * triangles whose gaps are small enough for tol are retired, the others split at their edge midpoints.  It stops when both
+ * gaps are <= tol (converged), when every triangle is retired, or before a level that would take the point walks past
+ * max_queries (the brackets reached are still valid).  stats (or NULL) = {levels, triangles bounded, point walks, candidate
+ * faces evaluated by the support-plane stage, faces of A skipped for a non-finite corner, faces of A whose fp64 area is 0,
+ * converged}.  NW_ERR_ARG for a face index outside [0, M), when A or B has no finite face, when A's finite faces have zero
+ * total area, for tol < 0, for max_queries below the number of vertices A uses, and in points mode.  Deterministic;
+ * changes nothing that nw_search reads; no collectives.  Any output may be NULL. */
+int nw_mean_distance_bounds(nw_ctx *h, const float *pos, int M, const int32_t *faces, int F, double tol, int64_t max_queries,
+                            double out[5], int64_t stats[7]);
 
 /* ---- measurement hooks (bench.py / profiling; not part of the reference surface) ------------------ */
 /* device-resident single-kernel launches on the handle's stream, for CUDA-event timing */

@@ -4,10 +4,13 @@
 repeated (pseudonormals and volume), and the 10^7 resident localisations signed and unsigned, alternating call by call.
 With --bounds, also the certified bounds of the Hausdorff distance between the two C3 fits (nw_hausdorff_bounds, both ways,
 tol = 0.01 nm) against the sampled hausdorff_distance at dx_min = 5, alternating call by call on one auxiliary handle.
+With --mean-bounds, the certified bounds of the area-weighted mean and RMS distances between the same two fits
+(nw_mean_distance_bounds, both ways, tol = 0.01 nm, the default budget), alternating with hausdorff_distance(dx_min = 5)
+and with the reference's average_squared_distance of two points_from_mesh(dx_min = 5) sample clouds (sampling included).
 
 Every time is a host clock around calls that end in a stream synchronise (each nw_surface_distance call does), so it is
 device time plus the call's small host overhead: the median and the minimum of `reps` calls after two warm-up calls.
-  python tools/surface_probe.py [--reps 10] [--signed] [--bounds] [--out FILE.json]"""
+  python tools/surface_probe.py [--reps 10] [--signed] [--bounds] [--mean-bounds] [--out FILE.json]"""
 import argparse
 import ctypes
 import json
@@ -104,11 +107,39 @@ def bounds_legs(fit_a, fit_b, reps):
     return res
 
 
+def mean_bounds_legs(fit_a, fit_b, reps):
+    """mean_distance_bounds(fit_a, fit_b, tol=0.01) against hausdorff_distance(dx_min=5) and average_squared_distance of
+    points_from_mesh samples, alternating; the first two on one auxiliary handle."""
+    aux = eu._lib.Handle(0)
+
+    def sampled():
+        return eu.average_squared_distance(eu.points_from_mesh(fit_a, dx_min=5), eu.points_from_mesh(fit_b, dx_min=5))
+    try:
+        r, s01, s10 = eu.mean_distance_bounds(fit_a, fit_b, tol=0.01, handle=aux, return_stats=True)
+        hd = eu.hausdorff_distance(fit_a, fit_b, dx_min=5, handle=aux)
+        np.random.seed(0)
+        asd = sampled()
+        res = dict(r._asdict(), tol=0.01, max_queries=eu.HAUSDORFF_MAX_QUERIES,
+                   stats_keys=['levels', 'entries_bounded', 'point_walks', 'candidate_faces', 'faces_nonfinite', 'faces_zero_area',
+                               'converged'],
+                   stats01=[int(x) for x in s01], stats10=[int(x) for x in s10],
+                   hausdorff_distance_dx5={'mean01': hd.mean01, 'mean10': hd.mean10},
+                   average_squared_distance_dx5=[float(x) for x in np.ravel(asd)])
+        res['times'] = timed_alternating({
+            'mean_distance_bounds_tol0.01': lambda: eu.mean_distance_bounds(fit_a, fit_b, tol=0.01, handle=aux),
+            'hausdorff_distance_dx5': lambda: eu.hausdorff_distance(fit_a, fit_b, dx_min=5, handle=aux),
+            'points_from_mesh_dx5_average_squared_distance': sampled}, reps)
+    finally:
+        aux.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--reps', type=int, default=10)
     ap.add_argument('--signed', action='store_true')
     ap.add_argument('--bounds', action='store_true')
+    ap.add_argument('--mean-bounds', action='store_true')
     ap.add_argument('--out', default=None)
     args = ap.parse_args()
     gpu = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
@@ -147,6 +178,8 @@ def main():
         res['signed'] = signed_legs(h, fit_b, P, args.reps)
     if args.bounds:
         res['bounds'] = bounds_legs(fit_a, fit_b, args.reps)
+    if args.mean_bounds:
+        res['mean_bounds'] = mean_bounds_legs(fit_a, fit_b, args.reps)
     line = json.dumps(res)
     print(line)
     if args.out:
